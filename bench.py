@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- VMC walker-updates/s (sample + E_loc + grad) on the N = 20 ground-state quantum dot.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" is one VMC iteration of reference src/FermionHO2D.py's loop body on `--walkers`
@@ -53,7 +53,15 @@ def parse():
                         "(configs[3]: Z 8, N 12, 32 RK4 steps, finite T) | slater_sweep (configs[4]: log|det| + gradient + "
                         "Laplacian, N = 6..30, 1e6 walkers).  The extra configurations print the same JSON shape; the driver "
                         "runs the default only.")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write what the last one computed as DIR/<name>.npy (n20, --impl ours; "
+                        "rank 0's walkers, a seeded sample of them when they exceed 60 MB)")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.config != "n20"):
+        p.error("--dump-outputs covers the n20 configuration of --impl ours")
+    return a
 
 
 class ClockSampler(threading.Thread):
@@ -127,6 +135,32 @@ def build_model(args, dev):
     cnf = CNF(Backflow(eta, mu=mu), (0.0, 1.0), nsteps=args.ode_steps)
     model = GSVMC(args.nup, args.ndown, HO2D(), FreeFermion(dev), cnf, CoulombPairPotential(args.Z), sp_potential=HO())
     return model.to(dev)
+
+
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, model):
+    """What a caller of one VMC iteration receives, as float64 .npy files: the per-walker results of the E_loc sweep
+    (model.last), the energy estimate, the parameter gradients and the parameters after the optimiser step.  Runs of
+    the same arguments see the same inputs, so two builds can be compared file by file."""
+    import numpy as np
+    last = model.last
+    per_walker = {k: getattr(last, k) for k in ("z", "delta_logp", "logp", "grad", "lap", "kinetic", "potential", "eloc")}
+    B = last.eloc.shape[0]
+    row_bytes = sum(t[0].numel() * 8 for t in per_walker.values())
+    rows = None
+    if B * row_bytes > DUMP_BYTES:
+        keep = DUMP_BYTES // row_bytes
+        rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:keep].sort().values.to(last.eloc.device)
+    arrays = {"walker_" + k: t if rows is None else t[rows] for k, t in per_walker.items()}
+    arrays["energy"] = model.observables_device()             # E, E_std
+    for name, p in model.named_parameters():
+        arrays["param." + name] = p.detach()
+        arrays["param_grad." + name] = p.grad
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to("cpu", torch.float64).numpy())
 
 
 def run_ours(args):
@@ -203,6 +237,8 @@ def run_ours(args):
     launches = L.lib().ff_launch_count() - launches0
     ms = t0.elapsed_time(t1)
     eloc_ms = sum(a.elapsed_time(b) for a, b in eloc_events) / max(len(eloc_events), 1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model)
 
     # end-to-end through the public API with HOST buffers: parameters come from pinned host
     # memory every step, energy moments and the gradient go back to the host.

@@ -141,31 +141,36 @@ def test_cnf_state_dict_has_the_reference_layout():
     assert torch.equal(cnf.v.mu.fc2.weight, old["v.mu.fc2.weight"])
 
 
-def test_reference_cnf_checkpoint_round_trip_if_reference_present():
-    """With /root/reference available (build container only): save from the real reference, load here, and back."""
-    import sys
-    ref = os.environ.get("FERMIFLOW_REFERENCE", "/root/reference")
-    if not os.path.isdir(os.path.join(ref, "src")):
-        pytest.skip("reference sources not present on this machine")
-    import subprocess
-    code = (
-        "import sys, torch\n"
-        "sys.path[:0] = [%r, %r]\n"
-        "from MLP import MLP; from equivariant_funs import Backflow; from flow import CNF\n"
-        "c = CNF(Backflow(MLP(1, 5), mu=MLP(1, 4)), (0., 1.))\n"
-        "torch.save(c.state_dict(), sys.argv[1])\n"
-        "if len(sys.argv) > 2: c.load_state_dict(torch.load(sys.argv[2]), strict=True); print('loaded-ours')\n"
-    ) % (os.path.join(ROOT, "oracle", "torchdiffeq_shim"), os.path.join(ref, "src"))
-    import tempfile
+def test_reference_cnf_checkpoint_round_trip(tmp_path):
+    """A checkpoint file as the reference writes it for CNF(Backflow(MLP(1, 5), mu=MLP(1, 4)), t_span) (keys of
+    REFERENCE_CNF_KEYS, MLP fc1 with bias and fc2 without, every `f.v.` entry the same tensor as its `v_wrapper.v.`
+    twin) loads here with strict=True, and the file saved back has the same keys, shapes, dtypes and sharing, which
+    is what the reference's strict load of it checks."""
+    from collections import OrderedDict
     from fermiflow_b200 import MLP, Backflow, CNF
-    with tempfile.TemporaryDirectory() as d:
-        a, b = os.path.join(d, "ref.pt"), os.path.join(d, "ours.pt")
-        subprocess.run([sys.executable, "-W", "ignore", "-c", code, a], check=True)
-        cnf = CNF(Backflow(MLP(1, 5), mu=MLP(1, 4)), (0.0, 1.0))
-        cnf.load_state_dict(torch.load(a), strict=True)
-        torch.save(cnf.state_dict(), b)
-        out = subprocess.run([sys.executable, "-W", "ignore", "-c", code, a, b], check=True, capture_output=True, text=True)
-        assert "loaded-ours" in out.stdout
+    H = {"eta": 5, "mu": 4}
+    shapes = {"fc1.weight": lambda h: (h, 1), "fc1.bias": lambda h: (h,), "fc2.weight": lambda h: (1, h)}
+    gen = torch.Generator().manual_seed(3)
+    ref = OrderedDict()
+    for k in REFERENCE_CNF_KEYS:
+        if k.startswith("f.v."):
+            ref[k] = ref["v_wrapper.v." + k[len("f.v."):]]
+        else:
+            net, layer = k.split(".")[2], ".".join(k.split(".")[3:])
+            ref[k] = torch.randn(shapes[layer](H[net]), generator=gen, dtype=torch.float64)
+    a, b = tmp_path / "ref.pt", tmp_path / "ours.pt"
+    torch.save(ref, a)
+    cnf = CNF(Backflow(MLP(1, 5), mu=MLP(1, 4)), (0.0, 1.0))
+    cnf.load_state_dict(torch.load(a), strict=True)
+    for k, v in ref.items():
+        assert torch.equal(cnf.state_dict()[k], v), k
+    torch.save(cnf.state_dict(), b)
+    ours = torch.load(b)
+    assert list(ours) == REFERENCE_CNF_KEYS
+    for k, v in ref.items():
+        assert ours[k].shape == v.shape and ours[k].dtype == v.dtype and torch.equal(ours[k], v), k
+        if k.startswith("f.v."):
+            assert ours[k].data_ptr() == ours["v_wrapper.v." + k[len("f.v."):]].data_ptr(), k
 
 
 def test_metropolis_seed_and_rank_offset(monkeypatch):

@@ -72,8 +72,11 @@ def _beta_worker(rank, world, port, out):
     gathered_s = [torch.zeros(B // world, dtype=torch.long) for _ in range(world)]
     dist.all_gather(gathered, w); dist.all_gather(gathered_E, E); dist.all_gather(gathered_s, st)
     if rank == 0:
-        out.put(({k: float(v) for k, v in obs.items() if k != "logp_states_all"}, float(nglobal), grad,
-                 torch.cat(gathered), torch.cat(gathered_E), torch.cat(gathered_s), lw_full, beta))
+        # numpy copies travel by value; a torch tensor in the queue would be fetched from this process, which may have
+        # exited by then
+        out.put(({k: float(v) for k, v in obs.items() if k != "logp_states_all"}, float(nglobal), grad.numpy(),
+                 torch.cat(gathered).numpy(), torch.cat(gathered_E).numpy(), torch.cat(gathered_s).numpy(),
+                 lw_full.numpy(), beta))
     dist.destroy_process_group()
 
 
@@ -90,6 +93,7 @@ def test_finite_temperature_estimators_allreduce_gloo():
     obs, nglobal, grad, w, E, st, lw_full, beta = q.get(timeout=120)
     for p in procs:
         p.join(timeout=60)
+    grad, w, E, st, lw_full = (torch.from_numpy(a) for a in (grad, w, E, st, lw_full))
     assert nglobal == 40
     lw = lw_full.clone().requires_grad_(True)
     ref = O.beta_vmc_estimators(E, st, lw, beta)
