@@ -24,9 +24,12 @@ int cuda_fail(cudaError_t e, const char* what) {
     return fail((int)e, "%s: %s", what, cudaGetErrorString(e));
 }
 
-const char* const kOptNames[OPT_COUNT] = {
+// in the order of enum Opt
+const char* const kOptNames[] = {
     "no_table", "no_w_balance", "no_rt_cache", "flow_warp_fill", "flow_cta", "flow_big", "eloc_generic", "slater_cta",
-    "metropolis_kernel", "adjoint_cta", "pgrad_direct", "pgrad_tile", "pgrad_fixed_range", "eloc_v2", "eloc_v4", "adjoint_no_prefetch", "finale_cta", "metropolis_no_split"};
+    "metropolis_kernel", "adjoint_cta", "pgrad_direct", "pgrad_tile", "pgrad_fixed_range", "adjoint_no_prefetch", "finale_cta",
+    "metropolis_no_split"};
+static_assert(sizeof(kOptNames) / sizeof(kOptNames[0]) == OPT_COUNT, "one name per option");
 std::atomic<int> g_opt[OPT_COUNT];
 std::atomic<long long> g_launches{0};
 

@@ -36,8 +36,6 @@ enum Opt {
     OPT_PGRAD_DIRECT,        // direct parameter-gradient kernel (every hidden unit) instead of binned Taylor moments
     OPT_PGRAD_TILE,          // walker-stages per tile of the binned kernel (0 -> 32)
     OPT_PGRAD_FIXED_RANGE,   // eta nodes over the fixed range instead of the sampled 99.9 % quantile
-    OPT_ELOC_V2,             // previous-generation E_loc sweep (eloc2_kernel: J and its RK partials in shared memory)
-    OPT_ELOC_V4,             // register-resident E_loc sweep without warp specialisation (eloc4_kernel)
     OPT_ADJOINT_NO_PREFETCH, // adjoint sweep without the bulk prefetch of the next stage's stash into L2
     OPT_FINALE_CTA,          // CTA-synchronous finale of the register-resident E_loc sweeps instead of one warp per walker
     OPT_METROPOLIS_NO_SPLIT, // register sampler: always one thread per walker (never one thread per spin block)

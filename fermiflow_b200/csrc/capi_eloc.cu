@@ -7,33 +7,6 @@ using namespace ffc;
 
 namespace {
 
-// Barrier-synchronous sweep with fused phases (ff_eloc2.cuh eloc2_kernel).
-template <int SN, int SMU>
-int launch_eloc2(ff::FlowArgs& a, cudaStream_t st) {
-    constexpr ff::Eloc2Geom g = ff::eloc2_geom(SN, SMU != 0);
-    constexpr ff::Eloc2Launch q = ff::eloc2_launch(SN, SMU != 0);
-    a.D = g.D; a.NP = g.NP; a.P = g.P; a.DP = g.DP; a.NV = g.NV; a.NSV = g.NSV; a.grec = ff::kGRec;
-    a.off_G = g.off_G; a.off_AM = g.off_AM; a.off_u = g.off_u; a.off_kLx = g.off_kLx; a.off_part = g.off_part;
-    a.off_x0 = g.off_x0; a.off_sl = g.off_sl; a.wstride = g.wstride; a.W = 1;
-    const int need = ff::slater_scratch_size(a.n_up, a.n - a.n_up) + 2 * g.D + g.n * g.n + g.NP + 8;
-    // finale scratch: the two RK partial buffers plus J1 (dead after the last stage; eloc2_kernel re-zeroes it)
-    if (need > 3 * g.MAT) return FF_FALLBACK;  // the generic kernel takes over
-    constexpr int NI = FF_ELOC2_ILP;
-    const int common = ff::kTabDoubles + 6 * (ff::coef_rows2<NI>(a.H_eta) + ff::coef_rows2<NI>(a.H_mu)) + 2 * ((g.NP + 7) / 8) + 2;
-    size_t smem = (size_t)(common + g.wstride) * 8;
-    if ((long long)smem > dev_info().smem_optin) return FF_FALLBACK;
-    {   // what is left of this CTA's share of the SM mirrors the head of the eta table (96 bytes per node)
-        const DevInfo di = dev_info();
-        // ... without lowering the number of resident CTAs the register allocation aims at
-        const int occ = ff::eloc2_min_blocks(q.threads);
-        const long long share = (long long)di.smem_sm / occ - di.smem_reserved - 64;
-        const long long room = std::min<long long>(share, di.smem_optin) - (long long)smem;
-        a.rt_cache_nodes = (a.rt_eta != nullptr && room > 0) ? (int)std::min<long long>(room / (8 * ff::kRtCoef), 2048) : 0;
-        smem += (size_t)a.rt_cache_nodes * 8 * ff::kRtCoef;
-    }
-    return launch_flow_kernel(ff::eloc2_kernel<SN, SMU>, a, q.threads, smem, st);
-}
-
 // Geometry of the finale kernel's walker block: [state: y, L, gDelta, (Delta, lapDelta), J D8 x DP][Slater scratch,
 // g0, reduction buffer][M = J J^T][x0]
 int plan_finale(ff::FlowArgs& a, int W) {
@@ -96,19 +69,8 @@ int launch_finale(const ff::FlowArgs& a, const double* fin, int stride, cudaStre
     return 0;
 }
 
-// Register-resident sweeps (ff_eloc5.cuh eloc5_kernel: specialised owner / worker warps; ff_eloc4.cuh eloc4_kernel under
-// option "eloc_v4") + finale kernel.
-// eloc5_kernel takes the per-SM counters, eloc4_kernel does not
-inline void launch_sweep(void (*kernel)(const ff::FlowArgs, double*, int*), unsigned grid, int threads, size_t smem, cudaStream_t st,
-                         const ff::FlowArgs& a, double* fin, int* sm_count) {
-    kernel<<<grid, threads, smem, st>>>(a, fin, sm_count);
-}
-inline void launch_sweep(void (*kernel)(const ff::FlowArgs, double*), unsigned grid, int threads, size_t smem, cudaStream_t st,
-                         const ff::FlowArgs& a, double* fin, int*) {
-    kernel<<<grid, threads, smem, st>>>(a, fin);
-}
-template <class Kernel>
-int launch_eloc_reg(Kernel kernel, int threads, size_t smem, int fin_stride, ff::FlowArgs& a, cudaStream_t st) {
+// Register-resident sweep (ff_eloc5.cuh eloc5_kernel) + finale kernel.
+int launch_eloc_reg(void (*kernel)(const ff::FlowArgs, double*, int*), int threads, size_t smem, int fin_stride, ff::FlowArgs& a, cudaStream_t st) {
     const DevInfo di = dev_info();
     if (a.B < 1) return 0;
     if ((long long)smem > di.smem_optin) return FF_FALLBACK;
@@ -144,14 +106,9 @@ int launch_eloc_reg(Kernel kernel, int threads, size_t smem, int fin_stride, ff:
     const int carve = (int)std::min<long long>(100, ((long long)occ * ((long long)smem + di.smem_reserved) * 100 + di.smem_sm - 1) / di.smem_sm);
     FF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
     const long long grid = std::min<long long>(a.B, (long long)di.sms * occ);
-    launch_sweep(kernel, (unsigned)grid, threads, smem, st, a, fin, sm_count);
+    kernel<<<(unsigned)grid, threads, smem, st>>>(a, fin, sm_count);
     FF_LAUNCHED();
     return launch_finale(a, fin, fin_stride, st);
-}
-template <int SN, int SMU>
-int launch_eloc4(ff::FlowArgs& a, cudaStream_t st) {
-    constexpr ff::Eloc4Geom g = ff::eloc4_geom(SN, SMU != 0);
-    return launch_eloc_reg(ff::eloc4_kernel<SN, SMU>, g.threads, (size_t)g.total * 8, g.fin_stride, a, st);
 }
 template <int SN, int SMU>
 int launch_eloc5(ff::FlowArgs& a, cudaStream_t st) {
@@ -170,52 +127,35 @@ int launch_eloc5(ff::FlowArgs& a, cudaStream_t st) {
     return launch_eloc_reg(ff::eloc5_kernel<SN, SMU>, g.threads, smem, g.fin_stride, a, st);
 }
 
-// Statically specialised E_loc sweeps (ff_eloc4.cuh; ff_eloc2.cuh under option "eloc_v2" or without the Taylor tables) for the particle numbers of the BASELINE.json configs; anything
-// else, or "eloc_generic", runs the generic flow_kernel<MODE_ELOC>.
+// Statically specialised E_loc sweep (ff_eloc5.cuh) for the particle numbers it is instantiated for; anything else, or
+// "eloc_generic", runs the generic flow_kernel<MODE_ELOC>.  Without the Taylor tables ("no_table") every item of the
+// static sweep takes its direct-evaluation path.
 int try_eloc_static(ff::FlowArgs& a, cudaStream_t st) {
     if (opt(OPT_ELOC_GENERIC)) return FF_FALLBACK;
-    if (!opt(OPT_ELOC_V2) && a.rt_eta != nullptr) {
-        if (opt(OPT_ELOC_V4) && a.H_mu > 0) {
-            switch (a.n) {
-                case 20: return launch_eloc4<20, 1>(a, st);
-                case 12: return launch_eloc4<12, 1>(a, st);
-                case 6: return launch_eloc4<6, 1>(a, st);
-                default: break;
-            }
-        }
-        if (a.H_mu > 0) {
-            switch (a.n) {       // one walker per CTA; below 6 particles the generic sweep packs several walkers into a CTA
-                case 20: return launch_eloc5<20, 1>(a, st);
-                case 19: return launch_eloc5<19, 1>(a, st);
-                case 18: return launch_eloc5<18, 1>(a, st);
-                case 17: return launch_eloc5<17, 1>(a, st);
-                case 16: return launch_eloc5<16, 1>(a, st);
-                case 15: return launch_eloc5<15, 1>(a, st);
-                case 14: return launch_eloc5<14, 1>(a, st);
-                case 13: return launch_eloc5<13, 1>(a, st);
-                case 12: return launch_eloc5<12, 1>(a, st);
-                case 11: return launch_eloc5<11, 1>(a, st);
-                case 10: return launch_eloc5<10, 1>(a, st);
-                case 9: return launch_eloc5<9, 1>(a, st);
-                case 8: return launch_eloc5<8, 1>(a, st);
-                case 7: return launch_eloc5<7, 1>(a, st);
-                case 6: return launch_eloc5<6, 1>(a, st);
-                default: break;
-            }
-        } else {                 // reference drivers' --nomu: no one-body backflow
-            switch (a.n) {
-                case 20: return launch_eloc5<20, 0>(a, st);
-                case 12: return launch_eloc5<12, 0>(a, st);
-                case 6: return launch_eloc5<6, 0>(a, st);
-                default: break;
-            }
+    if (a.H_mu > 0) {
+        switch (a.n) {       // one walker per CTA; below 6 particles the generic sweep packs several walkers into a CTA
+            case 20: return launch_eloc5<20, 1>(a, st);
+            case 19: return launch_eloc5<19, 1>(a, st);
+            case 18: return launch_eloc5<18, 1>(a, st);
+            case 17: return launch_eloc5<17, 1>(a, st);
+            case 16: return launch_eloc5<16, 1>(a, st);
+            case 15: return launch_eloc5<15, 1>(a, st);
+            case 14: return launch_eloc5<14, 1>(a, st);
+            case 13: return launch_eloc5<13, 1>(a, st);
+            case 12: return launch_eloc5<12, 1>(a, st);
+            case 11: return launch_eloc5<11, 1>(a, st);
+            case 10: return launch_eloc5<10, 1>(a, st);
+            case 9: return launch_eloc5<9, 1>(a, st);
+            case 8: return launch_eloc5<8, 1>(a, st);
+            case 7: return launch_eloc5<7, 1>(a, st);
+            case 6: return launch_eloc5<6, 1>(a, st);
+            default: return FF_FALLBACK;
         }
     }
-    if (a.H_mu <= 0) return FF_FALLBACK;
-    switch (a.n) {
-        case 20: return launch_eloc2<20, 1>(a, st);
-        case 12: return launch_eloc2<12, 1>(a, st);
-        case 6: return launch_eloc2<6, 1>(a, st);
+    switch (a.n) {           // reference drivers' --nomu: no one-body backflow
+        case 20: return launch_eloc5<20, 0>(a, st);
+        case 12: return launch_eloc5<12, 0>(a, st);
+        case 6: return launch_eloc5<6, 0>(a, st);
         default: return FF_FALLBACK;
     }
 }
@@ -224,14 +164,6 @@ int try_eloc_static(ff::FlowArgs& a, cudaStream_t st) {
 
 extern "C" {
 
-#ifdef FF_E4_TIMING
-int ff_debug_e4_cycles(unsigned long long* out, int reset) {
-    cudaDeviceSynchronize();
-    cudaMemcpyFromSymbol(out, ff::g_e4_cyc, sizeof(unsigned long long) * 64);
-    if (reset) { unsigned long long z[64] = {}; cudaMemcpyToSymbol(ff::g_e4_cyc, z, sizeof z); }
-    return 0;
-}
-#endif
 #ifdef FF_E5_TIMING
 int ff_debug_e5_cycles(unsigned long long* out, int reset) {
     cudaDeviceSynchronize();

@@ -1,13 +1,21 @@
-// E_loc sweep, register-resident Jacobian with specialised warps (eloc5_kernel); finale in eloc_finale_kernel.
+// E_loc sweep, register-resident Jacobian with specialised warps (eloc5_kernel).
 //
 // Same mathematics as flow_body<MODE_ELOC> (ff_flow.cuh; replaces utils.py:44-65 y_grad_laplacian + VMC.py:41-55 on
 // top of flow.py:42-56 / equivariant_funs.py:17-102): the forward-mode state (y, J, L, gDelta, Delta, lapDelta) of ONE
-// walker per CTA is integrated with the 3/8-rule RK4 (torchdiffeq rk4_alt_step_func).  As in eloc4_kernel the Jacobian
-// is carried transposed, K = J^T, in the accumulator layout of mma.m8n8k4 in the registers of NB "owner" warps (those
-// registers are the A operand of K' = K A, see ff_eloc4.cuh), its RK partials in shared memory.  What is different:
+// walker per CTA is integrated with the 3/8-rule RK4 (torchdiffeq rk4_alt_step_func).  The kernel writes the final
+// state to global memory (fin_stride doubles per walker); the base-distribution end of the sweep (Slater matrices,
+// <H0, J J^T>, E_loc) runs from there in a separate kernel at full occupancy (ff_finale.cuh).
 //
+//   * The Jacobian is carried TRANSPOSED, K = J^T, and its derivative is K' = K A (A = dv/dy is symmetric).
+//     Owner warp cb < NB owns the 8 rows [8 cb, 8 cb + 8) of K in the accumulator layout of mma.m8n8k4 (lane (g, t) holds
+//     K[8 cb + g][8 rb + 2 t + e], rb < NB, e < 2).  The contraction index of a matrix product may be permuted freely,
+//     so those registers ARE the A operand of the next product: k-step (rb, e) pairs K[.][8 rb + 2 t + e] with row
+//     8 rb + 2 t + e of A.  K never leaves the registers of its owner except as the shared copy the Gram matrix is
+//     formed from; its RK partials are in shared memory (see "RK in the accumulators" below).
+//   * A is stored with the rows of every block of 8 in the order 0 2 4 6 1 3 5 7 (a_row), which makes the owners'
+//     B-operand loads (rows 2 t + e of a block) bank-conflict free at the row pitch D8 + 4.
 //   * The CTA has NB owner warps and WW = ceil(P / 32) "worker" warps (N = 20: 5 + 7 = 384 threads at 80 registers,
-//     two CTAs = 24 warps per SM instead of 16).  Owners never evaluate items, workers never hold K: neither side
+//     two CTAs = 24 warps per SM).  Owners never evaluate items, workers never hold K: neither side
 //     carries the other's registers.
 //   * Per RK stage both kinds of warps have work in both phases, and they hand data over point to point (named barriers,
 //     see below) instead of meeting at CTA-wide barriers:
@@ -22,9 +30,82 @@
 //                 overlaps the owners' tensor-core work.
 //   * Nothing lags: M of stage s is formed in phase 1 of stage s and consumed in its phase 2.
 #pragma once
-#include "ff_eloc4.cuh"
+#include "ff_finale.cuh"
 
 namespace ff {
+
+// One RK sub-stage of the two-partial 3/8 rule for a scalar element.
+__device__ __forceinline__ double rk_elem(int sub, double s, double hk, double& B, double& C) {
+    if (sub == 0) { B = fma(hk, -1.0 / 3.0, s); C = fma(hk, 0.125, s); return fma(hk, 1.0 / 3.0, s); }
+    if (sub == 1) { const double b = B; B = (2.0 * s - b) - hk; C = fma(hk, 0.375, C); return b + hk; }
+    if (sub == 2) { C = fma(hk, 0.375, C); return B + hk; }
+    return fma(hk, 0.125, C);
+}
+
+// Ordered shared-memory load / tensor-core product (volatile asm keeps the program order): ptxas otherwise sinks
+// every operand load right in front of its DMMA and each product waits ~30 cycles for its own LDS.
+__device__ __forceinline__ double lds_ordered(const double* p) {
+    double v;
+    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"((unsigned)__cvta_generic_to_shared(p)));
+    return v;
+}
+__device__ __forceinline__ void dmma_ordered(double& c0, double& c1, double a, double b) {
+    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
+                 : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
+}
+
+// physical row of A that holds logical row r: rows of each block of 8 in the order 0 2 4 6 1 3 5 7
+__host__ __device__ constexpr int a_row(int r) { return (r & ~7) | ((r & 1) << 2) | ((r & 7) >> 1); }
+
+__device__ __forceinline__ void named_bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
+__device__ __forceinline__ void named_bar_arrive(int id, int count) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(count) : "memory"); }
+
+// Direct evaluation of f(d) = sum_h w2_h sigmoid(w1_h d + b1_h) and three derivatives from the parameters in global
+// memory (MLP.py:30-45): only for items the certified table does not cover (d beyond its range, invalid table).
+__device__ __noinline__ void radial_direct_global(const double* __restrict__ w1, const double* __restrict__ b1,
+                                                  const double* __restrict__ w2, int H, double d, double* f) {
+    double f0 = 0.0, f1 = 0.0, f2 = 0.0, f3 = 0.0;
+    for (int h = 0; h < H; ++h) {
+        const double w = __ldg(w1 + h), c = __ldg(w2 + h);
+        const double s0 = 1.0 / (1.0 + exp(-fma(w, d, __ldg(b1 + h))));
+        const double s1 = fma(-s0, s0, s0);
+        const double s2 = s1 * fma(-2.0, s0, 1.0);
+        const double s3 = s1 * fma(-6.0, s1, 1.0);
+        double cw = c;
+        f0 = fma(cw, s0, f0); cw *= w;
+        f1 = fma(cw, s1, f1); cw *= w;
+        f2 = fma(cw, s2, f2); cw *= w;
+        f3 = fma(cw, s3, f3);
+    }
+    f[0] = f0; f[1] = f1; f[2] = f2; f[3] = f3;
+}
+
+// Per-particle sum of component c < 3 of the three-component records G2[p][3] of the M-contractions.  Partner slot
+// k < i is pair (k, i) at record K_k + i (K_k a compile-time constant), slot k >= i is pair (i, k + 1) at record
+// U_i + k + 1.  Components 0, 1 change sign with the orientation of the pair, component 2 holds the pair total (halved
+// here); the one-body item of the particle is added last.
+template <int SN, int SMU>
+__device__ __forceinline__ double gather3(const double* __restrict__ G2, int i, int c) {
+    constexpr int n = SN, NP = SN * (SN - 1) / 2;
+    const double* pL = G2 + 3 * i + c;                                             // + 3 * (K_k - k - 1)
+    const double* pU = G2 + 3 * (i * (2 * n - i - 1) / 2 - i - 1) + c;             // + 3 * (k + 1)
+    double lo0 = 0.0, lo1 = 0.0, up0 = 0.0, up1 = 0.0;
+#pragma unroll
+    for (int k = 0; k < n - 1; ++k) {
+        if (k < i) { const double v = pL[3 * (k * (2 * n - k - 1) / 2 - k - 1)]; if (k & 1) lo1 += v; else lo0 += v; }
+        else { const double v = pU[3 * (k + 1)]; if (k & 1) up1 += v; else up0 += v; }
+    }
+    const double lo = lo0 + lo1, up = up0 + up1;
+    double acc = c < 2 ? up - lo : 0.5 * (up + lo);
+    if (SMU != 0) acc += G2[3 * (NP + i) + c];
+    return acc;
+}
+
+// Opaque copy of a lane-dependent index, taken once per RK stage: everything derived from it (dozens of shared-memory
+// addresses of the gathers, the contractions and the tensor-core fragments) is then recomputed inside the stage with
+// a handful of integer instructions instead of being hoisted out of the stage loop, where those loop invariants filled
+// the register file and spilled to local memory (first version: 120 M local loads per 9472 walkers).
+__device__ __forceinline__ int stage_local(int v) { asm volatile("" : "+r"(v)); return v; }
 
 struct Eloc5Geom {
     int n, D, D8, DP, NP, P, NB, ntri, MAT, RP, RMAT;

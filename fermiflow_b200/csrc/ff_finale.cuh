@@ -1,6 +1,7 @@
-// Base-distribution end of the E_loc sweep, ONE WARP PER WALKER (eloc_finale_warp_kernel).
+// Base-distribution end of the E_loc sweep, ONE WARP PER WALKER (eloc_finale_warp_kernel), and its CTA-synchronous
+// counterpart (eloc_finale_kernel: option "finale_cta", and the particle numbers the warp kernel is not instantiated for).
 //
-// Input: the final state of the forward-mode sweep in global memory (eloc4_kernel / eloc5_kernel): y = z = flow^-1(x),
+// Input: the final state of the forward-mode sweep in global memory (eloc5_kernel): y = z = flow^-1(x),
 // L_b = sum_a d2y_b / dx_a^2, gDelta, Delta, lapDelta and J = dy/dx (row-major).  At z the kernel evaluates
 //     log p0 = 2 (log|det Phi_up| + log|det Phi_dn|)                                          (base_dist.py:48-56)
 //     g0 = 2 B^a_ii,   H0_{ia,jb} = 2 (delta_ij C^{ab}_i - B^a_ij B^b_ji)                     (Jacobi's formula; slater.py:4-156)
@@ -11,8 +12,8 @@
 // shuffles, no CTA barrier).  M = J J^T never touches shared memory: the warp forms the upper block triangle on the tensor
 // cores with the operand fragments straight from global memory (every 8 x 4 fragment is eight full 32-byte sectors; the A
 // and the B operand of a block are the same kind of fragment) and contracts each accumulator element with H0 in place.
-// The CTA-synchronous finale it replaces (eloc_finale, ff_flow.cuh) spent 5.7 ms per 65536 walkers at N = 20 between its
-// barriers.
+// The CTA-synchronous finale (eloc_finale, ff_flow.cuh, run by eloc_finale_kernel) spent 5.7 ms per 65536 walkers at
+// N = 20 between its barriers.
 #pragma once
 #include "ff_flow.cuh"
 
@@ -240,6 +241,42 @@ __global__ void __launch_bounds__(128) eloc_finale_warp_kernel(const FlowArgs a,
             if (a.eloc) a.eloc[b] = kin + pot;
         }
         __syncwarp();
+    }
+}
+
+// Base-distribution end of the sweep for W walkers per CTA from the final states in global memory (eloc_finale,
+// ff_flow.cuh): Slater matrices and inverse at z, <H0, J J^T>, grad, E_loc.  Generic in n (run-time geometry in
+// FlowArgs: D, DP, NP, W, wstride, off_sl, off_AM, off_x0 as plan_finale sets them).
+__global__ void __launch_bounds__(256) eloc_finale_kernel(const FlowArgs a, const double* __restrict__ fin, int fin_stride) {
+    extern __shared__ __align__(16) double smem[];
+    const int tid = threadIdx.x, T = blockDim.x;
+    const int n = a.n, D = a.D, DP = a.DP, NP = a.NP, W = a.W, D8 = (D + 7) & ~7;
+    unsigned char* pair_i = reinterpret_cast<unsigned char*>(smem);
+    unsigned char* pair_j = pair_i + ((NP + 7) & ~7);
+    double* wbase = smem + 2 * ((NP + 7) / 8);
+    if ((wbase - smem) & 1) wbase += 1;
+    for (int p = tid; p < NP; p += T) {
+        int i = 0, rem = p;
+        while (rem >= n - 1 - i) { rem -= n - 1 - i; ++i; }
+        pair_i[p] = (unsigned char)i;
+        pair_j[p] = (unsigned char)(i + 1 + rem);
+    }
+    const int oJ = 3 * D + 2;
+    for (long long base = (long long)blockIdx.x * W; base < a.B; base += (long long)gridDim.x * W) {
+        __syncthreads();
+        for (int w = 0; w < W; ++w) {
+            double* Sw = wbase + (size_t)w * a.wstride;
+            const long long b = min(base + w, a.B - 1);          // padding walkers repeat the last one (results not stored)
+            const double* F = fin + (size_t)b * fin_stride;
+            for (int e = tid; e < oJ; e += T) Sw[e] = F[e];
+            for (int e = tid; e < D8 * DP; e += T) {
+                const int r = e / DP, c = e - r * DP;
+                Sw[oJ + e] = (r < D && c < D) ? F[oJ + r * D + c] : 0.0;
+            }
+            for (int e = tid; e < D; e += T) (Sw + a.off_x0)[e] = a.x_in[b * D + e];
+        }
+        __syncthreads();
+        eloc_finale(a, base, wbase, pair_i, pair_j);
     }
 }
 

@@ -194,27 +194,8 @@ __device__ __forceinline__ bool radial_table_eval(const RtHeader& T, double d, d
     radial_horner<ORD>(c, t, f);
     return true;
 }
-// The same with the first `ncache` nodes of the table mirrored in shared memory (`cache`, 16-byte aligned).
-template <int ORD>
-__device__ __forceinline__ bool radial_table_eval_cached(const RtHeader& T, const double* cache, int ncache, double d, double (&f)[4]) {
-    const double kf = rint(d * T.inv_delta);
-    if (T.coef == nullptr || !(kf < (double)T.n_nodes) || !(kf >= 0.0)) return false;
-    const double t = fma(-kf, T.delta, d);
-    const int k = (int)kf;
-    double c[kRtCoef];
-    if (k < ncache) {
-        const double2* c2 = reinterpret_cast<const double2*>(cache + (size_t)k * kRtCoef);
-#pragma unroll
-        for (int q = 0; q < kRtCoef / 2; ++q) { const double2 v = c2[q]; c[2 * q] = v.x; c[2 * q + 1] = v.y; }
-    } else {
-        const double2* c2 = reinterpret_cast<const double2*>(T.coef + (size_t)k * kRtCoef);
-#pragma unroll
-        for (int q = 0; q < kRtCoef / 2; ++q) { const double2 v = __ldg(c2 + q); c[2 * q] = v.x; c[2 * q + 1] = v.y; }
-    }
-    radial_horner<ORD>(c, t, f);
-    return true;
-}
-// The same with a COEFFICIENT-MAJOR mirror (cache[q * ncache + k]): lanes that look up different nodes read
+// The same with the first `ncache` nodes of the table mirrored in shared memory, COEFFICIENT-MAJOR
+// (cache[q * ncache + k]): lanes that look up different nodes read
 // neighbouring words of one coefficient row instead of rows 96 bytes apart (4 bank groups) -- for kernels whose lanes
 // all look up at once (one warp per walker).
 template <int ORD>

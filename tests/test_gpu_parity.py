@@ -224,7 +224,7 @@ CASES = [  # nup, ndown, H_eta, H_mu, nsteps, batch
     (3, 0, 8, 0, 8, 7),
     (1, 1, 5, 5, 4, 3),
     (6, 6, 16, 16, 8, 9),
-    (12, 0, 10, 10, 4, 6),      # spin-polarised N = 12 (BASELINE config 3): finale scratch extends into J1
+    (12, 0, 10, 10, 4, 6),      # spin-polarised N = 12 (BASELINE config 3): one 12 x 12 Slater block in the finale
     (5, 2, 50, 50, 4, 4),
     (10, 10, 50, 50, 16, 3),    # the benchmark configuration (BASELINE configs[2]): eloc5_kernel<20,1>, warp finale, warp adjoint, binned gradient
     (3, 3, 12, 0, 8, 6),        # --nomu on the register-resident sweep (eloc5_kernel<6,0>)
@@ -531,17 +531,17 @@ def test_warp_per_walker_flow_vs_oracle(dev, O):
         close(p.grad.reshape(-1), gr.reshape(-1), 1e-9, 1e-13)
 
 
-def _n20_model(dev, nsteps=8, H=50):
+def _dot_model(dev, nsteps=8, H=50, nup=10, ndn=10):
     from fermiflow_b200 import Backflow, CNF, HO2D, FreeFermion, GSVMC, HO, CoulombPairPotential
     eta, mu = rand_mlp(H, 21, 0.02, dev), rand_mlp(H, 22, 0.02, dev)
     cnf = CNF(Backflow(eta, mu=mu), (0.0, 1.0), nsteps=nsteps)
-    return GSVMC(10, 10, HO2D(), FreeFermion(dev), cnf, CoulombPairPotential(2.0), sp_potential=HO()).to(dev)
+    return GSVMC(nup, ndn, HO2D(), FreeFermion(dev), cnf, CoulombPairPotential(2.0), sp_potential=HO()).to(dev)
 
 
 def test_flow_kernel_variants_agree_full_size(dev):
     """N = 20: one-warp-per-walker sweeps against the CTA-synchronous flow_kernel (option flow_cta)
     and its 128-register build (flow_big) on the same walkers."""
-    model = _n20_model(dev)
+    model = _dot_model(dev)
     z, _ = model.sample((777,))
     outs = []
     for env in (dict(flow_cta=0, flow_big=0), dict(flow_cta=1, flow_big=0), dict(flow_cta=1, flow_big=1)):
@@ -555,16 +555,17 @@ def test_flow_kernel_variants_agree_full_size(dev):
         close(o[2], outs[0][2], 1e-12, 1e-14)
 
 
-@pytest.mark.parametrize("B", [1, 2, 297, 1500])
-def test_eloc_kernel_variants_agree_full_size(dev, B):
-    """N = 20: the default sweep (eloc5_kernel: register-resident Jacobian, specialised warps) against the generic
-    flow_kernel<MODE_ELOC> (option eloc_generic), with the Taylor tables and with direct evaluation of every hidden unit
-    (no_table: eloc2_kernel), against its predecessors (eloc_v4, eloc_v2) and without the table mirror (no_rt_cache)."""
-    model = _n20_model(dev, nsteps=4)
+@pytest.mark.parametrize("nup,ndn,B", [(10, 10, 1), (10, 10, 2), (10, 10, 297), (10, 10, 1500), (7, 6, 297), (3, 3, 297)])
+def test_eloc_kernel_variants_agree_full_size(dev, nup, ndn, B):
+    """N = 20, 13 and 6 at H = 50: the default sweep (eloc5_kernel: register-resident Jacobian, specialised warps)
+    against the generic flow_kernel<MODE_ELOC> (option eloc_generic), each with the Taylor tables and with direct
+    evaluation of every hidden unit (no_table: eloc5_kernel evaluates every item directly), against eloc5_kernel
+    without the table mirror (no_rt_cache) and with the CTA-synchronous finale (finale_cta)."""
+    model = _dot_model(dev, nsteps=4, nup=nup, ndn=ndn)
     _, x = model.sample((B,))
     res = []
     for env in (dict(eloc_generic=0, no_table=0), dict(eloc_generic=1, no_table=0), dict(eloc_generic=0, no_table=1),
-                dict(eloc_generic=1, no_table=1), dict(eloc_v4=1), dict(eloc_v2=1), dict(no_rt_cache=1), dict(finale_cta=1)):
+                dict(eloc_generic=1, no_table=1), dict(no_rt_cache=1), dict(finale_cta=1)):
         with _opts(**env):
             res.append(model.local_energy(x, stash=True))
     for r in res[1:]:
@@ -865,9 +866,8 @@ def test_calibrate_nsteps_meets_the_reference_tolerance(dev, O):
 
 
 def test_eloc_static_kernel_spin_polarised_many_walkers_per_cta(dev):
-    """Spin-polarised N = 12 (BASELINE config 3): the statically specialised sweep keeps its finale scratch partly
-    in the dead J1 buffer and re-zeroes it; with ~7 walkers per CTA it must agree with the generic kernel
-    (option eloc_generic), walker by walker."""
+    """Spin-polarised N = 12 (BASELINE config 3): eloc5_kernel<12,1> with one 12-particle spin block, 2101 walkers
+    (each CTA runs several in turn), against the generic kernel (option eloc_generic), walker by walker."""
     from fermiflow_b200 import Backflow, CNF, HO2D, FreeFermion, GSVMC, HO, CoulombPairPotential
     cnf = CNF(Backflow(rand_mlp(20, 5, 0.03, dev), mu=rand_mlp(20, 6, 0.03, dev)), (0.0, 1.0), nsteps=3)
     model = GSVMC(12, 0, HO2D(), FreeFermion(dev), cnf, CoulombPairPotential(8.0), sp_potential=HO()).to(dev)
