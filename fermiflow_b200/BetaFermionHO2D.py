@@ -12,6 +12,7 @@ from .VMC import BetaVMC
 from .base_dist import FreeFermion
 from .equivariant_funs import Backflow
 from .flow import CNF
+from .observables import sample_density
 from .orbitals import HO2D
 from .potentials import HO, CoulombPairPotential
 
@@ -34,6 +35,10 @@ def main(argv=None):
     p.add_argument("--iternum", type=int, default=1000)
     p.add_argument("--batch", type=int, default=8000)
     p.add_argument("--lr", type=float, default=1e-2)
+    p.add_argument("--density", metavar="FILE", help="after training, save the density and pair correlations of "
+                   "freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.DensityEstimator)")
+    p.add_argument("--density-batches", type=int, default=16, help="batches of --batch walkers for --density")
+    p.add_argument("--density-extent", type=float, default=6.0, help="half-width of the density grids")
     args = p.parse_args(argv)
 
     device = torch.device("cuda:%d" % args.cuda)
@@ -60,6 +65,8 @@ def main(argv=None):
         print("iter: %03d" % i, "F:", model.F, "F_std:", model.F_std, "E:", model.E, "E_std:", model.E_std,
               "S:", model.S, "S_analytical:", model.S_analytical,
               "Instant speed (hours per 100 iters):", (time.time() - start) * 100 / 3600)
+    if args.density:
+        sample_density(model, args.nup, args.ndown, args.batch, args.density_batches, args.density_extent, args.density)
     return history
 
 

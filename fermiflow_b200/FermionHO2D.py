@@ -13,6 +13,7 @@ from .VMC import GSVMC
 from .base_dist import FreeFermion
 from .equivariant_funs import Backflow
 from .flow import CNF
+from .observables import sample_density
 from .orbitals import HO2D
 from .potentials import HO, CoulombPairPotential
 
@@ -32,6 +33,10 @@ def main(argv=None):
     p.add_argument("--iternum", type=int, default=1000)
     p.add_argument("--batch", type=int, default=8000)
     p.add_argument("--lr", type=float, default=1e-2)
+    p.add_argument("--density", metavar="FILE", help="after training, save the density and pair correlations of "
+                   "freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.DensityEstimator)")
+    p.add_argument("--density-batches", type=int, default=16, help="batches of --batch walkers for --density")
+    p.add_argument("--density-extent", type=float, default=6.0, help="half-width of the density grids")
     args = p.parse_args(argv)
 
     device = torch.device("cuda:%d" % args.cuda)
@@ -56,6 +61,8 @@ def main(argv=None):
         history.append((model.E, model.E_std))
         print("iter: %03d" % i, "E:", model.E, "E_std:", model.E_std,
               "Instant speed (hours per 100 iters):", (time.time() - start) * 100 / 3600)
+    if args.density:
+        sample_density(model, args.nup, args.ndown, args.batch, args.density_batches, args.density_extent, args.density)
     return history
 
 

@@ -20,6 +20,11 @@ class FFModel(C.Structure):
                 ("t0", C.c_double), ("t1", C.c_double), ("nsteps", C.c_int)]
 
 
+class FFObsGrid(C.Structure):
+    _fields_ = [("extent", C.c_double), ("n_xy", C.c_int), ("n_rot", C.c_int),
+                ("r_max", C.c_double), ("n_r", C.c_int)]
+
+
 _lib = None
 _P, _LL, _I, _D = C.c_void_p, C.c_longlong, C.c_int, C.c_double
 _M = C.POINTER(FFModel)
@@ -44,6 +49,7 @@ SIGNATURES = {
     "ff_backward_work_size": ([_M, _LL, C.POINTER(_LL)], C.c_int),
     "ff_potential": ([_P, _LL, _I, _D, _I, _P, _P], C.c_int),
     "ff_occupation_sample": ([_P, _I, _P, _LL, _P, _P, _P, _P], C.c_int),
+    "ff_observables": ([_P, _LL, _I, _I, C.POINTER(FFObsGrid), _P, _LL, _P], C.c_int),
     "ff_fp64_peak": ([_I, C.POINTER(_D), _P], C.c_int),
     "ff_fp64_mma_peak": ([_I, C.POINTER(_D), _P], C.c_int),
 }

@@ -6,6 +6,7 @@
 #include "ff_pgrad_binned.cuh"
 #include "ff_misc.cuh"
 #include "ff_metro_reg.cuh"
+#include "ff_observables.cuh"
 
 namespace ffc {
 

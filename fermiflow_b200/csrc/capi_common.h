@@ -1,6 +1,7 @@
 // Host-side plumbing shared by the translation units of the C ABI (capi.cu, capi_eloc.cu): error reporting,
 // option switches, launch counter, device attributes.  Definitions live in capi.cu.
 #pragma once
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>

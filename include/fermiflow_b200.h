@@ -132,6 +132,34 @@ int ff_potential(const double* x, long long B, int n, double Z, int harmonic, do
 int ff_occupation_sample(const double* logits, int S, const double* uniforms, long long B,
                          int* state, int* counts, double* cdf_work, void* stream);
 
+/* Histograms of sampled walkers for the one-body density and the pair correlations (no reference counterpart: the
+ * reference reports energies only).  x [B][n_up+n_dn][2], particle i < n_up spin-up; 8-byte alignment suffices.
+ * Four sections, each switched off by 0 bins:
+ *   density     particles i on the square grid [-extent, extent)^2, n_xy x n_xy cells, channels up, down
+ *   radial      |r_i| over [0, r_max), n_r bins, channels up, down
+ *   separation  |r_i - r_j| of the pairs i < j over [0, r_max), n_r bins, channels up-up, down-down, up-down
+ *   rotated     ordered pairs i != j in the frame rotated so that particle i lies on the +x axis,
+ *               u = (x_i x_j + y_i y_j) / |r_i|, w = (x_i y_j - y_i x_j) / |r_i|, on [-extent, extent)^2 with
+ *               n_rot x n_rot cells, channels same spin, opposite spin
+ * Binning rule: s = nbins / (hi - lo) in double, bin k = floor((v - lo) * s) with every product and sum rounded
+ * separately (no FMA); k < 0, k >= nbins, a non-finite v and, in the rotated section, |r_i| == 0 count in the
+ * section's per-channel outside counter instead.
+ * Layout of counts (n_counts = 2 n_xy^2 + 2 n_r + 3 n_r + 2 n_rot^2 + 9):
+ *   [2][n_xy][n_xy] density (index [ch][ix][iy]), [2][n_r] radial, [3][n_r] separation, [2][n_rot][n_rot] rotated
+ *   (index [ch][iu][iw]), then the 9 outside counters in the same order: density up, down, radial up, down,
+ *   separation up-up, down-down, up-down, rotated same, opposite.
+ * ACCUMULATES into counts (the caller zeroes them); the counts are exact integers, independent of the order of
+ * execution.  B == 0 is a no-op.  -1 for bad particle numbers, B < 0, null pointers with B > 0, a non-positive extent
+ * or r_max of an enabled section, negative bin counts, n_counts not equal to the layout size, or (B > 0) a section
+ * whose bins do not fit in the shared memory of one block (a 128 x 128 density takes 128 KB and fits; sections that do
+ * not fit together are counted by one launch each). */
+typedef struct ff_obs_grid {
+    double extent; int n_xy; int n_rot;     /* square grids over [-extent, extent)^2; 0 cells: section off */
+    double r_max;  int n_r;                 /* radial and separation bins over [0, r_max); 0: off          */
+} ff_obs_grid;
+int ff_observables(const double* x, long long B, int n_up, int n_dn, const ff_obs_grid* g,
+                   unsigned long long* counts, long long n_counts, void* stream);
+
 /* Raw FP64 FMA throughput of the device (roofline denominator): runs `iters` dependent
  * DFMA chains on every SM and returns the achieved FLOP/s in *flops_host. */
 int ff_fp64_peak(int iters, double* flops_host, void* stream);
