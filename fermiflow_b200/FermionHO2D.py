@@ -13,7 +13,7 @@ from .VMC import GSVMC
 from .base_dist import FreeFermion
 from .equivariant_funs import Backflow
 from .flow import CNF
-from .observables import sample_density
+from .observables import sample_density, sample_momentum
 from .orbitals import HO2D
 from .potentials import HO, CoulombPairPotential
 
@@ -37,6 +37,10 @@ def main(argv=None):
                    "freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.DensityEstimator)")
     p.add_argument("--density-batches", type=int, default=16, help="batches of --batch walkers for --density")
     p.add_argument("--density-extent", type=float, default=6.0, help="half-width of the density grids")
+    p.add_argument("--momentum", metavar="FILE", help="after training, save the momentum distribution and one-body "
+                   "coherence of freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.MomentumEstimator)")
+    p.add_argument("--momentum-batches", type=int, default=16, help="batches of --batch walkers for --momentum")
+    p.add_argument("--momentum-kmax", type=float, default=4.0, help="half-width of the momentum grid")
     args = p.parse_args(argv)
 
     device = torch.device("cuda:%d" % args.cuda)
@@ -63,6 +67,8 @@ def main(argv=None):
               "Instant speed (hours per 100 iters):", (time.time() - start) * 100 / 3600)
     if args.density:
         sample_density(model, args.nup, args.ndown, args.batch, args.density_batches, args.density_extent, args.density)
+    if args.momentum:
+        sample_momentum(model, args.nup, args.ndown, args.batch, args.momentum_batches, args.momentum_kmax, args.momentum)
     return history
 
 

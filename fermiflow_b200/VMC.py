@@ -12,6 +12,7 @@ Walkers are independent Markov chains: under torch.distributed each rank works o
 `batch` walkers and only the energy moments and the few-KB parameter gradient are
 all-reduced (allreduce_gradients()).
 """
+import ctypes as C
 from collections import Counter
 
 import torch
@@ -74,6 +75,31 @@ class _LogpFromSweep(torch.autograd.Function):
         _, gparams = _backward_through_flow(ctx.owner.cnf, res.model, res.stash, B, g0, -g, False)
         res.stash = None            # 22 GB at 65536 walkers, N = 20: free it now, not when the graph dies
         return (None, None, None, None, None, None, *gparams)
+
+
+def _wavefunction_ratio(cnf, x, orb, walker_state, n_up, particle, disp):
+    """psi(x_b with r_i -> r_i + s) / psi(x_b) for every record (b, m), i = particle[b, m], s = disp[b, m], with the
+    sign of the Slater determinants (C ABI ff_wavefunction_ratio).  x [B, n, 2], particle integer [B, M], disp
+    [B, M, 2], all on the device; returns ratio [B, M].  A particle index outside [0, n) gives NaN."""
+    x = x.detach().contiguous()
+    if x.dim() != 3 or x.shape[-1] != 2:
+        raise ValueError("x must be [B, n, 2], got %s" % (tuple(x.shape),))
+    B, n, _ = x.shape
+    if particle.dim() != 2 or particle.shape[0] != B or tuple(disp.shape) != (B, particle.shape[1], 2):
+        raise ValueError("particle must be [B, M] and disp [B, M, 2] for B = %d walkers, got %s and %s"
+                         % (B, tuple(particle.shape), tuple(disp.shape)))
+    M = particle.shape[1]
+    p32 = particle.to(torch.int32).contiguous()
+    disp = disp.detach().contiguous()
+    model = cnf._model(n, n_up=n_up)
+    nw = C.c_longlong()
+    L.check(L.lib().ff_wavefunction_ratio_work_size(C.byref(model), B, M, C.byref(nw)))
+    work = torch.empty(nw.value, dtype=torch.float64, device=x.device)
+    ratio = torch.empty(B, M, dtype=torch.float64, device=x.device)
+    L.check(L.lib().ff_wavefunction_ratio(C.byref(model), L.ptr(x), B, L.ptr(orb, torch.int32),
+                                          L.ptr(walker_state, torch.int32) if walker_state is not None else None,
+                                          M, L.ptr(p32, torch.int32), L.ptr(disp), L.ptr(ratio), L.ptr(work), L.stream()))
+    return ratio
 
 
 def _multi_rank():
@@ -177,6 +203,11 @@ class GSVMC(_VMCBase):
         """log p, grad, laplacian, kinetic, potential, E_loc at x (VMC.py:44-55)."""
         res = eloc_sweep(self.cnf, x, self._orb(x.device), None, self.nup, self._Z, self._harmonic, stash=stash)
         return _add_external_potentials(self, res, x)
+
+    def wavefunction_ratio(self, x, particle, disp):
+        """psi(x with r_i -> r_i + s) / psi(x) per record, sign included: x [B, n, 2], particle [B, M] (i),
+        disp [B, M, 2] (s) -> ratio [B, M] (fermiflow_b200.observables.MomentumEstimator uses it)."""
+        return _wavefunction_ratio(self.cnf, x, self._orb(x.device), None, self.nup, particle, disp)
 
     def forward(self, batch):                                         # VMC.py:41-61
         _, x = self.sample((batch,))
@@ -285,6 +316,16 @@ class BetaVMC(_VMCBase):
         z, delta_logp = self.cnf.delta_logp(x, params_require_grad=params_require_grad)
         log_prob_z = _FreeFermionLogp.apply(z, self._state_table(x.device), self.state_indices, self.nup, self.ndown)
         return log_prob_z - delta_logp
+
+    def wavefunction_ratio(self, x, particle, disp, walker_state=None):
+        """GSVMC.wavefunction_ratio with each walker's own occupation row: walker_state (int [B]) defaults to the
+        state_indices of the last sample()."""
+        ws = getattr(self, "state_indices", None) if walker_state is None else walker_state
+        if ws is None or ws.shape != (x.shape[0],):
+            raise ValueError("walker_state must hold one state index per walker (%d), got %s"
+                             % (x.shape[0], None if ws is None else tuple(ws.shape)))
+        return _wavefunction_ratio(self.cnf, x, self._state_table(x.device), ws.to(torch.int32).contiguous(), self.nup,
+                                   particle, disp)
 
     def forward(self, batch):                                          # VMC.py:120-171
         _, x = self.sample((batch,))

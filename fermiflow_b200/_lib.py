@@ -25,6 +25,11 @@ class FFObsGrid(C.Structure):
                 ("r_max", C.c_double), ("n_r", C.c_int)]
 
 
+class FFMomGrid(C.Structure):
+    _fields_ = [("k_max", C.c_double), ("n_k", C.c_int), ("n_kr", C.c_int),
+                ("s_max", C.c_double), ("n_s", C.c_int)]
+
+
 _lib = None
 _P, _LL, _I, _D = C.c_void_p, C.c_longlong, C.c_int, C.c_double
 _M = C.POINTER(FFModel)
@@ -50,6 +55,9 @@ SIGNATURES = {
     "ff_potential": ([_P, _LL, _I, _D, _I, _P, _P], C.c_int),
     "ff_occupation_sample": ([_P, _I, _P, _LL, _P, _P, _P, _P], C.c_int),
     "ff_observables": ([_P, _LL, _I, _I, C.POINTER(FFObsGrid), _P, _LL, _P], C.c_int),
+    "ff_wavefunction_ratio_work_size": ([_M, _LL, _I, C.POINTER(_LL)], C.c_int),
+    "ff_wavefunction_ratio": ([_M, _P, _LL, _P, _P, _I, _P, _P, _P, _P, _P], C.c_int),
+    "ff_momentum_accumulate": ([_P, _P, _P, _LL, _I, C.POINTER(FFMomGrid), _P, _LL, _P], C.c_int),
     "ff_fp64_peak": ([_I, C.POINTER(_D), _P], C.c_int),
     "ff_fp64_mma_peak": ([_I, C.POINTER(_D), _P], C.c_int),
 }

@@ -7,6 +7,7 @@
 #include "ff_misc.cuh"
 #include "ff_metro_reg.cuh"
 #include "ff_observables.cuh"
+#include "ff_momentum.cuh"
 
 namespace ffc {
 

@@ -95,9 +95,11 @@ struct SlaterArgs {
     double scale;
     double *logabs, *grad, *lap;
     int W, wstride;       // doubles per walker: D + scratch + n*n
+    double* sign;         // [B] sign(det Phi_up det Phi_dn), written by the SIGN instantiations only (+1 for an empty block)
 };
 
-__global__ void __launch_bounds__(256) slater_kernel(const SlaterArgs a) {
+template <bool SIGN>
+__device__ __forceinline__ void slater_cta_body(const SlaterArgs& a) {
     extern __shared__ __align__(16) double smem[];
     const int tid = threadIdx.x, T = blockDim.x;
     const int n = a.n, D = 2 * n, W = a.W;
@@ -116,8 +118,8 @@ __global__ void __launch_bounds__(256) slater_kernel(const SlaterArgs a) {
         __syncthreads();
         auto orbp = [&](int w) { long long b = base + w; int row = (a.walker_state && b < a.B) ? a.walker_state[b] : 0;
                                  return a.orb + (size_t)row * n; };
-        if (deriv) slater_team<true>(W, n, a.n_up, [&](int w) { return (const double*)xw(w); }, scr, orbp);
-        else slater_team<false>(W, n, a.n_up, [&](int w) { return (const double*)xw(w); }, scr, orbp);
+        if (deriv) slater_team<true, SIGN>(W, n, a.n_up, [&](int w) { return (const double*)xw(w); }, scr, orbp);
+        else slater_team<false, SIGN>(W, n, a.n_up, [&](int w) { return (const double*)xw(w); }, scr, orbp);
         if (deriv) {
             for (int g = tid; g < W * n * n; g += T) {
                 int w = g / (n * n), rem = g - w * n * n;
@@ -156,9 +158,14 @@ __global__ void __launch_bounds__(256) slater_kernel(const SlaterArgs a) {
                 for (int k = 0; k < n * n; ++k) acc += red(w)[k];
                 a.lap[b] = a.scale * acc;
             }
+            if (SIGN && a.sign) a.sign[b] = (bu.ns ? S[bu.misc() + 3] : 1.0) * (bd.ns ? S[bd.misc() + 3] : 1.0);
         }
     }
 }
+
+__global__ void __launch_bounds__(256) slater_kernel(const SlaterArgs a) { slater_cta_body<false>(a); }
+// the same, also writing SlaterArgs::sign (ff_wavefunction_ratio)
+__global__ void __launch_bounds__(256) slater_sign_kernel(const SlaterArgs a) { slater_cta_body<true>(a); }
 
 // ---------------------------------------------------------------------------------------
 // The same with ONE WARP PER WALKER (spin blocks of at most 16 particles): no CTA barrier.
@@ -176,7 +183,8 @@ __host__ __device__ inline int slater_warp_slice(int nmax) {      // doubles of 
     return ff_even(nmax * (2 * nmax + 1) + nmax * kHermStride + 2);
 }
 
-__global__ void __launch_bounds__(256) slater_warp_kernel(const SlaterArgs a) {
+template <bool SIGN>
+__device__ __forceinline__ void slater_warp_body(const SlaterArgs& a) {
     extern __shared__ __align__(16) double smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
     const int n = a.n, D = 2 * n;
@@ -188,7 +196,7 @@ __global__ void __launch_bounds__(256) slater_warp_kernel(const SlaterArgs a) {
     const long long wstride = (long long)gridDim.x * nwarp;
     for (long long b = (long long)blockIdx.x * nwarp + warp; b < a.B; b += wstride) {
         const int* orb = a.orb + (size_t)(a.walker_state ? a.walker_state[b] : 0) * n;
-        double logdet = 0.0, lap = 0.0;
+        double logdet = 0.0, lap = 0.0, sgn = 1.0;
         for (int s = 0; s < 2; ++s) {
             const int ns = s ? n - a.n_up : a.n_up, i0 = s ? a.n_up : 0;
             if (ns == 0) continue;
@@ -230,6 +238,7 @@ __global__ void __launch_bounds__(256) slater_warp_kernel(const SlaterArgs a) {
                     if (ob > best || (ob == best && op < p)) { best = ob; p = op; }
                 }
                 logdet += log(best);
+                if (SIGN && ((A[p * LD + k] < 0.0) != (p != k))) sgn = -sgn;     // pivot sign, row swap
                 const double ipv = 1.0 / A[p * LD + k];
                 __syncwarp();
                 if (lane < 2 * ns) {                       // lane = column: swap rows k <-> p, scale row k
@@ -277,9 +286,14 @@ __global__ void __launch_bounds__(256) slater_warp_kernel(const SlaterArgs a) {
         if (lane == 0) {
             if (a.logabs) a.logabs[b] = a.scale * logdet;
             if (a.lap) a.lap[b] = a.scale * lap;
+            if (SIGN && a.sign) a.sign[b] = sgn;
         }
     }
 }
+
+__global__ void __launch_bounds__(256) slater_warp_kernel(const SlaterArgs a) { slater_warp_body<false>(a); }
+// the same, also writing SlaterArgs::sign (ff_wavefunction_ratio)
+__global__ void __launch_bounds__(256) slater_warp_sign_kernel(const SlaterArgs a) { slater_warp_body<true>(a); }
 
 // ---------------------------------------------------------------------------------------
 // Hessian-vector product of scale * (log|det Phi_up| + log|det Phi_dn|): the double backward of

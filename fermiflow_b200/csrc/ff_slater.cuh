@@ -55,8 +55,10 @@ __device__ __forceinline__ SlBlk slater_blk(int s, int n, int n_up) {
 // Builds Phi and its derivatives, inverts Phi (Gauss-Jordan, partial pivoting), forms
 // B^x, B^y, C.  On return, for spin block s of walker w (scratch pointer S = sptr(w)):
 //   S[blk.misc()+2] = log|det Phi|, S[blk.aug() + i*2ns + ns + j] = Phi^-1[i][j].
-// All threads of the CTA must call it.  DERIV = false stops after log|det|.
-template <bool DERIV, class ZPtr, class SPtr, class OrbPtr, class Team = CtaTeam>
+// All threads of the CTA must call it.  DERIV = false stops after log|det|.  SIGN = true also leaves
+// S[blk.misc()+3] = sign(det Phi) of each non-empty block: the product of the pivot signs, negated once per row
+// swap p != k.  Without SIGN the slot is not touched and the generated code is that of the sign-free routine.
+template <bool DERIV, bool SIGN = false, class ZPtr, class SPtr, class OrbPtr, class Team = CtaTeam>
 __device__ void slater_team(int W, int n, int n_up, ZPtr zptr, SPtr sptr, OrbPtr orbptr, Team team = Team()) {
     const int tid = team.tid(), T = team.size();
     const double inv_sqrt_pi = 0.56418958354775628695;
@@ -84,7 +86,10 @@ __device__ void slater_team(int W, int n, int n_up, ZPtr zptr, SPtr sptr, OrbPtr
                 S[blk.dyy() + i * ns + k] = inv_sqrt_pi * vx * vy2;
             }
         }
-        for (int w = tid; w < W; w += T) sptr(w)[blk.misc() + 2] = 0.0;
+        for (int w = tid; w < W; w += T) {
+            sptr(w)[blk.misc() + 2] = 0.0;
+            if (SIGN) sptr(w)[blk.misc() + 3] = 1.0;
+        }
     }
     team.sync();
     // ---- F2: Gauss-Jordan on [Phi | I] ---------------------------------------------------
@@ -105,6 +110,10 @@ __device__ void slater_team(int W, int n, int n_up, ZPtr zptr, SPtr sptr, OrbPtr
             S[blk.misc() + 0] = (double)p;
             S[blk.misc() + 1] = A[p * 2 * ns + k];
             S[blk.misc() + 2] += log(best);
+            if (SIGN) {
+                const double sg = (A[p * 2 * ns + k] < 0.0) != (p != k) ? -1.0 : 1.0;
+                S[blk.misc() + 3] *= sg;
+            }
         }
         team.sync();
         for (int s = 0; s < 2; ++s) {                    // swap rows k <-> p, scale row k

@@ -1,4 +1,6 @@
-"""Spin-resolved one-body density and pair correlations of sampled walkers (C ABI ff_observables).
+"""Spin-resolved one-body density and pair correlations of sampled walkers (C ABI ff_observables), and the momentum
+distribution and one-body coherence from signed wave-function ratios (C ABI ff_wavefunction_ratio,
+ff_momentum_accumulate).
 
     est = DensityEstimator(n_up, n_dn, extent=6.0)
     with torch.no_grad():
@@ -49,7 +51,50 @@ def observables(x, n_up, n_dn, extent, n_xy, r_max, n_r, n_rot, counts):
     return counts
 
 
-class DensityEstimator:
+class _BatchMeans:
+    """Running sums of per-batch vectors v_k (each a sum over the W_k walkers of batch k) for batch-means errors:
+    [sum v_k, sum v_k² / W_k, sum W_k, calls] in one float64 vector on `device`, so that ranks merge with one
+    all-reduce."""
+
+    def _init_state(self, n_values, device):
+        self.device = torch.device(device)
+        self._n_values = int(n_values)
+        self.state = torch.zeros(2 * self._n_values + 2, dtype=torch.float64, device=self.device)
+
+    def _merge(self, values, walkers):
+        """Add one batch of `walkers` walkers whose values summed to `values` (plain torch)."""
+        if walkers <= 0:
+            return
+        v = values.to(self.state.device, torch.float64)
+        nv = self._n_values
+        self.state[:nv] += v
+        self.state[nv:2 * nv].addcmul_(v, v, value=1.0 / walkers)
+        self.state[-2] += float(walkers)
+        self.state[-1] += 1.0
+
+    def allreduce(self):
+        """Sum the state over the ranks of torch.distributed (NCCL for CUDA state, gloo for CPU state); a no-op on one
+        rank.  Every rank must call it, as with VMC's allreduce_gradients, and then holds the merged state."""
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            dist.all_reduce(self.state)
+
+    def _per_walker(self):
+        """(mean per walker, its standard error, walkers, calls, sum v_k² / W_k) as device tensors.  Batch means
+        m_k = v_k / W_k weighted by W_k: var(mean) = Σ W_k (m_k − mean)² / ((K − 1) W); NaN below two calls."""
+        nv = self._n_values
+        s1, s2 = self.state[:nv], self.state[nv:2 * nv]
+        W, K = self.state[-2], self.state[-1]
+        mean = s1 / W
+        var = (s2 - W * mean * mean).clamp_min(0.0) / ((K - 1.0) * W)
+        err = torch.where(K >= 2, var.sqrt(), torch.full_like(var, float("nan")))
+        return mean, err, W, K, s2
+
+    def save(self, path):
+        """np.savez of result()."""
+        np.savez(path, **self.result())
+
+
+class DensityEstimator(_BatchMeans):
     """Spin-resolved one-body density, radial density, pair-separation distribution and rotated-frame pair density
     of walkers [B, n_up + n_dn, 2] (particle i < n_up is spin-up).
 
@@ -80,11 +125,10 @@ class DensityEstimator:
         self.extent = float(extent)
         self.r_max = float(extent if r_max is None else r_max)
         self.n_xy, self.n_r, self.n_rot = int(n_xy), int(n_r), int(n_rot)
-        self.device = torch.device(device)
         self.layout, self.n_bins = count_layout(self.n_xy, self.n_r, self.n_rot)
         self.n_counts = self.n_bins + _OUTSIDE
         # [sum of counts, sum over calls of counts² / walkers, walkers, calls]: one vector, one all-reduce
-        self.state = torch.zeros(2 * self.n_counts + 2, dtype=torch.float64, device=self.device)
+        self._init_state(self.n_counts, device)
         self._buf = None
 
     def accumulate(self, x):
@@ -97,30 +141,11 @@ class DensityEstimator:
 
     def _add_batch(self, counts, walkers):
         """Merge the counts of one batch of `walkers` walkers into the running sums (plain torch)."""
-        if walkers <= 0:
-            return
-        c = counts.to(self.state.device, torch.float64)
-        nc = self.n_counts
-        self.state[:nc] += c
-        self.state[nc:2 * nc].addcmul_(c, c, value=1.0 / walkers)
-        self.state[-2] += float(walkers)
-        self.state[-1] += 1.0
-
-    def allreduce(self):
-        """Sum the state over the ranks of torch.distributed (NCCL for CUDA state, gloo for CPU state); a no-op on one
-        rank.  Every rank must call it, as with VMC's allreduce_gradients, and then holds the merged state."""
-        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-            dist.all_reduce(self.state)
+        self._merge(counts, walkers)
 
     def result(self):
         """dict of float64 numpy arrays (see the class docstring)."""
-        nc = self.n_counts
-        s1, s2 = self.state[:nc], self.state[nc:2 * nc]
-        W, K = self.state[-2], self.state[-1]
-        mean = s1 / W
-        # batch means m_k = c_k / B_k weighted by B_k: var(mean) = Σ B_k (m_k − mean)² / ((K − 1) W)
-        var = (s2 - W * mean * mean).clamp_min(0.0) / ((K - 1.0) * W)
-        err = torch.where(K >= 2, var.sqrt(), torch.full_like(var, float("nan")))
+        mean, err, W, K, _ = self._per_walker()
         nu, nd = self.n_up, self.n_dn
         n = nu + nd
         f64 = dict(dtype=torch.float64, device=self.state.device)
@@ -147,10 +172,6 @@ class DensityEstimator:
         out["n_up"], out["n_dn"] = torch.tensor(float(nu), **f64), torch.tensor(float(nd), **f64)
         return {k: v.cpu().numpy() for k, v in out.items()}
 
-    def save(self, path):
-        """np.savez of result()."""
-        np.savez(path, **self.result())
-
 
 def sample_density(model, n_up, n_dn, batch, batches, extent, path):
     """The --density option of the drivers: `batches` batches of `batch` walkers from model.sample at the current
@@ -166,4 +187,150 @@ def sample_density(model, n_up, n_dn, batch, batches, extent, path):
         res = est.result()
         print("density: %d walkers saved to %s; outside the density grid: up %.3g, down %.3g (fraction of particles)"
               % (res["walkers"], path, res["outside_fraction"][0], res["outside_fraction"][1]))
+    return est
+
+
+def sums_layout(n_k, n_kr, n_s):
+    """{section: (offset, shape)} of the sums of ff_momentum_accumulate (include/fermiflow_b200.h) and their length."""
+    out, off = {}, 0
+    for name, shape in (("momentum", (2, n_k, n_k)), ("radial", (2, n_kr)), ("ratio", (2, n_s)), ("records", (2, n_s)),
+                        ("channel", (2,))):
+        out[name] = (off, shape)
+        off += math.prod(shape)
+    return out, off
+
+
+def momentum_accumulate(ratio, particle, disp, n_up, k_max, n_k, n_kr, s_max, n_s, sums):
+    """ff_momentum_accumulate on CUDA records (ratio float64 [R], particle int32 [R], disp float64 [R, 2]): ADDS the
+    sums to `sums` (float64, the layout of sums_layout)."""
+    g = L.FFMomGrid(float(k_max), int(n_k), int(n_kr), float(s_max), int(n_s))
+    R = ratio.numel()
+    L.check(L.lib().ff_momentum_accumulate(L.ptr(ratio.reshape(-1)), L.ptr(particle.reshape(-1), torch.int32),
+                                           L.ptr(disp.reshape(-1, 2)), R, int(n_up), C.byref(g), L.ptr(sums),
+                                           sums.numel(), L.stream()))
+    return sums
+
+
+class MomentumEstimator(_BatchMeans):
+    """Spin-resolved momentum distribution n_c(k) and one-body coherence g_c(|s|) of a VMC model (GSVMC or BetaVMC)
+    from signed wave-function ratios.  A record is one walker x ~ |ψ|², one particle i drawn uniformly from all n and
+    one displacement s drawn uniformly in the disk |s| < s_max; its ratio is ρ = ψ(x with r_i → r_i + s) / ψ(x)
+    (model.wavefunction_ratio, sign included) and its channel c = (i ≥ n_up).  With `moves` = M records per walker
+    and W walkers in all:
+
+      n_c(k) = (2π)⁻² ∫ d²s cos(k·s) Σ_{i∈c} ⟨ρ_i(s)⟩  ≈  n s_max² / (4π M W) Σ_records 1{c} ρ cos(k·s)
+
+    normalised to ∫ n_c(k) d²k = n_c (up to the part of ⟨ρ_i(s)⟩ beyond s_max).  ρ is real and even in s because ψ is
+    real, so the cosine carries all of it.  The radial n_c(|k|) is the same sum with J0(|k| |s|) in place of the
+    cosine.  The one-body coherence g_c(|s|) = (1 / n_c) ∫ d²r ρ1_c(r, r + s), averaged over directions, is the mean
+    of ρ over the records of channel c whose |s| falls in the annulus; g_c(0) = 1.  For BetaVMC each walker uses its
+    own occupation row, and the same formulas give the quantities of the mixed state.
+
+    result() returns float64 numpy arrays:
+      momentum [2][n_k][n_k]      n_c at the cell centres of [-k_max, k_max)², index [c][ix][iy] (k_edges)
+      momentum_radial [2][n_kr]   n_c(|k|) at k_radial = (j + 1/2) k_max / n_kr
+      coherence [2][n_s]          g_c in the |s| bins s_edges over [0, s_max) (NaN for a bin without records)
+    each with `<name>_err` (batch means over the calls of accumulate(), weighted by each call's walker count; NaN with
+    fewer than two calls), and k_edges, k_radial, s_edges, walkers, calls, moves, n_up, n_dn.
+    """
+
+    def __init__(self, n_up, n_dn, k_max=4.0, n_k=64, n_kr=128, s_max=8.0, n_s=64, moves=8,
+                 device=torch.device("cuda")):
+        if n_up < 0 or n_dn < 0 or n_up + n_dn < 1:
+            raise ValueError("bad particle numbers %d/%d" % (n_up, n_dn))
+        if moves < 1:
+            raise ValueError("moves must be at least 1, got %d" % moves)
+        if not (k_max > 0 and math.isfinite(k_max) and s_max > 0 and math.isfinite(s_max)):
+            raise ValueError("k_max and s_max must be positive and finite, got %r and %r" % (k_max, s_max))
+        if min(n_k, n_kr, n_s) < 0:
+            raise ValueError("negative bin count (n_k %d, n_kr %d, n_s %d)" % (n_k, n_kr, n_s))
+        self.n_up, self.n_dn = int(n_up), int(n_dn)
+        self.k_max, self.s_max = float(k_max), float(s_max)
+        self.n_k, self.n_kr, self.n_s = int(n_k), int(n_kr), int(n_s)
+        self.moves = int(moves)
+        self.layout, self.n_sums = sums_layout(self.n_k, self.n_kr, self.n_s)
+        # the sums, then ratio sum + record count per |s| bin: its squares give the cross moment the error of the
+        # coherence (a ratio of two means) needs
+        self._init_state(self.n_sums + 2 * self.n_s, device)
+        self._buf = None
+
+    def accumulate(self, model, x, generator=None):
+        """Add one batch of independent walkers x (CUDA float64 [B, n_up + n_dn, 2], drawn by model.sample at the
+        current parameters): `moves` records per walker, drawn on the device (torch.randint / torch.rand with
+        `generator`); no host synchronisation."""
+        n = self.n_up + self.n_dn
+        if x.dim() != 3 or x.shape[-1] != 2 or x.shape[1] != n:
+            raise ValueError("x must be [B, %d, 2], got %s" % (n, tuple(x.shape)))
+        if not x.is_cuda:
+            raise RuntimeError("MomentumEstimator needs CUDA walkers (got %s); no CPU fallback" % x.device)
+        B, M, dev = x.shape[0], self.moves, x.device
+        particle = torch.randint(0, n, (B, M), device=dev, dtype=torch.int32, generator=generator)
+        u = torch.rand(B, M, 2, device=dev, dtype=torch.float64, generator=generator)
+        r = self.s_max * u[..., 0].sqrt()
+        phi = (2 * math.pi) * u[..., 1]
+        disp = torch.stack((r * phi.cos(), r * phi.sin()), -1)
+        ratio = model.wavefunction_ratio(x, particle, disp)
+        if self._buf is None or self._buf.device != dev:
+            self._buf = torch.empty(self.n_sums, dtype=torch.float64, device=dev)
+        self._buf.zero_()
+        momentum_accumulate(ratio, particle, disp, self.n_up, self.k_max, self.n_k, self.n_kr, self.s_max, self.n_s,
+                            self._buf)
+        self._add_batch(self._buf, B)
+
+    def _add_batch(self, sums, walkers):
+        """Merge the sums of one batch of `walkers` walkers into the running state (plain torch)."""
+        o1, sh = self.layout["ratio"]
+        o2, _ = self.layout["records"]
+        k = math.prod(sh)
+        self._merge(torch.cat((sums, sums[o1:o1 + k] + sums[o2:o2 + k])), walkers)
+
+    def result(self):
+        """dict of float64 numpy arrays (see the class docstring)."""
+        mean, err, W, K, s2 = self._per_walker()
+        nu, nd = self.n_up, self.n_dn
+        f64 = dict(dtype=torch.float64, device=self.state.device)
+        norm = (nu + nd) * self.s_max ** 2 / (4 * math.pi * self.moves)
+        out = {}
+
+        def sect(name, t=mean):
+            off, shape = self.layout[name]
+            return t[off:off + math.prod(shape)].reshape(shape)
+
+        out["momentum"], out["momentum_err"] = norm * sect("momentum"), norm * sect("momentum", err)
+        out["momentum_radial"], out["momentum_radial_err"] = norm * sect("radial"), norm * sect("radial", err)
+        # coherence g = S / N per bin (S, N: ratio sum and records per walker); delta method over the batch means:
+        # var(g) = Σ W_k (s_k − g n_k)² / ((K − 1) W N²), with Σ S_k N_k / W_k from the squares of S_k + N_k
+        S, N = sect("ratio"), sect("records")
+        g = S / N
+        ns = self.n_sums
+        q = lambda name: sect(name, s2)                                  # noqa: E731
+        cross = 0.5 * (s2[ns:].reshape(S.shape) - q("ratio") - q("records"))
+        dev2 = q("ratio") - 2 * g * cross + g * g * q("records")        # Σ W_k (s_k − g n_k)², Σ W_k (s_k − g n_k) = 0
+        var = dev2.clamp_min(0.0) / ((K - 1.0) * W * N * N)
+        out["coherence"] = g
+        out["coherence_err"] = torch.where(K >= 2, var.sqrt(), torch.full_like(var, float("nan")))
+        out["k_edges"] = torch.linspace(-self.k_max, self.k_max, self.n_k + 1, **f64)
+        out["k_radial"] = (torch.arange(self.n_kr, **f64) + 0.5) * (self.k_max / max(self.n_kr, 1))
+        out["s_edges"] = torch.linspace(0.0, self.s_max, self.n_s + 1, **f64)
+        out["walkers"], out["calls"] = W, K
+        out["moves"] = torch.tensor(float(self.moves), **f64)
+        out["n_up"], out["n_dn"] = torch.tensor(float(nu), **f64), torch.tensor(float(nd), **f64)
+        return {k: v.cpu().numpy() for k, v in out.items()}
+
+
+def sample_momentum(model, n_up, n_dn, batch, batches, k_max, path):
+    """The --momentum option of the drivers: `batches` batches of `batch` walkers from model.sample at the current
+    parameters, `moves` = 8 one-particle moves per walker, merged over ranks and saved to `path` by rank 0."""
+    est = MomentumEstimator(n_up, n_dn, k_max=k_max, device=next(model.parameters()).device)
+    with torch.no_grad():
+        for _ in range(batches):
+            _, x = model.sample((batch,))
+            est.accumulate(model, x)
+    est.allreduce()
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0:
+        est.save(path)
+        res = est.result()
+        dk = 2 * est.k_max / est.n_k
+        print("momentum: %d walkers saved to %s; integral of n(k) over the grid: up %.4g, down %.4g"
+              % (res["walkers"], path, res["momentum"][0].sum() * dk * dk, res["momentum"][1].sum() * dk * dk))
     return est

@@ -160,6 +160,50 @@ typedef struct ff_obs_grid {
 int ff_observables(const double* x, long long B, int n_up, int n_dn, const ff_obs_grid* g,
                    unsigned long long* counts, long long n_counts, void* stream);
 
+/* Signed wave-function ratios of one-particle moves (no reference counterpart; the off-diagonal observables below need
+ * the wave function with its sign at configurations that were not sampled):
+ *   psi(x) = sign(det Phi_up(z) det Phi_dn(z)) exp(log p(x) / 2),   z = flow^-1(x)
+ * (the flow's Jacobian determinant is positive, so the sign comes from the Slater determinants alone).  A record is one
+ * walker b, one particle i = particle[b][m] (int32 [B][M]) and one displacement s = disp[b][m] ([B][M][2]); its ratio is
+ *   ratio[b][m] = psi(x_b with r_i -> r_i + s) / psi(x_b).
+ * orb and walker_state as in ff_eloc (walker_state nullable: row 0 for every walker).  The call evaluates B (M + 1)
+ * configurations with the flow sweep of ff_cnf_delta_logp and the Slater kernels; slot 0 of each walker is x itself, so
+ * a record with s = 0 gives 1 to rounding.  A particle index outside [0, n) gives a NaN ratio for that record (nothing
+ * synchronises the host to check it).  work: ff_wavefunction_ratio_work_size doubles, 8-byte alignment suffices for
+ * every buffer.  -1 for bad particle numbers (check as ff_cnf_delta_logp, at most 36 per spin), B or M < 1 and null
+ * buffers. */
+int ff_wavefunction_ratio_work_size(const ff_model* m, long long B, int M, long long* n_work);
+int ff_wavefunction_ratio(const ff_model* m, const double* x, long long B, const int* orb, const int* walker_state,
+                          int M, const int* particle /* int32 [B][M] */, const double* disp /* [B][M][2] */,
+                          double* ratio /* [B][M] */, double* work, void* stream);
+
+/* Momentum distribution and one-body coherence from R records (ratio [R], particle int32 [R], disp [R][2], for example
+ * the B M records of ff_wavefunction_ratio).  A record's channel is c = (particle >= n_up).  Three sections, each
+ * switched off by 0 bins:
+ *   momentum  sum of ratio cos(k.s) at the n_k x n_k cell centres k = (kx_a, ky_b) of [-k_max, k_max)^2,
+ *             kx_a = -k_max + (a + 1/2) 2 k_max / n_k
+ *   radial    sum of ratio J0(k_j |s|) at k_j = (j + 1/2) k_max / n_kr (the direction average of cos(k.s))
+ *   coherence sum of ratio and number of records per |s| bin over [0, s_max): bin floor(|s| n_s / s_max), |s| with every
+ *             product and sum rounded separately; records with |s| >= s_max are in no bin
+ * With particles drawn uniformly from all n and s uniformly in the disk |s| < s_max, M records per walker and W walkers,
+ *   n_c(k) ~= n s_max^2 / (4 pi M W) sum over the records of channel c of ratio cos(k.s)
+ * (normalised to the integral of n_c(k) d^2k = n_c), and g_c(|s|) = sum of ratio / records in the bin of |s|.
+ * Layout of sums (n_sums = 2 n_k^2 + 2 n_kr + 4 n_s + 2):
+ *   [2][n_k][n_k] sum ratio cos(k.s) (index [c][a][b]), [2][n_kr] sum ratio J0(k|s|), [2][n_s] sum ratio,
+ *   [2][n_s] records (doubles, exact below 2^53), [2] records per channel.
+ * ACCUMULATES into sums (the caller zeroes them).  Fixed summation order without floating-point atomics: two calls on
+ * the same inputs give bit-identical sums.  A non-finite ratio propagates into the sums of its channel.  Scratch comes
+ * from the stream-ordered allocator.  -1 for n_up < 0, R < 1, null pointers, a non-positive or non-finite k_max / s_max
+ * of an enabled section, negative bin counts, n_sums not equal to the layout size, or a grid whose per-record tables
+ * (4 n_k + n_kr + 3 doubles) do not fit in the shared memory of one block. */
+typedef struct ff_mom_grid {
+    double k_max; int n_k;    /* n_k x n_k cell centres of [-k_max, k_max)^2; 0: off                  */
+    int n_kr;                 /* radial points k_j = (j + 1/2) k_max / n_kr (J0 average); 0: off       */
+    double s_max; int n_s;    /* |s| bins over [0, s_max) for g(s): ratio sums and record counts; 0: off */
+} ff_mom_grid;
+int ff_momentum_accumulate(const double* ratio, const int* particle, const double* disp, long long R, int n_up,
+                           const ff_mom_grid* g, double* sums, long long n_sums, void* stream);
+
 /* Raw FP64 FMA throughput of the device (roofline denominator): runs `iters` dependent
  * DFMA chains on every SM and returns the achieved FLOP/s in *flops_host. */
 int ff_fp64_peak(int iters, double* flops_host, void* stream);
