@@ -13,7 +13,7 @@ from .VMC import GSVMC
 from .base_dist import FreeFermion
 from .equivariant_funs import Backflow
 from .flow import CNF
-from .observables import sample_density, sample_momentum
+from .observables import sample_density, sample_momentum, sample_renyi
 from .orbitals import HO2D
 from .potentials import HO, CoulombPairPotential
 
@@ -41,6 +41,12 @@ def main(argv=None):
                    "coherence of freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.MomentumEstimator)")
     p.add_argument("--momentum-batches", type=int, default=16, help="batches of --batch walkers for --momentum")
     p.add_argument("--momentum-kmax", type=float, default=4.0, help="half-width of the momentum grid")
+    p.add_argument("--renyi", metavar="FILE", help="after training, save the second Renyi entropy of spatial regions, "
+                   "from replica swaps of freshly sampled walkers, to FILE (.npz, fermiflow_b200.observables.RenyiEstimator)")
+    p.add_argument("--renyi-batches", type=int, default=16, help="batches of --batch walkers for --renyi")
+    p.add_argument("--renyi-a", type=lambda s: [float(v) for v in s.split(",")], default=[0.5, 1.0, 1.5, 2.0, 2.5, 3.0],
+                   help="comma-separated region parameters for --renyi: disk radii or half-plane edges x < a")
+    p.add_argument("--renyi-kind", choices=("disk", "halfplane"), default="disk", help="region kind for --renyi")
     args = p.parse_args(argv)
 
     device = torch.device("cuda:%d" % args.cuda)
@@ -69,6 +75,8 @@ def main(argv=None):
         sample_density(model, args.nup, args.ndown, args.batch, args.density_batches, args.density_extent, args.density)
     if args.momentum:
         sample_momentum(model, args.nup, args.ndown, args.batch, args.momentum_batches, args.momentum_kmax, args.momentum)
+    if args.renyi:
+        sample_renyi(model, args.nup, args.ndown, args.batch, args.renyi_batches, args.renyi_a, args.renyi_kind, args.renyi)
     return history
 
 

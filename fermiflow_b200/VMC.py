@@ -102,6 +102,39 @@ def _wavefunction_ratio(cnf, x, orb, walker_state, n_up, particle, disp):
     return ratio
 
 
+_REGION_KINDS = {"disk": 0, "halfplane": 1}
+
+
+def _swap_ratio(cnf, x, orb, walker_state, n_up, pairs, a, kind):
+    """psi(x') psi(y') / (psi(x) psi(y)) for every pair p (x = x[pairs[p, 0]], y = x[pairs[p, 1]]) and region q, x'
+    and y' the two walkers with their particles in region q swapped (C ABI ff_swap_ratio).  x [B, n, 2] and pairs
+    integer [P, 2] on the device, a: Q region parameters (disk radii or half-plane edges), kind "disk" or "halfplane";
+    returns ratio [P, Q] and sector int32 [P, 2, Q].  A walker index outside [0, B) gives NaN and sector -1."""
+    x = x.detach().contiguous()
+    if x.dim() != 3 or x.shape[-1] != 2:
+        raise ValueError("x must be [B, n, 2], got %s" % (tuple(x.shape),))
+    if pairs.dim() != 2 or pairs.shape[1] != 2:
+        raise ValueError("pairs must be [P, 2], got %s" % (tuple(pairs.shape),))
+    if kind not in _REGION_KINDS:
+        raise ValueError("kind must be one of %s, got %r" % (sorted(_REGION_KINDS), kind))
+    B, n, _ = x.shape
+    P = pairs.shape[0]
+    av = (C.c_double * len(a))(*[float(v) for v in a])
+    reg = L.FFSwapRegions(_REGION_KINDS[kind], len(a), av)
+    p32 = pairs.to(torch.int32).contiguous()
+    model = cnf._model(n, n_up=n_up)
+    nw = C.c_longlong()
+    L.check(L.lib().ff_swap_ratio_work_size(C.byref(model), P, len(a), C.byref(nw)))
+    work = torch.empty(nw.value, dtype=torch.float64, device=x.device)
+    ratio = torch.empty(P, len(a), dtype=torch.float64, device=x.device)
+    sector = torch.empty(P, 2, len(a), dtype=torch.int32, device=x.device)
+    L.check(L.lib().ff_swap_ratio(C.byref(model), L.ptr(x), B, L.ptr(orb, torch.int32),
+                                  L.ptr(walker_state, torch.int32) if walker_state is not None else None,
+                                  P, L.ptr(p32, torch.int32), C.byref(reg), L.ptr(ratio), L.ptr(sector, torch.int32),
+                                  L.ptr(work), L.stream()))
+    return ratio, sector
+
+
 def _multi_rank():
     return dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
 
@@ -208,6 +241,12 @@ class GSVMC(_VMCBase):
         """psi(x with r_i -> r_i + s) / psi(x) per record, sign included: x [B, n, 2], particle [B, M] (i),
         disp [B, M, 2] (s) -> ratio [B, M] (fermiflow_b200.observables.MomentumEstimator uses it)."""
         return _wavefunction_ratio(self.cnf, x, self._orb(x.device), None, self.nup, particle, disp)
+
+    def swap_ratio(self, x, pairs, a, kind="disk"):
+        """Replica swap ratios psi(x') psi(y') / (psi(x) psi(y)) of the walker pairs [P, 2] for the regions a (disk
+        radii or half-plane edges, Q of them): x [B, n, 2] -> ratio [P, Q], sector int32 [P, 2, Q]
+        (fermiflow_b200.observables.RenyiEstimator uses it)."""
+        return _swap_ratio(self.cnf, x, self._orb(x.device), None, self.nup, pairs, a, kind)
 
     def forward(self, batch):                                         # VMC.py:41-61
         _, x = self.sample((batch,))
@@ -317,15 +356,25 @@ class BetaVMC(_VMCBase):
         log_prob_z = _FreeFermionLogp.apply(z, self._state_table(x.device), self.state_indices, self.nup, self.ndown)
         return log_prob_z - delta_logp
 
-    def wavefunction_ratio(self, x, particle, disp, walker_state=None):
-        """GSVMC.wavefunction_ratio with each walker's own occupation row: walker_state (int [B]) defaults to the
-        state_indices of the last sample()."""
+    def _walker_state(self, x, walker_state):
+        """int32 occupation row per walker of x: walker_state, or by default the state_indices of the last sample()."""
         ws = getattr(self, "state_indices", None) if walker_state is None else walker_state
         if ws is None or ws.shape != (x.shape[0],):
             raise ValueError("walker_state must hold one state index per walker (%d), got %s"
                              % (x.shape[0], None if ws is None else tuple(ws.shape)))
-        return _wavefunction_ratio(self.cnf, x, self._state_table(x.device), ws.to(torch.int32).contiguous(), self.nup,
-                                   particle, disp)
+        return ws.to(torch.int32).contiguous()
+
+    def wavefunction_ratio(self, x, particle, disp, walker_state=None):
+        """GSVMC.wavefunction_ratio with each walker's own occupation row: walker_state (int [B]) defaults to the
+        state_indices of the last sample()."""
+        return _wavefunction_ratio(self.cnf, x, self._state_table(x.device), self._walker_state(x, walker_state),
+                                   self.nup, particle, disp)
+
+    def swap_ratio(self, x, pairs, a, kind="disk", walker_state=None):
+        """GSVMC.swap_ratio with each walker's own occupation row (the two sides of a pair may sit in different
+        states): walker_state (int [B]) defaults to the state_indices of the last sample()."""
+        return _swap_ratio(self.cnf, x, self._state_table(x.device), self._walker_state(x, walker_state), self.nup,
+                           pairs, a, kind)
 
     def forward(self, batch):                                          # VMC.py:120-171
         _, x = self.sample((batch,))

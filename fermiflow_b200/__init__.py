@@ -11,4 +11,4 @@ from .base_dist import FreeFermion  # noqa: F401
 from .potentials import HO, CoulombPairPotential  # noqa: F401
 from .slater import LogAbsSlaterDet, LogAbsSlaterDetMultStates  # noqa: F401
 from .VMC import GSVMC, BetaVMC  # noqa: F401
-from .observables import DensityEstimator, MomentumEstimator  # noqa: F401
+from .observables import DensityEstimator, MomentumEstimator, RenyiEstimator  # noqa: F401

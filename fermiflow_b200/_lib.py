@@ -30,6 +30,10 @@ class FFMomGrid(C.Structure):
                 ("s_max", C.c_double), ("n_s", C.c_int)]
 
 
+class FFSwapRegions(C.Structure):
+    _fields_ = [("kind", C.c_int), ("Q", C.c_int), ("a", C.POINTER(C.c_double))]
+
+
 _lib = None
 _P, _LL, _I, _D = C.c_void_p, C.c_longlong, C.c_int, C.c_double
 _M = C.POINTER(FFModel)
@@ -58,6 +62,9 @@ SIGNATURES = {
     "ff_wavefunction_ratio_work_size": ([_M, _LL, _I, C.POINTER(_LL)], C.c_int),
     "ff_wavefunction_ratio": ([_M, _P, _LL, _P, _P, _I, _P, _P, _P, _P, _P], C.c_int),
     "ff_momentum_accumulate": ([_P, _P, _P, _LL, _I, C.POINTER(FFMomGrid), _P, _LL, _P], C.c_int),
+    "ff_swap_ratio_work_size": ([_M, _LL, _I, C.POINTER(_LL)], C.c_int),
+    "ff_swap_ratio": ([_M, _P, _LL, _P, _P, _LL, _P, C.POINTER(FFSwapRegions), _P, _P, _P, _P], C.c_int),
+    "ff_swap_accumulate": ([_P, _P, _LL, _I, _I, _I, _P, _LL, _P], C.c_int),
     "ff_fp64_peak": ([_I, C.POINTER(_D), _P], C.c_int),
     "ff_fp64_mma_peak": ([_I, C.POINTER(_D), _P], C.c_int),
 }

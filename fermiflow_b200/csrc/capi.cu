@@ -8,6 +8,7 @@
 #include "ff_metro_reg.cuh"
 #include "ff_observables.cuh"
 #include "ff_momentum.cuh"
+#include "ff_renyi.cuh"
 
 namespace ffc {
 

@@ -1,6 +1,7 @@
-"""Spin-resolved one-body density and pair correlations of sampled walkers (C ABI ff_observables), and the momentum
+"""Spin-resolved one-body density and pair correlations of sampled walkers (C ABI ff_observables), the momentum
 distribution and one-body coherence from signed wave-function ratios (C ABI ff_wavefunction_ratio,
-ff_momentum_accumulate).
+ff_momentum_accumulate), and the second Rényi entropy of spatial regions from replica swap ratios (C ABI ff_swap_ratio,
+ff_swap_accumulate).
 
     est = DensityEstimator(n_up, n_dn, extent=6.0)
     with torch.no_grad():
@@ -333,4 +334,159 @@ def sample_momentum(model, n_up, n_dn, batch, batches, k_max, path):
         dk = 2 * est.k_max / est.n_k
         print("momentum: %d walkers saved to %s; integral of n(k) over the grid: up %.4g, down %.4g"
               % (res["walkers"], path, res["momentum"][0].sum() * dk * dk, res["momentum"][1].sum() * dk * dk))
+    return est
+
+
+def swap_layout(Q, n_up, n_dn):
+    """{section: (offset, shape)} of the sums of ff_swap_accumulate (include/fermiflow_b200.h) and their length."""
+    sec = (Q, n_up + 1, n_dn + 1)
+    out, off = {}, 0
+    for name, shape in (("ratio", sec), ("replicas", sec), ("matched", sec), ("skipped", (Q,)), ("pairs", (1,))):
+        out[name] = (off, shape)
+        off += math.prod(shape)
+    return out, off
+
+
+def swap_accumulate(ratio, sector, n_up, n_dn, sums):
+    """ff_swap_accumulate on CUDA records (ratio float64 [P, Q], sector int32 [P, 2, Q]): ADDS the sums to `sums`
+    (float64, the layout of swap_layout)."""
+    P, Q = ratio.shape
+    ratio, sector = ratio.contiguous(), sector.contiguous()
+    L.check(L.lib().ff_swap_accumulate(L.ptr(ratio), L.ptr(sector, torch.int32), P, Q, int(n_up), int(n_dn),
+                                       L.ptr(sums), sums.numel(), L.stream()))
+    return sums
+
+
+class RenyiEstimator(_BatchMeans):
+    """Second Rényi entropy S2(A) = −ln Tr ρ_A² of spatial regions A of a VMC model (GSVMC or BetaVMC), from the
+    replica swap estimator (Hastings et al. 2010; for fermions McMinis & Tubman 2013):
+
+      Tr ρ_A² = ⟨ ψ(x′) ψ(y′) / (ψ(x) ψ(y)) ⟩,   x, y independent draws from ρ,
+
+    x′ being x with its particles inside A replaced by those of y (slot by slot within each spin block) and y′ the
+    reverse; a pair whose replicas hold different numbers (n_A↑, n_A↓) contributes exactly 0.  The regions are all of
+    one `kind`: "disk" |r| < a_q about the trap centre or "halfplane" x < a_q, one per entry of `a` (1 to 32).  Each
+    call of accumulate() pairs the walkers by a random permutation on the device (the last walker is dropped when B is
+    odd).  The pairing must be random: BetaVMC samples its walkers' states sorted, so neighbouring walkers are
+    correlated, and pairing them would bias Tr ρ² towards Σ_s p_s Tr ρ_s².  For BetaVMC each replica uses its own
+    occupation row, and the estimate is Tr ρ_A² of the mixed state ρ = Σ_s p_s |ψ_s⟩⟨ψ_s|.
+
+    ρ_A is block diagonal in (a, b) = (n_A↑, n_A↓), so the same records resolve the sectors: P(a, b) is the fraction of
+    replicas in the sector, Tr ρ_{A,ab}² the sum of the ratios of the pairs in that sector over all pairs
+    (Σ_ab Tr ρ_ab² = Tr ρ_A²) and S2(a, b) = −ln(Tr ρ_ab² / P(a, b)²) the entropy of the normalised block.
+
+    Limit: the mean ratio is e^{−S2} while each record is of order one, so the relative error grows as e^{S2} / √pairs;
+    regions with S2 ≳ 4 need far more samples than the default driver draws.  Swapping incrementally growing regions
+    (the ratio trick) would remove this, and is not done here.
+
+    result() returns float64 numpy arrays:
+      swap [Q]                              Tr ρ_A² per region
+      S2 [Q]                                −ln swap; its error swap_err / swap (NaN where swap ≤ 0)
+      sector_prob [Q][n_up + 1][n_dn + 1]   P(a, b)
+      sector_swap [Q][n_up + 1][n_dn + 1]   Tr ρ_{A,ab}²
+      S2_sector [Q][n_up + 1][n_dn + 1]     S2(a, b) (NaN for an empty sector or a non-positive sector_swap)
+    each with `<name>_err` (batch means over the calls of accumulate(), weighted by each call's pair count; NaN with
+    fewer than two calls), and a, kind, pairs, calls, n_up, n_dn.
+    """
+
+    def __init__(self, n_up, n_dn, a=(0.5, 1.0, 1.5, 2.0, 2.5, 3.0), kind="disk", device=torch.device("cuda")):
+        if n_up < 0 or n_dn < 0 or n_up + n_dn < 1:
+            raise ValueError("bad particle numbers %d/%d" % (n_up, n_dn))
+        if kind not in ("disk", "halfplane"):
+            raise ValueError("kind must be 'disk' or 'halfplane', got %r" % (kind,))
+        a = tuple(float(v) for v in a)
+        if not 1 <= len(a) <= 32:
+            raise ValueError("between 1 and 32 regions, got %d" % len(a))
+        if not all(math.isfinite(v) for v in a) or (kind == "disk" and min(a) < 0):
+            raise ValueError("region parameters must be finite (and radii non-negative), got %r" % (a,))
+        self.n_up, self.n_dn = int(n_up), int(n_dn)
+        self.a, self.kind, self.Q = a, kind, len(a)
+        self.layout, self.n_sums = swap_layout(self.Q, self.n_up, self.n_dn)
+        self._n_cells = self.Q * (self.n_up + 1) * (self.n_dn + 1)
+        # the sums, then the ratio sum per region (its error) and ratio sum + replicas per sector (the cross moment
+        # the error of S2_sector needs)
+        self._init_state(self.n_sums + self.Q + self._n_cells, device)
+        self._buf = None
+
+    def accumulate(self, model, x, generator=None):
+        """Add one batch of independent walkers x (CUDA float64 [B, n_up + n_dn, 2], B ≥ 2, drawn by model.sample at
+        the current parameters): B // 2 pairs from torch.randperm with `generator`; no host synchronisation."""
+        n = self.n_up + self.n_dn
+        if x.dim() != 3 or x.shape[-1] != 2 or x.shape[1] != n:
+            raise ValueError("x must be [B, %d, 2], got %s" % (n, tuple(x.shape)))
+        if not x.is_cuda:
+            raise RuntimeError("RenyiEstimator needs CUDA walkers (got %s); no CPU fallback" % x.device)
+        B, dev = x.shape[0], x.device
+        if B < 2:
+            raise ValueError("at least two walkers are needed for one pair, got %d" % B)
+        P = B // 2
+        pairs = torch.randperm(B, device=dev, generator=generator)[:2 * P].view(P, 2)
+        ratio, sector = model.swap_ratio(x, pairs, self.a, self.kind)
+        if self._buf is None or self._buf.device != dev:
+            self._buf = torch.empty(self.n_sums, dtype=torch.float64, device=dev)
+        self._buf.zero_()
+        swap_accumulate(ratio, sector, self.n_up, self.n_dn, self._buf)
+        self._add_batch(self._buf, P)
+
+    def _add_batch(self, sums, pairs):
+        """Merge the sums of one batch of `pairs` pairs into the running state (plain torch)."""
+        o1, _ = self.layout["ratio"]
+        o2, _ = self.layout["replicas"]
+        k = self._n_cells
+        per_region = sums[o1:o1 + k].reshape(self.Q, -1).sum(1)
+        self._merge(torch.cat((sums, per_region, sums[o1:o1 + k] + sums[o2:o2 + k])), pairs)
+
+    def result(self):
+        """dict of float64 numpy arrays, and `kind` as a string array (see the class docstring)."""
+        mean, err, W, K, s2 = self._per_walker()
+        f64 = dict(dtype=torch.float64, device=self.state.device)
+        nan = torch.tensor(float("nan"), **f64)
+        ns, Q = self.n_sums, self.Q
+        shape = self.layout["ratio"][1]
+
+        def sect(name, t=mean):
+            off, sh = self.layout[name]
+            return t[off:off + math.prod(sh)].reshape(sh)
+
+        out = {}
+        swap, swap_err = mean[ns:ns + Q], err[ns:ns + Q]
+        ok = swap > 0
+        out["swap"], out["swap_err"] = swap, swap_err
+        out["S2"] = torch.where(ok, -swap.clamp_min(1e-300).log(), nan)
+        out["S2_err"] = torch.where(ok, swap_err / swap, nan)
+        T, R = sect("ratio"), sect("replicas")                          # per pair: ratio sum, replicas
+        out["sector_prob"], out["sector_prob_err"] = 0.5 * R, 0.5 * sect("replicas", err)
+        out["sector_swap"], out["sector_swap_err"] = T, sect("ratio", err)
+        # S2(a, b) = −ln T + 2 ln R + const; delta method over the batch means with the cross moment
+        # Σ T_k R_k / W_k taken from the squares of T_k + R_k
+        good = (T > 0) & (R > 0)
+        Tg, Rg = torch.where(good, T, 1.0), torch.where(good, R, 1.0)
+        qT, qR = sect("ratio", s2) - W * T * T, sect("replicas", s2) - W * R * R
+        cross = 0.5 * (s2[ns + Q:].reshape(shape) - sect("ratio", s2) - sect("replicas", s2)) - W * T * R
+        dev2 = qT / (Tg * Tg) + 4 * qR / (Rg * Rg) - 4 * cross / (Tg * Rg)
+        var = dev2.clamp_min(0.0) / ((K - 1.0) * W)
+        out["S2_sector"] = torch.where(good, -(Tg / (0.25 * Rg * Rg)).log(), nan)
+        out["S2_sector_err"] = torch.where(good & (K >= 2), var.sqrt(), nan)
+        out["a"] = torch.tensor(self.a, **f64)
+        out["pairs"], out["calls"] = W, K
+        out["n_up"], out["n_dn"] = torch.tensor(float(self.n_up), **f64), torch.tensor(float(self.n_dn), **f64)
+        res = {k: v.cpu().numpy() for k, v in out.items()}
+        res["kind"] = np.array(self.kind)
+        return res
+
+
+def sample_renyi(model, n_up, n_dn, batch, batches, a, kind, path):
+    """The --renyi option of the drivers: `batches` batches of `batch` walkers from model.sample at the current
+    parameters, randomly paired, merged over ranks and saved to `path` by rank 0."""
+    est = RenyiEstimator(n_up, n_dn, a=a, kind=kind, device=next(model.parameters()).device)
+    with torch.no_grad():
+        for _ in range(batches):
+            _, x = model.sample((batch,))
+            est.accumulate(model, x)
+    est.allreduce()
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0:
+        est.save(path)
+        res = est.result()
+        print("renyi: %d pairs saved to %s; S2 per %s: %s" % (res["pairs"], path, kind, ", ".join(
+            "%g: %.4g +- %.2g" % (v, s, e) for v, s, e in zip(est.a, res["S2"], res["S2_err"]))))
     return est

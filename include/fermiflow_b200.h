@@ -204,6 +204,53 @@ typedef struct ff_mom_grid {
 int ff_momentum_accumulate(const double* ratio, const int* particle, const double* disp, long long R, int n_up,
                            const ff_mom_grid* g, double* sums, long long n_sums, void* stream);
 
+/* Replica swap ratios of spatial regions, for the second Renyi entropy (no reference counterpart):
+ *   exp(-S2(A)) = Tr rho_A^2 = < psi(x') psi(y') / (psi(x) psi(y)) >,   x, y independent draws from rho,
+ * with psi(x) = sign(det Phi_up(z) det Phi_dn(z)) exp(log p(x) / 2) as in ff_wavefunction_ratio.  Pair p is the two
+ * walkers x = x_{pairs[p][0]} and y = x_{pairs[p][1]} (pairs int32 [P][2]; the caller chooses the pairing, and the
+ * pairs should be independent: ff_occupation_sample returns sorted states, so neighbouring walkers of BetaVMC are not).
+ * Regions (ff_swap_regions, all of one kind, 1 <= Q <= 32): kind 0 the disks |r| < a_q about the trap centre, decided
+ * as x*x + y*y < a_q*a_q; kind 1 the half-planes x < a_q; every product and sum is rounded separately (no FMA).
+ * For region q, x' is x with its particles inside A_q replaced by those of y, slot by slot within each spin block: the
+ * k-th A-particle of x, in increasing particle index, takes the position of the k-th A-particle of y; y' is the
+ * reverse.  Another pairing of the A-particles permutes x' and y' by pi and pi^-1, so the product of the two signs
+ * does not change.  Each configuration is evaluated with the occupation row of its own walker (orb and walker_state as
+ * in ff_eloc; walker_state nullable: row 0 for every walker), so for BetaVMC the records estimate Tr rho_A^2 of the
+ * mixed state.  Outputs:
+ *   sector[p][s][q]  n_A_up (n_dn + 1) + n_A_dn of side s (int32 [P][2][Q])
+ *   ratio[p][q]      the pair ratio; exactly 0 when the two sides' sectors differ (the swapped configurations do not
+ *                    exist), exactly 1 when region q holds no particle of either side (x' = x, y' = y)
+ * A walker index outside [0, B) gives a NaN ratio and sector -1 on both sides for every region of that pair (nothing
+ * synchronises the host to check it, and nothing is read out of bounds).  The call evaluates 2 P (Q + 1)
+ * configurations with the flow sweep of ff_cnf_delta_logp and the SIGN Slater kernels.  work:
+ * ff_swap_ratio_work_size doubles, 8-byte alignment suffices for every buffer.  -1 for bad particle numbers (check as
+ * ff_cnf_delta_logp, at most 36 per spin), B or P < 1, null regions, Q outside [1, 32], a kind other than 0 or 1, a
+ * null or non-finite a_q, a negative radius, and null buffers. */
+typedef struct ff_swap_regions {
+    int kind;                 /* 0: disks |r| < a_q, 1: half-planes x < a_q  */
+    int Q;                    /* number of regions, 1 ... 32                 */
+    const double* a;          /* HOST [Q]: radii (>= 0) or half-plane edges  */
+} ff_swap_regions;
+int ff_swap_ratio_work_size(const ff_model* m, long long P, int Q, long long* n_work);
+int ff_swap_ratio(const ff_model* m, const double* x, long long B, const int* orb, const int* walker_state,
+                  long long P, const int* pairs /* int32 [P][2] */, const ff_swap_regions* reg,
+                  double* ratio /* [P][Q] */, int* sector /* int32 [P][2][Q] */, double* work, void* stream);
+
+/* Sector-resolved sums of P Q swap records (ratio [P][Q], sector int32 [P][2][Q], as ff_swap_ratio writes them), with
+ * n_sec = (n_up + 1)(n_dn + 1) sectors k = a (n_dn + 1) + b.  A record (p, q) whose two sectors both lie in
+ * [0, n_sec) counts both replicas in their sectors, and when the sectors are equal it is a matched pair of that
+ * sector and adds its ratio; any other record is skipped.  Layout of sums (n_sums = 3 Q n_sec + Q + 1):
+ *   [Q][n_sec] sum of the ratios of the matched pairs,   [Q][n_sec] replicas (both sides counted),
+ *   [Q][n_sec] matched pairs,   [Q] skipped records,   [1] pairs P
+ * (counts as doubles, exact below 2^53).  With W pairs in all: Tr rho_A^2 ~= sum over the sectors of the ratio sums / W,
+ * P(a, b) ~= replicas / (2 W), Tr rho_{A,ab}^2 ~= ratio sum of (a, b) / W and S2(a, b) = -ln(Tr rho_ab^2 / P(a, b)^2).
+ * ACCUMULATES into sums (the caller zeroes them).  Fixed summation order without floating-point atomics: two calls on
+ * the same inputs give bit-identical sums.  A non-finite ratio of a matched record propagates into its cell.  Scratch
+ * comes from the stream-ordered allocator.  -1 for bad particle numbers (n_up, n_dn >= 0, at most 36 each, n >= 1),
+ * P < 1, Q outside [1, 32], n_sums not equal to the layout size, and null buffers. */
+int ff_swap_accumulate(const double* ratio, const int* sector, long long P, int Q, int n_up, int n_dn,
+                       double* sums, long long n_sums, void* stream);
+
 /* Raw FP64 FMA throughput of the device (roofline denominator): runs `iters` dependent
  * DFMA chains on every SM and returns the achieved FLOP/s in *flops_host. */
 int ff_fp64_peak(int iters, double* flops_host, void* stream);
