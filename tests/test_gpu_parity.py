@@ -555,12 +555,13 @@ def test_flow_kernel_variants_agree_full_size(dev):
         close(o[2], outs[0][2], 1e-12, 1e-14)
 
 
-@pytest.mark.parametrize("nup,ndn,B", [(10, 10, 1), (10, 10, 2), (10, 10, 297), (10, 10, 1500), (7, 6, 297), (3, 3, 297)])
+@pytest.mark.parametrize("nup,ndn,B", [(10, 10, 1), (10, 10, 2), (10, 10, 297), (10, 10, 1500)])
 def test_eloc_kernel_variants_agree_full_size(dev, nup, ndn, B):
-    """N = 20, 13 and 6 at H = 50: the default sweep (eloc5_kernel: register-resident Jacobian, specialised warps)
-    against the generic flow_kernel<MODE_ELOC> (option eloc_generic), each with the Taylor tables and with direct
-    evaluation of every hidden unit (no_table: eloc5_kernel evaluates every item directly), against eloc5_kernel
-    without the table mirror (no_rt_cache) and with the CTA-synchronous finale (finale_cta)."""
+    """N = 20 at H = 50, the benchmark's particle number, at four batch sizes: the default sweep (eloc5_kernel:
+    register-resident Jacobian, specialised warps) against the generic flow_kernel<MODE_ELOC> (option eloc_generic),
+    each with the Taylor tables and with direct evaluation of every hidden unit (no_table: eloc5_kernel evaluates every
+    item directly), against eloc5_kernel without the table mirror (no_rt_cache) and with the CTA-synchronous finale
+    (finale_cta).  Every other instantiation: tests/test_gpu_eloc_specialisations.py."""
     model = _dot_model(dev, nsteps=4, nup=nup, ndn=ndn)
     _, x = model.sample((B,))
     res = []
