@@ -13,7 +13,7 @@ from .VMC import GSVMC
 from .base_dist import FreeFermion
 from .equivariant_funs import Backflow
 from .flow import CNF
-from .observables import sample_density, sample_momentum, sample_renyi
+from .observables import sample_density, sample_momentum, sample_natural_orbitals, sample_renyi
 from .orbitals import HO2D
 from .potentials import HO, CoulombPairPotential
 
@@ -47,6 +47,13 @@ def main(argv=None):
     p.add_argument("--renyi-a", type=lambda s: [float(v) for v in s.split(",")], default=[0.5, 1.0, 1.5, 2.0, 2.5, 3.0],
                    help="comma-separated region parameters for --renyi: disk radii or half-plane edges x < a")
     p.add_argument("--renyi-kind", choices=("disk", "halfplane"), default="disk", help="region kind for --renyi")
+    p.add_argument("--natural-orbitals", metavar="FILE", help="after training, save the one-body density matrix in the "
+                   "HO2D basis and its natural-orbital occupations, from one-particle moves of freshly sampled walkers, to "
+                   "FILE (.npz, fermiflow_b200.observables.DensityMatrixEstimator)")
+    p.add_argument("--natural-orbitals-batches", type=int, default=16,
+                   help="batches of --batch walkers for --natural-orbitals")
+    p.add_argument("--natural-orbitals-shells", type=int, default=7,
+                   help="oscillator shells 0 ... S of the basis for --natural-orbitals ((S + 1)(S + 2) / 2 orbitals)")
     args = p.parse_args(argv)
 
     device = torch.device("cuda:%d" % args.cuda)
@@ -77,6 +84,9 @@ def main(argv=None):
         sample_momentum(model, args.nup, args.ndown, args.batch, args.momentum_batches, args.momentum_kmax, args.momentum)
     if args.renyi:
         sample_renyi(model, args.nup, args.ndown, args.batch, args.renyi_batches, args.renyi_a, args.renyi_kind, args.renyi)
+    if args.natural_orbitals:
+        sample_natural_orbitals(model, args.nup, args.ndown, args.batch, args.natural_orbitals_batches,
+                                args.natural_orbitals_shells, args.natural_orbitals)
     return history
 
 

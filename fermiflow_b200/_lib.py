@@ -62,6 +62,7 @@ SIGNATURES = {
     "ff_wavefunction_ratio_work_size": ([_M, _LL, _I, C.POINTER(_LL)], C.c_int),
     "ff_wavefunction_ratio": ([_M, _P, _LL, _P, _P, _I, _P, _P, _P, _P, _P], C.c_int),
     "ff_momentum_accumulate": ([_P, _P, _P, _LL, _I, C.POINTER(FFMomGrid), _P, _LL, _P], C.c_int),
+    "ff_density_matrix_accumulate": ([_P, _LL, _I, _I, _I, _P, _P, _P, _I, _P, _LL, _P], C.c_int),
     "ff_swap_ratio_work_size": ([_M, _LL, _I, C.POINTER(_LL)], C.c_int),
     "ff_swap_ratio": ([_M, _P, _LL, _P, _P, _LL, _P, C.POINTER(FFSwapRegions), _P, _P, _P, _P], C.c_int),
     "ff_swap_accumulate": ([_P, _P, _LL, _I, _I, _I, _P, _LL, _P], C.c_int),

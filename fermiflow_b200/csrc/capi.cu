@@ -9,6 +9,7 @@
 #include "ff_observables.cuh"
 #include "ff_momentum.cuh"
 #include "ff_renyi.cuh"
+#include "ff_density_matrix.cuh"
 
 namespace ffc {
 

@@ -1,7 +1,8 @@
 """Spin-resolved one-body density and pair correlations of sampled walkers (C ABI ff_observables), the momentum
 distribution and one-body coherence from signed wave-function ratios (C ABI ff_wavefunction_ratio,
-ff_momentum_accumulate), and the second Rényi entropy of spatial regions from replica swap ratios (C ABI ff_swap_ratio,
-ff_swap_accumulate).
+ff_momentum_accumulate), the second Rényi entropy of spatial regions from replica swap ratios (C ABI ff_swap_ratio,
+ff_swap_accumulate), and the one-body density matrix in the oscillator basis with its natural-orbital occupations
+(C ABI ff_wavefunction_ratio, ff_density_matrix_accumulate).
 
     est = DensityEstimator(n_up, n_dn, extent=6.0)
     with torch.no_grad():
@@ -24,6 +25,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib as L
+from .orbitals import HO2D
 
 # sections of the count vector (include/fermiflow_b200.h ff_observables): name, channels, square grid
 _SECTIONS = (("density", 2, True), ("radial", 2, False), ("separation", 3, False), ("rotated", 2, True))
@@ -54,13 +56,15 @@ def observables(x, n_up, n_dn, extent, n_xy, r_max, n_r, n_rot, counts):
 
 class _BatchMeans:
     """Running sums of per-batch vectors v_k (each a sum over the W_k walkers of batch k) for batch-means errors:
-    [sum v_k, sum v_k² / W_k, sum W_k, calls] in one float64 vector on `device`, so that ranks merge with one
-    all-reduce."""
+    [sum v_k, sum v_k² / W_k, extra sums, sum W_k, calls] in one float64 vector on `device`, so that ranks merge with
+    one all-reduce."""
 
-    def _init_state(self, n_values, device):
+    def _init_state(self, n_values, device, n_extra=0):
+        """`n_extra` further running sums (after the squares, before the walker and call counts) for an estimator's
+        own second moments; they travel in the same all-reduce."""
         self.device = torch.device(device)
         self._n_values = int(n_values)
-        self.state = torch.zeros(2 * self._n_values + 2, dtype=torch.float64, device=self.device)
+        self.state = torch.zeros(2 * self._n_values + int(n_extra) + 2, dtype=torch.float64, device=self.device)
 
     def _merge(self, values, walkers):
         """Add one batch of `walkers` walkers whose values summed to `values` (plain torch)."""
@@ -489,4 +493,187 @@ def sample_renyi(model, n_up, n_dn, batch, batches, a, kind, path):
         res = est.result()
         print("renyi: %d pairs saved to %s; S2 per %s: %s" % (res["pairs"], path, kind, ", ".join(
             "%g: %.4g +- %.2g" % (v, s, e) for v, s, e in zip(est.a, res["S2"], res["S2_err"]))))
+    return est
+
+
+def density_matrix_layout(K):
+    """{section: (offset, shape)} of the sums of ff_density_matrix_accumulate (include/fermiflow_b200.h) for K orbitals
+    and their length 2 K² + 3."""
+    out, off = {}, 0
+    for name, shape in (("matrix", (2, K, K)), ("records", (2,)), ("skipped", (1,))):
+        out[name] = (off, shape)
+        off += math.prod(shape)
+    return out, off
+
+
+def density_matrix_accumulate(x, particle, disp, w, n_up, n_dn, n_orb, sums):
+    """ff_density_matrix_accumulate on CUDA walkers x (float64 [B, n_up + n_dn, 2]) and records (particle int32 [B, M],
+    disp float64 [B, M, 2], w float64 [B, M]): ADDS the sums to `sums` (float64, the layout of density_matrix_layout)."""
+    if particle.dim() != 2:
+        raise ValueError("particle must be [B, M], got %s" % (tuple(particle.shape),))
+    B, M = particle.shape
+    if x.dim() != 3 or tuple(x.shape) != (B, n_up + n_dn, 2) or tuple(disp.shape) != (B, M, 2) \
+            or tuple(w.shape) != (B, M):
+        raise ValueError("x must be [%d, %d, 2], disp [%d, %d, 2] and w [%d, %d], got %s, %s and %s"
+                         % (B, n_up + n_dn, B, M, B, M, tuple(x.shape), tuple(disp.shape), tuple(w.shape)))
+    L.check(L.lib().ff_density_matrix_accumulate(L.ptr(x), B, int(n_up), int(n_dn), M, L.ptr(particle, torch.int32),
+                                                 L.ptr(disp), L.ptr(w), int(n_orb), L.ptr(sums), sums.numel(),
+                                                 L.stream()))
+    return sums
+
+
+class DensityMatrixEstimator(_BatchMeans):
+    """Spin-resolved one-body density matrix of a VMC model (GSVMC or BetaVMC) in the first K = (shells + 1)(shells + 2)
+    / 2 HO2D orbitals, D^c_ab = ∫∫ φ_a(r) ρ1_c(r, r′) φ_b(r′) dr dr′, and its spectrum, the natural-orbital occupations.
+    A Slater determinant has occupations of exactly 1 and 0; correlation and Wigner localisation spread them out.
+
+    A record is one walker x ~ |ψ|², one particle i drawn uniformly from all n and one point r′ drawn from the Gaussian
+    q(r′) = exp(−|r′|² / 2σ²) / (2πσ²) about the trap centre; its ratio is ρ = ψ(x with r_i → r′) / ψ(x)
+    (model.wavefunction_ratio, sign included) and its channel c = (i ≥ n_up).  With `moves` = M records per walker and
+    W walkers in all:
+
+      D^c_ab ≈ n / (M W) Σ_{records of c} ½ [φ_a(r_i) φ_b(r′) + φ_b(r_i) φ_a(r′)] ρ / q(r′)
+
+    ψ(…r′…) φ_b(r′) decays like exp(−|r′|²), so the weight's second moment ∫ (ψ φ_b)² / q is finite only for σ > 1/2.
+    σ = 1.5 is the default: it keeps that margin, and the Gaussian still reaches r′ ≈ 4, where the shell-7 orbitals
+    and the outer particles of the dot have their weight.  A narrower q samples them rarely with large weights; a wider
+    one spends records where ψ is negligible.  On a B200, with the benchmark's random flow at N = 20 and 12 + 0 and
+    4 batches of 65536 walkers (scripts/dev_natural_orbitals_timing.py), σ = 1.5 gave the smallest error of the trace
+    among σ = 1, 1.5, 2 and 3: 0.022 and 0.029 against 0.18 and 0.097 at σ = 1 and 0.068 and 0.041 at σ = 2.  The
+    estimate is unbiased for every σ > 1/2.
+
+    Tr D^c = Tr(P ρ1_c) ≤ n_c, P the projector onto the basis; it equals n_c only when ρ1 lies in the span of the K
+    orbitals, so `trace` is the basis coverage.  For BetaVMC each walker uses its own occupation row, and the estimate is
+    D of the mixed state.
+
+    Errors are batch means over the calls of accumulate(), weighted by each call's walker count (NaN with fewer than
+    two calls).  The occupation errors use the first-order delta method, λ_k = v_kᵀ D v_k with the eigenvector v_k
+    held fixed, and the covariance of the K(K + 1)/2 independent entries of D across batches, kept in the state
+    (about 7 MB at K = 36), so that allreduce() stays one all-reduce.  Two limits: near-degenerate occupations (for
+    example symmetry partners in a circular dot) have only first-order individual errors, since their eigenvectors mix
+    from batch to batch, while their sum is robust; and the eigenvalues of a noisy matrix are biased at O(error²) (the
+    largest pushed up, the smallest down).
+
+    result() returns float64 numpy arrays:
+      density_matrix [2][K][K]      D^c (+ _err, per entry)
+      trace [2]                     Tr D^c (+ _err)
+      occupations [2][K]            eigenvalues of D^c in descending order (+ _err)
+      natural_orbitals [2][K][K]    columns: the eigenvectors in the HO2D basis, largest component positive
+      shell_weight [2][K][shells+1] squared coefficients of natural orbital k summed per oscillator shell nx + ny
+      orbital_quanta [K][2]         (nx, ny) of the basis orbitals
+    and walkers, calls, moves, sigma, n_up, n_dn.
+    """
+
+    def __init__(self, n_up, n_dn, shells=7, sigma=1.5, moves=8, device=torch.device("cuda")):
+        if n_up < 0 or n_dn < 0 or n_up + n_dn < 1:
+            raise ValueError("bad particle numbers %d/%d" % (n_up, n_dn))
+        if not 0 <= shells <= 7:
+            raise ValueError("shells must be in [0, 7] (HO2D has 36 orbitals), got %d" % shells)
+        if not (math.isfinite(sigma) and sigma > 0.5):
+            raise ValueError("sigma must be finite and above 1/2 (the weights' variance is infinite below), got %r"
+                             % (sigma,))
+        if moves < 1:
+            raise ValueError("moves must be at least 1, got %d" % moves)
+        self.n_up, self.n_dn = int(n_up), int(n_dn)
+        self.shells, self.sigma, self.moves = int(shells), float(sigma), int(moves)
+        self.K = K = (self.shells + 1) * (self.shells + 2) // 2
+        self.layout, self.n_sums = density_matrix_layout(K)
+        self._tri = torch.triu_indices(K, K)                            # the independent entries a <= b
+        self._P = self._tri.shape[1]
+        self._tri_dev = self._tri.to(device)
+        # the sums, then Σ_batches m m^T / W of the independent entries m of each channel (the covariance of D)
+        self._init_state(self.n_sums, device, n_extra=2 * self._P * self._P)
+        self._buf = None
+
+    def accumulate(self, model, x, generator=None):
+        """Add one batch of independent walkers x (CUDA float64 [B, n_up + n_dn, 2], drawn by model.sample at the
+        current parameters): `moves` records per walker, drawn on the device (torch.randint / torch.randn with
+        `generator`); no host synchronisation."""
+        n = self.n_up + self.n_dn
+        if x.dim() != 3 or x.shape[-1] != 2 or x.shape[1] != n:
+            raise ValueError("x must be [B, %d, 2], got %s" % (n, tuple(x.shape)))
+        if not x.is_cuda:
+            raise RuntimeError("DensityMatrixEstimator needs CUDA walkers (got %s); no CPU fallback" % x.device)
+        x = x.detach().contiguous()
+        B, M, dev = x.shape[0], self.moves, x.device
+        particle = torch.randint(0, n, (B, M), device=dev, dtype=torch.int32, generator=generator)
+        rp = self.sigma * torch.randn(B, M, 2, device=dev, dtype=torch.float64, generator=generator)
+        disp = rp - torch.gather(x, 1, particle.long()[..., None].expand(B, M, 2))
+        ratio = model.wavefunction_ratio(x, particle, disp)
+        s2 = self.sigma ** 2
+        w = ratio * ((2 * math.pi * s2) * torch.exp((rp * rp).sum(-1) / (2 * s2)))           # ρ / q(r′)
+        if self._buf is None or self._buf.device != dev:
+            self._buf = torch.empty(self.n_sums, dtype=torch.float64, device=dev)
+        self._buf.zero_()
+        density_matrix_accumulate(x, particle, disp, w, self.n_up, self.n_dn, self.K, self._buf)
+        self._add_batch(self._buf, B)
+
+    def _add_batch(self, sums, walkers):
+        """Merge the sums of one batch of `walkers` walkers into the running state (plain torch)."""
+        if walkers <= 0:
+            return
+        v = sums.to(self.state.device, torch.float64)
+        self._merge(v, walkers)
+        K, P = self.K, self._P
+        m = v[:2 * K * K].view(2, K, K)[:, self._tri_dev[0], self._tri_dev[1]]              # [2, P]
+        o = 2 * self._n_values
+        self.state[o:o + 2 * P * P].view(2, P, P).baddbmm_(m[:, :, None], m[:, None, :], alpha=1.0 / walkers)
+
+    def result(self):
+        """dict of float64 numpy arrays (see the class docstring)."""
+        mean, err, W, Kc, _ = self._per_walker()
+        K, P = self.K, self._P
+        norm = (self.n_up + self.n_dn) / self.moves
+        m = mean[:2 * K * K].view(2, K, K)
+        o = 2 * self._n_values
+        mt = m[:, self._tri_dev[0], self._tri_dev[1]]
+        # covariance of the mean of the independent entries of D, from the batch means as in _per_walker
+        cov = (self.state[o:o + 2 * P * P].view(2, P, P) - W * mt[:, :, None] * mt[:, None, :]) \
+            * (norm * norm / ((Kc - 1.0) * W))
+        D, D_err, cov, W, Kc = (t.cpu() for t in (norm * m, norm * err[:2 * K * K].view(2, K, K), cov, W, Kc))
+        ta, tb = self._tri
+        diag = (ta == tb).to(torch.float64)
+        evals, evecs = torch.linalg.eigh(D)
+        occ, V = evals.flip(-1), evecs.flip(-1)
+        big = V.abs().argmax(-2, keepdim=True)
+        V = V * torch.where(torch.gather(V, -2, big) < 0, -1.0, 1.0)
+        G = V[:, ta, :] * V[:, tb, :] * (2.0 - diag)[None, :, None]                         # dλ_k / dD_ab, [2, P, K]
+        nan = torch.tensor(float("nan"), dtype=torch.float64)
+
+        def sd(var):
+            return torch.where(Kc >= 2, var.clamp_min(0.0).sqrt(), nan)
+
+        quanta = torch.tensor([(orb.nx, orb.ny) for orb in HO2D().orbitals[:K]], dtype=torch.float64)
+        shell = torch.nn.functional.one_hot(quanta.sum(1).long(), self.shells + 1).to(torch.float64)   # [K, shells+1]
+        out = dict(density_matrix=D, density_matrix_err=D_err,
+                   trace=D.diagonal(dim1=1, dim2=2).sum(-1), trace_err=sd(torch.einsum("p,cpq,q->c", diag, cov, diag)),
+                   occupations=occ, occupations_err=sd(torch.einsum("cpk,cpq,cqk->ck", G, cov, G)),
+                   natural_orbitals=V, shell_weight=torch.einsum("cak,as->cks", V * V, shell), orbital_quanta=quanta,
+                   walkers=W, calls=Kc)
+        f64 = dict(dtype=torch.float64)
+        out["moves"], out["sigma"] = torch.tensor(float(self.moves), **f64), torch.tensor(self.sigma, **f64)
+        out["n_up"], out["n_dn"] = torch.tensor(float(self.n_up), **f64), torch.tensor(float(self.n_dn), **f64)
+        return {k: v.numpy() for k, v in out.items()}
+
+
+def sample_natural_orbitals(model, n_up, n_dn, batch, batches, shells, path):
+    """The --natural-orbitals option of the drivers: `batches` batches of `batch` walkers from model.sample at the
+    current parameters, `moves` = 8 one-particle moves per walker, merged over ranks and saved to `path` by rank 0."""
+    est = DensityMatrixEstimator(n_up, n_dn, shells=shells, device=next(model.parameters()).device)
+    with torch.no_grad():
+        for _ in range(batches):
+            _, x = model.sample((batch,))
+            est.accumulate(model, x)
+    est.allreduce()
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0:
+        est.save(path)
+        res = est.result()
+        lines = []
+        for c, (name, nc) in enumerate((("up", n_up), ("down", n_dn))):
+            lead = ", ".join("%.4f +- %.2g" % (v, e) for v, e in
+                             list(zip(res["occupations"][c], res["occupations_err"][c]))[:min(nc + 2, est.K)])
+            lines.append("%s: trace %.4f +- %.2g of %d, leading occupations %s"
+                         % (name, res["trace"][c], res["trace_err"][c], nc, lead))
+        print("natural orbitals: %d walkers, %d orbitals saved to %s; %s" % (res["walkers"], est.K, path,
+                                                                            "; ".join(lines)))
     return est

@@ -204,6 +204,30 @@ typedef struct ff_mom_grid {
 int ff_momentum_accumulate(const double* ratio, const int* particle, const double* disp, long long R, int n_up,
                            const ff_mom_grid* g, double* sums, long long n_sums, void* stream);
 
+/* One-body density matrix in the first K HO2D orbitals phi_0 ... phi_{K-1} (orbitals.py:89 order, shells 0 ... 7,
+ * phi_a(r) = pi^-1/2 exp(-r^2/2) h_nx(x) h_ny(y)), per spin channel c:
+ *   D^c_ab = integral of phi_a(r) rho1_c(r, r') phi_b(r') dr dr'.
+ * Records r = b M + m as in ff_wavefunction_ratio: walker b of x [B][n_up+n_dn][2], particle i = particle[b][m]
+ * (int32 [B][M]), displacement disp[b][m] ([B][M][2]) and weight w[b][m] ([B][M]).  The moved position is
+ * r' = r_i + disp with one rounded add per coordinate, the position ff_wavefunction_ratio moves the particle to.  A
+ * record's channel is c = (i >= n_up).  With particles drawn uniformly from all n, r' drawn from a density q(r') and
+ * w = ratio / q(r'), ratio = psi(x with r_i -> r') / psi(x) of ff_wavefunction_ratio,
+ *   D^c_ab ~= n / (M W) sum over the records of channel c of 1/2 [phi_a(r_i) phi_b(r') + phi_b(r_i) phi_a(r')] w
+ * over W walkers; the kernel knows nothing about q and sums whatever w it is given.  Layout of sums
+ * (n_sums = 2 K^2 + 3):
+ *   [2][K][K] the symmetrised sums above (index [c][a][b], both triangles written, so the matrices are exactly
+ *   symmetric), [2] records per channel, [1] skipped records
+ * (counts as doubles, exact below 2^53).  A record whose particle index lies outside [0, n) is skipped: neither x nor
+ * w is read for it (nothing synchronises the host to check the indices).  ACCUMULATES into sums (the caller zeroes
+ * them).  Fixed summation order without floating-point atomics: two calls on the same inputs give bit-identical sums.
+ * A non-finite w propagates into the sums of its channel.  Scratch comes from the stream-ordered allocator; 8-byte
+ * alignment suffices for every buffer.  -1 for bad particle numbers (n_up, n_dn >= 0, at most 36 each, n >= 1), B or
+ * M < 1, K = n_orb outside [1, 36], n_sums not equal to the layout size, null buffers, and a tile of records whose
+ * tables (32 (2 K + 37) doubles) do not fit in the shared memory of one block. */
+int ff_density_matrix_accumulate(const double* x, long long B, int n_up, int n_dn, int M,
+                                 const int* particle /* int32 [B][M] */, const double* disp /* [B][M][2] */,
+                                 const double* w /* [B][M] */, int n_orb, double* sums, long long n_sums, void* stream);
+
 /* Replica swap ratios of spatial regions, for the second Renyi entropy (no reference counterpart):
  *   exp(-S2(A)) = Tr rho_A^2 = < psi(x') psi(y') / (psi(x) psi(y)) >,   x, y independent draws from rho,
  * with psi(x) = sign(det Phi_up(z) det Phi_dn(z)) exp(log p(x) / 2) as in ff_wavefunction_ratio.  Pair p is the two
