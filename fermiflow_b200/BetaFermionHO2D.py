@@ -12,7 +12,7 @@ from .VMC import BetaVMC
 from .base_dist import FreeFermion
 from .equivariant_funs import Backflow
 from .flow import CNF
-from .observables import sample_density, sample_momentum, sample_natural_orbitals, sample_renyi
+from .observables import add_driver_options, run_driver_options
 from .orbitals import HO2D
 from .potentials import HO, CoulombPairPotential
 
@@ -35,27 +35,7 @@ def main(argv=None):
     p.add_argument("--iternum", type=int, default=1000)
     p.add_argument("--batch", type=int, default=8000)
     p.add_argument("--lr", type=float, default=1e-2)
-    p.add_argument("--density", metavar="FILE", help="after training, save the density and pair correlations of "
-                   "freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.DensityEstimator)")
-    p.add_argument("--density-batches", type=int, default=16, help="batches of --batch walkers for --density")
-    p.add_argument("--density-extent", type=float, default=6.0, help="half-width of the density grids")
-    p.add_argument("--momentum", metavar="FILE", help="after training, save the momentum distribution and one-body "
-                   "coherence of freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.MomentumEstimator)")
-    p.add_argument("--momentum-batches", type=int, default=16, help="batches of --batch walkers for --momentum")
-    p.add_argument("--momentum-kmax", type=float, default=4.0, help="half-width of the momentum grid")
-    p.add_argument("--renyi", metavar="FILE", help="after training, save the second Renyi entropy of spatial regions, "
-                   "from replica swaps of freshly sampled walkers, to FILE (.npz, fermiflow_b200.observables.RenyiEstimator)")
-    p.add_argument("--renyi-batches", type=int, default=16, help="batches of --batch walkers for --renyi")
-    p.add_argument("--renyi-a", type=lambda s: [float(v) for v in s.split(",")], default=[0.5, 1.0, 1.5, 2.0, 2.5, 3.0],
-                   help="comma-separated region parameters for --renyi: disk radii or half-plane edges x < a")
-    p.add_argument("--renyi-kind", choices=("disk", "halfplane"), default="disk", help="region kind for --renyi")
-    p.add_argument("--natural-orbitals", metavar="FILE", help="after training, save the one-body density matrix in the "
-                   "HO2D basis and its natural-orbital occupations, from one-particle moves of freshly sampled walkers, to "
-                   "FILE (.npz, fermiflow_b200.observables.DensityMatrixEstimator)")
-    p.add_argument("--natural-orbitals-batches", type=int, default=16,
-                   help="batches of --batch walkers for --natural-orbitals")
-    p.add_argument("--natural-orbitals-shells", type=int, default=7,
-                   help="oscillator shells 0 ... S of the basis for --natural-orbitals ((S + 1)(S + 2) / 2 orbitals)")
+    add_driver_options(p)
     args = p.parse_args(argv)
 
     device = torch.device("cuda:%d" % args.cuda)
@@ -82,15 +62,7 @@ def main(argv=None):
         print("iter: %03d" % i, "F:", model.F, "F_std:", model.F_std, "E:", model.E, "E_std:", model.E_std,
               "S:", model.S, "S_analytical:", model.S_analytical,
               "Instant speed (hours per 100 iters):", (time.time() - start) * 100 / 3600)
-    if args.density:
-        sample_density(model, args.nup, args.ndown, args.batch, args.density_batches, args.density_extent, args.density)
-    if args.momentum:
-        sample_momentum(model, args.nup, args.ndown, args.batch, args.momentum_batches, args.momentum_kmax, args.momentum)
-    if args.renyi:
-        sample_renyi(model, args.nup, args.ndown, args.batch, args.renyi_batches, args.renyi_a, args.renyi_kind, args.renyi)
-    if args.natural_orbitals:
-        sample_natural_orbitals(model, args.nup, args.ndown, args.batch, args.natural_orbitals_batches,
-                                args.natural_orbitals_shells, args.natural_orbitals)
+    run_driver_options(model, args)
     return history
 
 

@@ -77,24 +77,31 @@ class _LogpFromSweep(torch.autograd.Function):
         return (None, None, None, None, None, None, *gparams)
 
 
+def _ratio_setup(cnf, x, n_up, work_size, rows, cols):
+    """The start of both ratio entry points: x [B, n, 2] checked, detached and contiguous, the model struct of cnf for
+    its n particles, and the work buffer that work_size (ff_wavefunction_ratio_work_size or ff_swap_ratio_work_size)
+    asks for `rows` x `cols` records."""
+    x = x.detach().contiguous()
+    if x.dim() != 3 or x.shape[-1] != 2:
+        raise ValueError("x must be [B, n, 2], got %s" % (tuple(x.shape),))
+    model = cnf._model(x.shape[1], n_up=n_up)
+    nw = C.c_longlong()
+    L.check(work_size(C.byref(model), rows, cols, C.byref(nw)))
+    return x, model, torch.empty(nw.value, dtype=torch.float64, device=x.device)
+
+
 def _wavefunction_ratio(cnf, x, orb, walker_state, n_up, particle, disp):
     """psi(x_b with r_i -> r_i + s) / psi(x_b) for every record (b, m), i = particle[b, m], s = disp[b, m], with the
     sign of the Slater determinants (C ABI ff_wavefunction_ratio).  x [B, n, 2], particle integer [B, M], disp
     [B, M, 2], all on the device; returns ratio [B, M].  A particle index outside [0, n) gives NaN."""
-    x = x.detach().contiguous()
-    if x.dim() != 3 or x.shape[-1] != 2:
-        raise ValueError("x must be [B, n, 2], got %s" % (tuple(x.shape),))
-    B, n, _ = x.shape
+    B = x.shape[0]
     if particle.dim() != 2 or particle.shape[0] != B or tuple(disp.shape) != (B, particle.shape[1], 2):
         raise ValueError("particle must be [B, M] and disp [B, M, 2] for B = %d walkers, got %s and %s"
                          % (B, tuple(particle.shape), tuple(disp.shape)))
     M = particle.shape[1]
     p32 = particle.to(torch.int32).contiguous()
     disp = disp.detach().contiguous()
-    model = cnf._model(n, n_up=n_up)
-    nw = C.c_longlong()
-    L.check(L.lib().ff_wavefunction_ratio_work_size(C.byref(model), B, M, C.byref(nw)))
-    work = torch.empty(nw.value, dtype=torch.float64, device=x.device)
+    x, model, work = _ratio_setup(cnf, x, n_up, L.lib().ff_wavefunction_ratio_work_size, B, M)
     ratio = torch.empty(B, M, dtype=torch.float64, device=x.device)
     L.check(L.lib().ff_wavefunction_ratio(C.byref(model), L.ptr(x), B, L.ptr(orb, torch.int32),
                                           L.ptr(walker_state, torch.int32) if walker_state is not None else None,
@@ -110,25 +117,18 @@ def _swap_ratio(cnf, x, orb, walker_state, n_up, pairs, a, kind):
     and y' the two walkers with their particles in region q swapped (C ABI ff_swap_ratio).  x [B, n, 2] and pairs
     integer [P, 2] on the device, a: Q region parameters (disk radii or half-plane edges), kind "disk" or "halfplane";
     returns ratio [P, Q] and sector int32 [P, 2, Q].  A walker index outside [0, B) gives NaN and sector -1."""
-    x = x.detach().contiguous()
-    if x.dim() != 3 or x.shape[-1] != 2:
-        raise ValueError("x must be [B, n, 2], got %s" % (tuple(x.shape),))
     if pairs.dim() != 2 or pairs.shape[1] != 2:
         raise ValueError("pairs must be [P, 2], got %s" % (tuple(pairs.shape),))
     if kind not in _REGION_KINDS:
         raise ValueError("kind must be one of %s, got %r" % (sorted(_REGION_KINDS), kind))
-    B, n, _ = x.shape
     P = pairs.shape[0]
     av = (C.c_double * len(a))(*[float(v) for v in a])
     reg = L.FFSwapRegions(_REGION_KINDS[kind], len(a), av)
     p32 = pairs.to(torch.int32).contiguous()
-    model = cnf._model(n, n_up=n_up)
-    nw = C.c_longlong()
-    L.check(L.lib().ff_swap_ratio_work_size(C.byref(model), P, len(a), C.byref(nw)))
-    work = torch.empty(nw.value, dtype=torch.float64, device=x.device)
+    x, model, work = _ratio_setup(cnf, x, n_up, L.lib().ff_swap_ratio_work_size, P, len(a))
     ratio = torch.empty(P, len(a), dtype=torch.float64, device=x.device)
     sector = torch.empty(P, 2, len(a), dtype=torch.int32, device=x.device)
-    L.check(L.lib().ff_swap_ratio(C.byref(model), L.ptr(x), B, L.ptr(orb, torch.int32),
+    L.check(L.lib().ff_swap_ratio(C.byref(model), L.ptr(x), x.shape[0], L.ptr(orb, torch.int32),
                                   L.ptr(walker_state, torch.int32) if walker_state is not None else None,
                                   P, L.ptr(p32, torch.int32), C.byref(reg), L.ptr(ratio), L.ptr(sector, torch.int32),
                                   L.ptr(work), L.stream()))

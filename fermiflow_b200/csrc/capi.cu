@@ -94,6 +94,28 @@ int RadialTables::build(const ff_model* m, cudaStream_t stream, ff::FlowArgs& a)
     return 0;
 }
 
+// Two-stage fixed-order sums of the estimators: scratch for `grid` rows of n_sums doubles, launch_partial(partial)
+// launches the caller's partial kernel (one row per CTA) on st, reduce_partial_rows_kernel adds the rows in order to
+// sums, and the scratch is freed on every path.  `what` names the kernels in the error message.
+template <class LaunchPartial>
+static int partial_sums(long long grid, long long n_sums, double* sums, const DevInfo& di, cudaStream_t st,
+                        const char* what, LaunchPartial launch_partial) {
+    double* partial = nullptr;
+    FF_CUDA(cudaMallocAsync((void**)&partial, (size_t)grid * n_sums * sizeof(double), st));
+    launch_partial(partial);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    cudaError_t le = cudaGetLastError();
+    if (le == cudaSuccess) {
+        const long long rgrid = std::min<long long>((n_sums + 255) / 256, (long long)di.sms * 8);
+        ff::reduce_partial_rows_kernel<<<(unsigned)rgrid, 256, 0, st>>>(partial, (int)grid, n_sums, sums);
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        le = cudaGetLastError();
+    }
+    cudaFreeAsync(partial, st);
+    if (le != cudaSuccess) return cuda_fail(le, what);
+    return 0;
+}
+
 }  // namespace ffc
 
 using namespace ffc;

@@ -13,7 +13,7 @@
 //                                  owns up to kDmUnits "units" -- a cell a <= b (both channels), the records per
 //                                  channel, the skipped records -- and sums every record of its chunk in order in
 //                                  registers; at the end it writes both triangles of its cells to the CTA's partial row.
-//   momentum_reduce_kernel         sums[q] += sum over g = 0, 1, ... of partial[g][q], in CTA order.
+//   reduce_partial_rows_kernel (ff_misc.cuh)  sums[q] += sum over g = 0, 1, ... of partial[g][q], in CTA order.
 // A record whose particle index lies outside [0, n) reads neither x nor w; it only counts as skipped.
 #pragma once
 #include "ff_common.cuh"

@@ -1,6 +1,6 @@
 // Stand-alone stages of the path: backflow evaluation, Slater log|det| with derivatives,
 // the Metropolis sampler of the free-fermion base distribution, potentials, Boltzmann
-// occupation sampling and an FP64 throughput probe.
+// occupation sampling, the ordered reduction of per-CTA partial sums and an FP64 throughput probe.
 #pragma once
 #include "ff_common.cuh"
 #include "ff_slater.cuh"
@@ -755,6 +755,16 @@ __global__ void occupation_fill_kernel(const int* counts, int S, long long B, in
         const long long st = start; const int c = counts[s];
         for (int k = threadIdx.x; k < c; k += blockDim.x) if (st + k < B) state[st + k] = s;
         __syncthreads();
+    }
+}
+
+// sums[q] += sum over p = 0, 1, ... of partial[p][q], in row order: the fixed-order second stage of the estimators'
+// partial-sum kernels (ff_momentum_accumulate, ff_swap_accumulate, ff_density_matrix_accumulate), one row per CTA
+__global__ void __launch_bounds__(256) reduce_partial_rows_kernel(const double* partial, int parts, long long n_sums, double* sums) {
+    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < n_sums; q += (long long)gridDim.x * blockDim.x) {
+        double s = 0.0;
+        for (int p = 0; p < parts; ++p) s += partial[(long long)p * n_sums + q];
+        sums[q] += s;
     }
 }
 

@@ -16,7 +16,7 @@
 //                            rho J0(k_j |s|) in shared memory; then each thread owns a fixed set of output "units"
 //                            (a k cell, a radial point, an |s| bin, ...) for both channels, sums the tile's records in
 //                            order and adds the tile sum to its units in the CTA's partial row.
-//   momentum_reduce_kernel   sums[q] += sum over g = 0, 1, ... of partial[g][q], in CTA order.
+//   reduce_partial_rows_kernel (ff_misc.cuh)  sums[q] += sum over g = 0, 1, ... of partial[g][q], in CTA order.
 // The grid (and so the rounding) depends only on R, the grid sizes and the device: two calls on the same inputs give
 // bit-identical sums.
 #pragma once
@@ -177,14 +177,6 @@ __global__ void __launch_bounds__(kMomThreads) momentum_partial_kernel(const Mom
             part[o] += s0;
             part[o + st] += s1;
         }
-    }
-}
-
-__global__ void __launch_bounds__(256) momentum_reduce_kernel(const double* partial, int parts, long long n_sums, double* sums) {
-    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < n_sums; q += (long long)gridDim.x * blockDim.x) {
-        double s = 0.0;
-        for (int p = 0; p < parts; ++p) s += partial[(long long)p * n_sums + q];
-        sums[q] += s;
     }
 }
 

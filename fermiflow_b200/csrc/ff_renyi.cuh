@@ -18,7 +18,7 @@
 //   renyi_partial_kernel   CTA g takes pairs [g chunk, (g + 1) chunk) in tiles of kRenyiTile pairs; each thread owns
 //                          fixed cells (q, sector) or (q, skipped), adds the tile's records in order and the tile sum to
 //                          its cells in the CTA's partial row
-//   momentum_reduce_kernel sums[i] += sum over g = 0, 1, ... of partial[g][i], in CTA order (ff_momentum.cuh)
+//   reduce_partial_rows_kernel (ff_misc.cuh)  sums[i] += sum over g = 0, 1, ... of partial[g][i], in CTA order
 // The grid depends only on P, Q, n_sec and the device: two calls on the same inputs give bit-identical sums.
 #pragma once
 #include "ff_common.cuh"

@@ -32,16 +32,20 @@ _SECTIONS = (("density", 2, True), ("radial", 2, False), ("separation", 3, False
 _OUTSIDE = 9
 
 
+def _layout(sections):
+    """({name: (offset, shape)}, length) of the sections ((name, shape), ...) laid out one after the other."""
+    out, off = {}, 0
+    for name, shape in sections:
+        out[name] = (off, shape)
+        off += math.prod(shape)
+    return out, off
+
+
 def count_layout(n_xy, n_r, n_rot):
     """{section: (offset, shape)} of the count vector and the offset of the 9 outside counters; the order is the one
     include/fermiflow_b200.h documents for ff_observables."""
     nb = dict(density=n_xy, radial=n_r, separation=n_r, rotated=n_rot)
-    out, off = {}, 0
-    for name, nch, square in _SECTIONS:
-        shape = (nch, nb[name], nb[name]) if square else (nch, nb[name])
-        out[name] = (off, shape)
-        off += math.prod(shape)
-    return out, off
+    return _layout((name, (nch, nb[name], nb[name]) if square else (nch, nb[name])) for name, nch, square in _SECTIONS)
 
 
 def observables(x, n_up, n_dn, extent, n_xy, r_max, n_r, n_rot, counts):
@@ -58,6 +62,41 @@ class _BatchMeans:
     """Running sums of per-batch vectors v_k (each a sum over the W_k walkers of batch k) for batch-means errors:
     [sum v_k, sum v_k² / W_k, extra sums, sum W_k, calls] in one float64 vector on `device`, so that ranks merge with
     one all-reduce."""
+
+    def __init__(self, n_up, n_dn):
+        if n_up < 0 or n_dn < 0 or n_up + n_dn < 1:
+            raise ValueError("bad particle numbers %d/%d" % (n_up, n_dn))
+        self.n_up, self.n_dn = int(n_up), int(n_dn)
+        self._buf = None
+
+    @staticmethod
+    def _check_moves(moves):
+        if moves < 1:
+            raise ValueError("moves must be at least 1, got %d" % moves)
+        return int(moves)
+
+    def _check_walkers(self, x):
+        n = self.n_up + self.n_dn
+        if x.dim() != 3 or x.shape[-1] != 2 or x.shape[1] != n:
+            raise ValueError("x must be [B, %d, 2], got %s" % (n, tuple(x.shape)))
+        if not x.is_cuda:
+            raise RuntimeError("%s needs CUDA walkers (got %s); no CPU fallback" % (type(self).__name__, x.device))
+
+    def _zeroed_sums(self, n, device, dtype=torch.float64):
+        """The buffer for the sums of one batch on `device`, zeroed; allocated again only when the device changes."""
+        if self._buf is None or self._buf.device != device:
+            self._buf = torch.empty(n, dtype=dtype, device=device)
+        return self._buf.zero_()
+
+    def _section(self, t, name):
+        """Section `name` of self.layout in the vector t, in its shape."""
+        off, shape = self.layout[name]
+        return t[off:off + math.prod(shape)].reshape(shape)
+
+    @staticmethod
+    def _stderr(var, calls):
+        """sqrt(var), NaN with fewer than two calls."""
+        return torch.where(calls >= 2, var.sqrt(), torch.full_like(var, float("nan")))
 
     def _init_state(self, n_values, device, n_extra=0):
         """`n_extra` further running sums (after the squares, before the walker and call counts) for an estimator's
@@ -90,9 +129,7 @@ class _BatchMeans:
         s1, s2 = self.state[:nv], self.state[nv:2 * nv]
         W, K = self.state[-2], self.state[-1]
         mean = s1 / W
-        var = (s2 - W * mean * mean).clamp_min(0.0) / ((K - 1.0) * W)
-        err = torch.where(K >= 2, var.sqrt(), torch.full_like(var, float("nan")))
-        return mean, err, W, K, s2
+        return mean, self._stderr((s2 - W * mean * mean).clamp_min(0.0) / ((K - 1.0) * W), K), W, K, s2
 
     def save(self, path):
         """np.savez of result()."""
@@ -124,9 +161,7 @@ class DensityEstimator(_BatchMeans):
     """
 
     def __init__(self, n_up, n_dn, extent, n_xy=64, r_max=None, n_r=128, n_rot=64, device=torch.device("cuda")):
-        if n_up < 0 or n_dn < 0 or n_up + n_dn < 1:
-            raise ValueError("bad particle numbers %d/%d" % (n_up, n_dn))
-        self.n_up, self.n_dn = int(n_up), int(n_dn)
+        super().__init__(n_up, n_dn)
         self.extent = float(extent)
         self.r_max = float(extent if r_max is None else r_max)
         self.n_xy, self.n_r, self.n_rot = int(n_xy), int(n_r), int(n_rot)
@@ -134,15 +169,12 @@ class DensityEstimator(_BatchMeans):
         self.n_counts = self.n_bins + _OUTSIDE
         # [sum of counts, sum over calls of counts² / walkers, walkers, calls]: one vector, one all-reduce
         self._init_state(self.n_counts, device)
-        self._buf = None
 
     def accumulate(self, x):
         """Add one batch of independent walkers x (CUDA float64 [B, n_up + n_dn, 2]); no host synchronisation."""
-        if self._buf is None or self._buf.device != x.device:
-            self._buf = torch.empty(self.n_counts, dtype=torch.int64, device=x.device)
-        self._buf.zero_()
-        observables(x, self.n_up, self.n_dn, self.extent, self.n_xy, self.r_max, self.n_r, self.n_rot, self._buf)
-        self._add_batch(self._buf, x.shape[0])
+        counts = self._zeroed_sums(self.n_counts, x.device, torch.int64)
+        observables(x, self.n_up, self.n_dn, self.extent, self.n_xy, self.r_max, self.n_r, self.n_rot, counts)
+        self._add_batch(counts, x.shape[0])
 
     def _add_batch(self, counts, walkers):
         """Merge the counts of one batch of `walkers` walkers into the running sums (plain torch)."""
@@ -161,11 +193,9 @@ class DensityEstimator(_BatchMeans):
         per_bin = dict(density=torch.full((), dxy * dxy, **f64), radial=annulus, separation=annulus,
                        rotated=torch.full((), drot * drot * n, **f64))
         out = {}
-        for name, nch, _ in _SECTIONS:
-            off, shape = self.layout[name]
-            m, e = (t[off:off + math.prod(shape)].reshape(shape) for t in (mean, err))
+        for name, _, _ in _SECTIONS:
             norm = per_bin[name]
-            out[name], out[name + "_err"] = m / norm, e / norm
+            out[name], out[name + "_err"] = self._section(mean, name) / norm, self._section(err, name) / norm
         items = torch.tensor([nu, nd, nu, nd, nu * (nu - 1) / 2, nd * (nd - 1) / 2, nu * nd,
                               nu * (nu - 1) + nd * (nd - 1), 2 * nu * nd], **f64)
         out["outside_fraction"] = mean[self.n_bins:] / items
@@ -178,31 +208,15 @@ class DensityEstimator(_BatchMeans):
         return {k: v.cpu().numpy() for k, v in out.items()}
 
 
-def sample_density(model, n_up, n_dn, batch, batches, extent, path):
-    """The --density option of the drivers: `batches` batches of `batch` walkers from model.sample at the current
-    parameters, merged over ranks and saved to `path` by rank 0."""
-    est = DensityEstimator(n_up, n_dn, extent, device=next(model.parameters()).device)
-    with torch.no_grad():
-        for _ in range(batches):
-            _, x = model.sample((batch,))
-            est.accumulate(x)
-    est.allreduce()
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0:
-        est.save(path)
-        res = est.result()
-        print("density: %d walkers saved to %s; outside the density grid: up %.3g, down %.3g (fraction of particles)"
-              % (res["walkers"], path, res["outside_fraction"][0], res["outside_fraction"][1]))
-    return est
+    def _summary(self, res, path):
+        return ("density: %d walkers saved to %s; outside the density grid: up %.3g, down %.3g (fraction of particles)"
+                % (res["walkers"], path, res["outside_fraction"][0], res["outside_fraction"][1]))
 
 
 def sums_layout(n_k, n_kr, n_s):
     """{section: (offset, shape)} of the sums of ff_momentum_accumulate (include/fermiflow_b200.h) and their length."""
-    out, off = {}, 0
-    for name, shape in (("momentum", (2, n_k, n_k)), ("radial", (2, n_kr)), ("ratio", (2, n_s)), ("records", (2, n_s)),
-                        ("channel", (2,))):
-        out[name] = (off, shape)
-        off += math.prod(shape)
-    return out, off
+    return _layout((("momentum", (2, n_k, n_k)), ("radial", (2, n_kr)), ("ratio", (2, n_s)), ("records", (2, n_s)),
+                    ("channel", (2,))))
 
 
 def momentum_accumulate(ratio, particle, disp, n_up, k_max, n_k, n_kr, s_max, n_s, sums):
@@ -241,53 +255,40 @@ class MomentumEstimator(_BatchMeans):
 
     def __init__(self, n_up, n_dn, k_max=4.0, n_k=64, n_kr=128, s_max=8.0, n_s=64, moves=8,
                  device=torch.device("cuda")):
-        if n_up < 0 or n_dn < 0 or n_up + n_dn < 1:
-            raise ValueError("bad particle numbers %d/%d" % (n_up, n_dn))
-        if moves < 1:
-            raise ValueError("moves must be at least 1, got %d" % moves)
+        super().__init__(n_up, n_dn)
+        self.moves = self._check_moves(moves)
         if not (k_max > 0 and math.isfinite(k_max) and s_max > 0 and math.isfinite(s_max)):
             raise ValueError("k_max and s_max must be positive and finite, got %r and %r" % (k_max, s_max))
         if min(n_k, n_kr, n_s) < 0:
             raise ValueError("negative bin count (n_k %d, n_kr %d, n_s %d)" % (n_k, n_kr, n_s))
-        self.n_up, self.n_dn = int(n_up), int(n_dn)
         self.k_max, self.s_max = float(k_max), float(s_max)
         self.n_k, self.n_kr, self.n_s = int(n_k), int(n_kr), int(n_s)
-        self.moves = int(moves)
         self.layout, self.n_sums = sums_layout(self.n_k, self.n_kr, self.n_s)
         # the sums, then ratio sum + record count per |s| bin: its squares give the cross moment the error of the
         # coherence (a ratio of two means) needs
         self._init_state(self.n_sums + 2 * self.n_s, device)
-        self._buf = None
 
     def accumulate(self, model, x, generator=None):
         """Add one batch of independent walkers x (CUDA float64 [B, n_up + n_dn, 2], drawn by model.sample at the
         current parameters): `moves` records per walker, drawn on the device (torch.randint / torch.rand with
         `generator`); no host synchronisation."""
-        n = self.n_up + self.n_dn
-        if x.dim() != 3 or x.shape[-1] != 2 or x.shape[1] != n:
-            raise ValueError("x must be [B, %d, 2], got %s" % (n, tuple(x.shape)))
-        if not x.is_cuda:
-            raise RuntimeError("MomentumEstimator needs CUDA walkers (got %s); no CPU fallback" % x.device)
+        self._check_walkers(x)
         B, M, dev = x.shape[0], self.moves, x.device
-        particle = torch.randint(0, n, (B, M), device=dev, dtype=torch.int32, generator=generator)
+        particle = torch.randint(0, self.n_up + self.n_dn, (B, M), device=dev, dtype=torch.int32, generator=generator)
         u = torch.rand(B, M, 2, device=dev, dtype=torch.float64, generator=generator)
         r = self.s_max * u[..., 0].sqrt()
         phi = (2 * math.pi) * u[..., 1]
         disp = torch.stack((r * phi.cos(), r * phi.sin()), -1)
         ratio = model.wavefunction_ratio(x, particle, disp)
-        if self._buf is None or self._buf.device != dev:
-            self._buf = torch.empty(self.n_sums, dtype=torch.float64, device=dev)
-        self._buf.zero_()
+        sums = self._zeroed_sums(self.n_sums, dev)
         momentum_accumulate(ratio, particle, disp, self.n_up, self.k_max, self.n_k, self.n_kr, self.s_max, self.n_s,
-                            self._buf)
-        self._add_batch(self._buf, B)
+                            sums)
+        self._add_batch(sums, B)
 
     def _add_batch(self, sums, walkers):
         """Merge the sums of one batch of `walkers` walkers into the running state (plain torch)."""
-        o1, sh = self.layout["ratio"]
-        o2, _ = self.layout["records"]
-        k = math.prod(sh)
-        self._merge(torch.cat((sums, sums[o1:o1 + k] + sums[o2:o2 + k])), walkers)
+        both = self._section(sums, "ratio") + self._section(sums, "records")
+        self._merge(torch.cat((sums, both.reshape(-1))), walkers)
 
     def result(self):
         """dict of float64 numpy arrays (see the class docstring)."""
@@ -296,24 +297,18 @@ class MomentumEstimator(_BatchMeans):
         f64 = dict(dtype=torch.float64, device=self.state.device)
         norm = (nu + nd) * self.s_max ** 2 / (4 * math.pi * self.moves)
         out = {}
-
-        def sect(name, t=mean):
-            off, shape = self.layout[name]
-            return t[off:off + math.prod(shape)].reshape(shape)
-
-        out["momentum"], out["momentum_err"] = norm * sect("momentum"), norm * sect("momentum", err)
-        out["momentum_radial"], out["momentum_radial_err"] = norm * sect("radial"), norm * sect("radial", err)
+        sect = self._section
+        out["momentum"], out["momentum_err"] = norm * sect(mean, "momentum"), norm * sect(err, "momentum")
+        out["momentum_radial"], out["momentum_radial_err"] = norm * sect(mean, "radial"), norm * sect(err, "radial")
         # coherence g = S / N per bin (S, N: ratio sum and records per walker); delta method over the batch means:
         # var(g) = Σ W_k (s_k − g n_k)² / ((K − 1) W N²), with Σ S_k N_k / W_k from the squares of S_k + N_k
-        S, N = sect("ratio"), sect("records")
+        S, N = sect(mean, "ratio"), sect(mean, "records")
         g = S / N
-        ns = self.n_sums
-        q = lambda name: sect(name, s2)                                  # noqa: E731
-        cross = 0.5 * (s2[ns:].reshape(S.shape) - q("ratio") - q("records"))
-        dev2 = q("ratio") - 2 * g * cross + g * g * q("records")        # Σ W_k (s_k − g n_k)², Σ W_k (s_k − g n_k) = 0
-        var = dev2.clamp_min(0.0) / ((K - 1.0) * W * N * N)
+        qS, qN = sect(s2, "ratio"), sect(s2, "records")
+        cross = 0.5 * (s2[self.n_sums:].reshape(S.shape) - qS - qN)
+        dev2 = qS - 2 * g * cross + g * g * qN                          # Σ W_k (s_k − g n_k)², Σ W_k (s_k − g n_k) = 0
         out["coherence"] = g
-        out["coherence_err"] = torch.where(K >= 2, var.sqrt(), torch.full_like(var, float("nan")))
+        out["coherence_err"] = self._stderr(dev2.clamp_min(0.0) / ((K - 1.0) * W * N * N), K)
         out["k_edges"] = torch.linspace(-self.k_max, self.k_max, self.n_k + 1, **f64)
         out["k_radial"] = (torch.arange(self.n_kr, **f64) + 0.5) * (self.k_max / max(self.n_kr, 1))
         out["s_edges"] = torch.linspace(0.0, self.s_max, self.n_s + 1, **f64)
@@ -322,33 +317,16 @@ class MomentumEstimator(_BatchMeans):
         out["n_up"], out["n_dn"] = torch.tensor(float(nu), **f64), torch.tensor(float(nd), **f64)
         return {k: v.cpu().numpy() for k, v in out.items()}
 
-
-def sample_momentum(model, n_up, n_dn, batch, batches, k_max, path):
-    """The --momentum option of the drivers: `batches` batches of `batch` walkers from model.sample at the current
-    parameters, `moves` = 8 one-particle moves per walker, merged over ranks and saved to `path` by rank 0."""
-    est = MomentumEstimator(n_up, n_dn, k_max=k_max, device=next(model.parameters()).device)
-    with torch.no_grad():
-        for _ in range(batches):
-            _, x = model.sample((batch,))
-            est.accumulate(model, x)
-    est.allreduce()
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0:
-        est.save(path)
-        res = est.result()
-        dk = 2 * est.k_max / est.n_k
-        print("momentum: %d walkers saved to %s; integral of n(k) over the grid: up %.4g, down %.4g"
-              % (res["walkers"], path, res["momentum"][0].sum() * dk * dk, res["momentum"][1].sum() * dk * dk))
-    return est
+    def _summary(self, res, path):
+        dk = 2 * self.k_max / self.n_k
+        return ("momentum: %d walkers saved to %s; integral of n(k) over the grid: up %.4g, down %.4g"
+                % (res["walkers"], path, res["momentum"][0].sum() * dk * dk, res["momentum"][1].sum() * dk * dk))
 
 
 def swap_layout(Q, n_up, n_dn):
     """{section: (offset, shape)} of the sums of ff_swap_accumulate (include/fermiflow_b200.h) and their length."""
     sec = (Q, n_up + 1, n_dn + 1)
-    out, off = {}, 0
-    for name, shape in (("ratio", sec), ("replicas", sec), ("matched", sec), ("skipped", (Q,)), ("pairs", (1,))):
-        out[name] = (off, shape)
-        off += math.prod(shape)
-    return out, off
+    return _layout((("ratio", sec), ("replicas", sec), ("matched", sec), ("skipped", (Q,)), ("pairs", (1,))))
 
 
 def swap_accumulate(ratio, sector, n_up, n_dn, sums):
@@ -394,8 +372,7 @@ class RenyiEstimator(_BatchMeans):
     """
 
     def __init__(self, n_up, n_dn, a=(0.5, 1.0, 1.5, 2.0, 2.5, 3.0), kind="disk", device=torch.device("cuda")):
-        if n_up < 0 or n_dn < 0 or n_up + n_dn < 1:
-            raise ValueError("bad particle numbers %d/%d" % (n_up, n_dn))
+        super().__init__(n_up, n_dn)
         if kind not in ("disk", "halfplane"):
             raise ValueError("kind must be 'disk' or 'halfplane', got %r" % (kind,))
         a = tuple(float(v) for v in a)
@@ -403,42 +380,32 @@ class RenyiEstimator(_BatchMeans):
             raise ValueError("between 1 and 32 regions, got %d" % len(a))
         if not all(math.isfinite(v) for v in a) or (kind == "disk" and min(a) < 0):
             raise ValueError("region parameters must be finite (and radii non-negative), got %r" % (a,))
-        self.n_up, self.n_dn = int(n_up), int(n_dn)
         self.a, self.kind, self.Q = a, kind, len(a)
         self.layout, self.n_sums = swap_layout(self.Q, self.n_up, self.n_dn)
         self._n_cells = self.Q * (self.n_up + 1) * (self.n_dn + 1)
         # the sums, then the ratio sum per region (its error) and ratio sum + replicas per sector (the cross moment
         # the error of S2_sector needs)
         self._init_state(self.n_sums + self.Q + self._n_cells, device)
-        self._buf = None
 
     def accumulate(self, model, x, generator=None):
         """Add one batch of independent walkers x (CUDA float64 [B, n_up + n_dn, 2], B ≥ 2, drawn by model.sample at
         the current parameters): B // 2 pairs from torch.randperm with `generator`; no host synchronisation."""
-        n = self.n_up + self.n_dn
-        if x.dim() != 3 or x.shape[-1] != 2 or x.shape[1] != n:
-            raise ValueError("x must be [B, %d, 2], got %s" % (n, tuple(x.shape)))
-        if not x.is_cuda:
-            raise RuntimeError("RenyiEstimator needs CUDA walkers (got %s); no CPU fallback" % x.device)
+        self._check_walkers(x)
         B, dev = x.shape[0], x.device
         if B < 2:
             raise ValueError("at least two walkers are needed for one pair, got %d" % B)
         P = B // 2
         pairs = torch.randperm(B, device=dev, generator=generator)[:2 * P].view(P, 2)
         ratio, sector = model.swap_ratio(x, pairs, self.a, self.kind)
-        if self._buf is None or self._buf.device != dev:
-            self._buf = torch.empty(self.n_sums, dtype=torch.float64, device=dev)
-        self._buf.zero_()
-        swap_accumulate(ratio, sector, self.n_up, self.n_dn, self._buf)
-        self._add_batch(self._buf, P)
+        sums = self._zeroed_sums(self.n_sums, dev)
+        swap_accumulate(ratio, sector, self.n_up, self.n_dn, sums)
+        self._add_batch(sums, P)
 
     def _add_batch(self, sums, pairs):
         """Merge the sums of one batch of `pairs` pairs into the running state (plain torch)."""
-        o1, _ = self.layout["ratio"]
-        o2, _ = self.layout["replicas"]
-        k = self._n_cells
-        per_region = sums[o1:o1 + k].reshape(self.Q, -1).sum(1)
-        self._merge(torch.cat((sums, per_region, sums[o1:o1 + k] + sums[o2:o2 + k])), pairs)
+        T = self._section(sums, "ratio")
+        per_region = T.reshape(self.Q, -1).sum(1)
+        self._merge(torch.cat((sums, per_region, (T + self._section(sums, "replicas")).reshape(-1))), pairs)
 
     def result(self):
         """dict of float64 numpy arrays, and `kind` as a string array (see the class docstring)."""
@@ -446,27 +413,22 @@ class RenyiEstimator(_BatchMeans):
         f64 = dict(dtype=torch.float64, device=self.state.device)
         nan = torch.tensor(float("nan"), **f64)
         ns, Q = self.n_sums, self.Q
-        shape = self.layout["ratio"][1]
-
-        def sect(name, t=mean):
-            off, sh = self.layout[name]
-            return t[off:off + math.prod(sh)].reshape(sh)
-
+        sect = self._section
         out = {}
         swap, swap_err = mean[ns:ns + Q], err[ns:ns + Q]
         ok = swap > 0
         out["swap"], out["swap_err"] = swap, swap_err
         out["S2"] = torch.where(ok, -swap.clamp_min(1e-300).log(), nan)
         out["S2_err"] = torch.where(ok, swap_err / swap, nan)
-        T, R = sect("ratio"), sect("replicas")                          # per pair: ratio sum, replicas
-        out["sector_prob"], out["sector_prob_err"] = 0.5 * R, 0.5 * sect("replicas", err)
-        out["sector_swap"], out["sector_swap_err"] = T, sect("ratio", err)
+        T, R = sect(mean, "ratio"), sect(mean, "replicas")              # per pair: ratio sum, replicas
+        out["sector_prob"], out["sector_prob_err"] = 0.5 * R, 0.5 * sect(err, "replicas")
+        out["sector_swap"], out["sector_swap_err"] = T, sect(err, "ratio")
         # S2(a, b) = −ln T + 2 ln R + const; delta method over the batch means with the cross moment
         # Σ T_k R_k / W_k taken from the squares of T_k + R_k
         good = (T > 0) & (R > 0)
         Tg, Rg = torch.where(good, T, 1.0), torch.where(good, R, 1.0)
-        qT, qR = sect("ratio", s2) - W * T * T, sect("replicas", s2) - W * R * R
-        cross = 0.5 * (s2[ns + Q:].reshape(shape) - sect("ratio", s2) - sect("replicas", s2)) - W * T * R
+        qT, qR = sect(s2, "ratio") - W * T * T, sect(s2, "replicas") - W * R * R
+        cross = 0.5 * (s2[ns + Q:].reshape(T.shape) - sect(s2, "ratio") - sect(s2, "replicas")) - W * T * R
         dev2 = qT / (Tg * Tg) + 4 * qR / (Rg * Rg) - 4 * cross / (Tg * Rg)
         var = dev2.clamp_min(0.0) / ((K - 1.0) * W)
         out["S2_sector"] = torch.where(good, -(Tg / (0.25 * Rg * Rg)).log(), nan)
@@ -478,32 +440,15 @@ class RenyiEstimator(_BatchMeans):
         res["kind"] = np.array(self.kind)
         return res
 
-
-def sample_renyi(model, n_up, n_dn, batch, batches, a, kind, path):
-    """The --renyi option of the drivers: `batches` batches of `batch` walkers from model.sample at the current
-    parameters, randomly paired, merged over ranks and saved to `path` by rank 0."""
-    est = RenyiEstimator(n_up, n_dn, a=a, kind=kind, device=next(model.parameters()).device)
-    with torch.no_grad():
-        for _ in range(batches):
-            _, x = model.sample((batch,))
-            est.accumulate(model, x)
-    est.allreduce()
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0:
-        est.save(path)
-        res = est.result()
-        print("renyi: %d pairs saved to %s; S2 per %s: %s" % (res["pairs"], path, kind, ", ".join(
-            "%g: %.4g +- %.2g" % (v, s, e) for v, s, e in zip(est.a, res["S2"], res["S2_err"]))))
-    return est
+    def _summary(self, res, path):
+        return "renyi: %d pairs saved to %s; S2 per %s: %s" % (res["pairs"], path, self.kind, ", ".join(
+            "%g: %.4g +- %.2g" % (v, s, e) for v, s, e in zip(self.a, res["S2"], res["S2_err"])))
 
 
 def density_matrix_layout(K):
     """{section: (offset, shape)} of the sums of ff_density_matrix_accumulate (include/fermiflow_b200.h) for K orbitals
     and their length 2 K² + 3."""
-    out, off = {}, 0
-    for name, shape in (("matrix", (2, K, K)), ("records", (2,)), ("skipped", (1,))):
-        out[name] = (off, shape)
-        off += math.prod(shape)
-    return out, off
+    return _layout((("matrix", (2, K, K)), ("records", (2,)), ("skipped", (1,))))
 
 
 def density_matrix_accumulate(x, particle, disp, w, n_up, n_dn, n_orb, sums):
@@ -565,17 +510,14 @@ class DensityMatrixEstimator(_BatchMeans):
     """
 
     def __init__(self, n_up, n_dn, shells=7, sigma=1.5, moves=8, device=torch.device("cuda")):
-        if n_up < 0 or n_dn < 0 or n_up + n_dn < 1:
-            raise ValueError("bad particle numbers %d/%d" % (n_up, n_dn))
+        super().__init__(n_up, n_dn)
         if not 0 <= shells <= 7:
             raise ValueError("shells must be in [0, 7] (HO2D has 36 orbitals), got %d" % shells)
         if not (math.isfinite(sigma) and sigma > 0.5):
             raise ValueError("sigma must be finite and above 1/2 (the weights' variance is infinite below), got %r"
                              % (sigma,))
-        if moves < 1:
-            raise ValueError("moves must be at least 1, got %d" % moves)
-        self.n_up, self.n_dn = int(n_up), int(n_dn)
-        self.shells, self.sigma, self.moves = int(shells), float(sigma), int(moves)
+        self.moves = self._check_moves(moves)
+        self.shells, self.sigma = int(shells), float(sigma)
         self.K = K = (self.shells + 1) * (self.shells + 2) // 2
         self.layout, self.n_sums = density_matrix_layout(K)
         self._tri = torch.triu_indices(K, K)                            # the independent entries a <= b
@@ -583,30 +525,23 @@ class DensityMatrixEstimator(_BatchMeans):
         self._tri_dev = self._tri.to(device)
         # the sums, then Σ_batches m m^T / W of the independent entries m of each channel (the covariance of D)
         self._init_state(self.n_sums, device, n_extra=2 * self._P * self._P)
-        self._buf = None
 
     def accumulate(self, model, x, generator=None):
         """Add one batch of independent walkers x (CUDA float64 [B, n_up + n_dn, 2], drawn by model.sample at the
         current parameters): `moves` records per walker, drawn on the device (torch.randint / torch.randn with
         `generator`); no host synchronisation."""
-        n = self.n_up + self.n_dn
-        if x.dim() != 3 or x.shape[-1] != 2 or x.shape[1] != n:
-            raise ValueError("x must be [B, %d, 2], got %s" % (n, tuple(x.shape)))
-        if not x.is_cuda:
-            raise RuntimeError("DensityMatrixEstimator needs CUDA walkers (got %s); no CPU fallback" % x.device)
+        self._check_walkers(x)
         x = x.detach().contiguous()
         B, M, dev = x.shape[0], self.moves, x.device
-        particle = torch.randint(0, n, (B, M), device=dev, dtype=torch.int32, generator=generator)
+        particle = torch.randint(0, self.n_up + self.n_dn, (B, M), device=dev, dtype=torch.int32, generator=generator)
         rp = self.sigma * torch.randn(B, M, 2, device=dev, dtype=torch.float64, generator=generator)
         disp = rp - torch.gather(x, 1, particle.long()[..., None].expand(B, M, 2))
         ratio = model.wavefunction_ratio(x, particle, disp)
         s2 = self.sigma ** 2
         w = ratio * ((2 * math.pi * s2) * torch.exp((rp * rp).sum(-1) / (2 * s2)))           # ρ / q(r′)
-        if self._buf is None or self._buf.device != dev:
-            self._buf = torch.empty(self.n_sums, dtype=torch.float64, device=dev)
-        self._buf.zero_()
-        density_matrix_accumulate(x, particle, disp, w, self.n_up, self.n_dn, self.K, self._buf)
-        self._add_batch(self._buf, B)
+        sums = self._zeroed_sums(self.n_sums, dev)
+        density_matrix_accumulate(x, particle, disp, w, self.n_up, self.n_dn, self.K, sums)
+        self._add_batch(sums, B)
 
     def _add_batch(self, sums, walkers):
         """Merge the sums of one batch of `walkers` walkers into the running state (plain torch)."""
@@ -638,10 +573,9 @@ class DensityMatrixEstimator(_BatchMeans):
         big = V.abs().argmax(-2, keepdim=True)
         V = V * torch.where(torch.gather(V, -2, big) < 0, -1.0, 1.0)
         G = V[:, ta, :] * V[:, tb, :] * (2.0 - diag)[None, :, None]                         # dλ_k / dD_ab, [2, P, K]
-        nan = torch.tensor(float("nan"), dtype=torch.float64)
 
         def sd(var):
-            return torch.where(Kc >= 2, var.clamp_min(0.0).sqrt(), nan)
+            return self._stderr(var.clamp_min(0.0), Kc)
 
         quanta = torch.tensor([(orb.nx, orb.ny) for orb in HO2D().orbitals[:K]], dtype=torch.float64)
         shell = torch.nn.functional.one_hot(quanta.sum(1).long(), self.shells + 1).to(torch.float64)   # [K, shells+1]
@@ -655,25 +589,67 @@ class DensityMatrixEstimator(_BatchMeans):
         out["n_up"], out["n_dn"] = torch.tensor(float(self.n_up), **f64), torch.tensor(float(self.n_dn), **f64)
         return {k: v.numpy() for k, v in out.items()}
 
-
-def sample_natural_orbitals(model, n_up, n_dn, batch, batches, shells, path):
-    """The --natural-orbitals option of the drivers: `batches` batches of `batch` walkers from model.sample at the
-    current parameters, `moves` = 8 one-particle moves per walker, merged over ranks and saved to `path` by rank 0."""
-    est = DensityMatrixEstimator(n_up, n_dn, shells=shells, device=next(model.parameters()).device)
-    with torch.no_grad():
-        for _ in range(batches):
-            _, x = model.sample((batch,))
-            est.accumulate(model, x)
-    est.allreduce()
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0:
-        est.save(path)
-        res = est.result()
+    def _summary(self, res, path):
         lines = []
-        for c, (name, nc) in enumerate((("up", n_up), ("down", n_dn))):
+        for c, (name, nc) in enumerate((("up", self.n_up), ("down", self.n_dn))):
             lead = ", ".join("%.4f +- %.2g" % (v, e) for v, e in
-                             list(zip(res["occupations"][c], res["occupations_err"][c]))[:min(nc + 2, est.K)])
+                             list(zip(res["occupations"][c], res["occupations_err"][c]))[:min(nc + 2, self.K)])
             lines.append("%s: trace %.4f +- %.2g of %d, leading occupations %s"
                          % (name, res["trace"][c], res["trace_err"][c], nc, lead))
-        print("natural orbitals: %d walkers, %d orbitals saved to %s; %s" % (res["walkers"], est.K, path,
-                                                                            "; ".join(lines)))
-    return est
+        return "natural orbitals: %d walkers, %d orbitals saved to %s; %s" % (res["walkers"], self.K, path,
+                                                                             "; ".join(lines))
+
+
+def add_driver_options(p):
+    """The estimator options of the drivers (FermionHO2D, BetaFermionHO2D) on the argparse parser p."""
+    p.add_argument("--density", metavar="FILE", help="after training, save the density and pair correlations of "
+                   "freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.DensityEstimator)")
+    p.add_argument("--density-batches", type=int, default=16, help="batches of --batch walkers for --density")
+    p.add_argument("--density-extent", type=float, default=6.0, help="half-width of the density grids")
+    p.add_argument("--momentum", metavar="FILE", help="after training, save the momentum distribution and one-body "
+                   "coherence of freshly sampled walkers to FILE (.npz, fermiflow_b200.observables.MomentumEstimator)")
+    p.add_argument("--momentum-batches", type=int, default=16, help="batches of --batch walkers for --momentum")
+    p.add_argument("--momentum-kmax", type=float, default=4.0, help="half-width of the momentum grid")
+    p.add_argument("--renyi", metavar="FILE", help="after training, save the second Renyi entropy of spatial regions, "
+                   "from replica swaps of freshly sampled walkers, to FILE (.npz, fermiflow_b200.observables.RenyiEstimator)")
+    p.add_argument("--renyi-batches", type=int, default=16, help="batches of --batch walkers for --renyi")
+    p.add_argument("--renyi-a", type=lambda s: [float(v) for v in s.split(",")], default=[0.5, 1.0, 1.5, 2.0, 2.5, 3.0],
+                   help="comma-separated region parameters for --renyi: disk radii or half-plane edges x < a")
+    p.add_argument("--renyi-kind", choices=("disk", "halfplane"), default="disk", help="region kind for --renyi")
+    p.add_argument("--natural-orbitals", metavar="FILE", help="after training, save the one-body density matrix in the "
+                   "HO2D basis and its natural-orbital occupations, from one-particle moves of freshly sampled walkers, to "
+                   "FILE (.npz, fermiflow_b200.observables.DensityMatrixEstimator)")
+    p.add_argument("--natural-orbitals-batches", type=int, default=16,
+                   help="batches of --batch walkers for --natural-orbitals")
+    p.add_argument("--natural-orbitals-shells", type=int, default=7,
+                   help="oscillator shells 0 ... S of the basis for --natural-orbitals ((S + 1)(S + 2) / 2 orbitals)")
+
+
+# per option of add_driver_options: its destination, the estimator made from the parsed arguments, and whether the
+# estimator's accumulate() takes the model
+_DRIVER_ESTIMATORS = (
+    ("density", lambda a, dev: DensityEstimator(a.nup, a.ndown, a.density_extent, device=dev), False),
+    ("momentum", lambda a, dev: MomentumEstimator(a.nup, a.ndown, k_max=a.momentum_kmax, device=dev), True),
+    ("renyi", lambda a, dev: RenyiEstimator(a.nup, a.ndown, a=a.renyi_a, kind=a.renyi_kind, device=dev), True),
+    ("natural_orbitals",
+     lambda a, dev: DensityMatrixEstimator(a.nup, a.ndown, shells=a.natural_orbitals_shells, device=dev), True),
+)
+
+
+def run_driver_options(model, args):
+    """After training, for each estimator option of add_driver_options that names a file: its --X-batches batches of
+    --batch walkers from model.sample at the current parameters, merged over ranks; rank 0 saves the estimate to the
+    file and prints one summary line."""
+    for name, make, takes_model in _DRIVER_ESTIMATORS:
+        path = getattr(args, name)
+        if not path:
+            continue
+        est = make(args, next(model.parameters()).device)
+        with torch.no_grad():
+            for _ in range(getattr(args, name + "_batches")):
+                _, x = model.sample((args.batch,))
+                est.accumulate(*((model, x) if takes_model else (x,)))
+        est.allreduce()
+        if not (dist.is_available() and dist.is_initialized()) or dist.get_rank() == 0:
+            est.save(path)
+            print(est._summary(est.result(), path))
