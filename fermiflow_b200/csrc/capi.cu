@@ -30,9 +30,7 @@ int cuda_fail(cudaError_t e, const char* what) {
 
 // in the order of enum Opt
 const char* const kOptNames[] = {
-    "no_table", "no_w_balance", "no_rt_cache", "flow_warp_fill", "flow_cta", "flow_big", "eloc_generic", "slater_cta",
-    "metropolis_kernel", "adjoint_cta", "pgrad_direct", "pgrad_tile", "pgrad_fixed_range", "adjoint_no_prefetch", "finale_cta",
-    "metropolis_no_split"};
+    "no_table", "flow_cta", "eloc_generic", "slater_cta", "metropolis_kernel", "adjoint_cta", "pgrad_direct"};
 static_assert(sizeof(kOptNames) / sizeof(kOptNames[0]) == OPT_COUNT, "one name per option");
 std::atomic<int> g_opt[OPT_COUNT];
 std::atomic<long long> g_launches{0};

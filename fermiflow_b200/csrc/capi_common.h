@@ -21,25 +21,17 @@ int cuda_fail(cudaError_t e, const char* what);
 // capacity errors reported to the caller (-1, -2)
 constexpr int FF_FALLBACK = -1000;
 
-// Kernel-variant switches (tests, A/B timing): set explicitly through ff_set_option, process-wide atomics.  The
+// Kernel-path switches: each forces a path the library also picks by itself for some inputs, so that tests can compare
+// it with the default path at sizes where both run.  Set explicitly through ff_set_option, process-wide atomics.  The
 // library never reads the environment.  0 = default behaviour for every option.
 enum Opt {
     OPT_NO_TABLE,            // evaluate every hidden unit instead of the certified Taylor tables
-    OPT_NO_W_BALANCE,        // several walkers per CTA: do not rebalance the walkers over the rounds
-    OPT_NO_RT_CACHE,         // no shared-memory mirror of the head of the eta table
-    OPT_FLOW_WARP_FILL,      // per cent of lanes the pair items must fill for the warp-per-walker sweeps (0 -> 60)
     OPT_FLOW_CTA,            // CTA-synchronous flow sweeps instead of warp-per-walker
-    OPT_FLOW_BIG,            // 128-register build of the CTA-synchronous sweeps
     OPT_ELOC_GENERIC,        // generic flow_kernel<MODE_ELOC> instead of the statically specialised eloc kernels
     OPT_SLATER_CTA,          // CTA-cooperative Slater kernel instead of warp-per-walker
     OPT_METROPOLIS_KERNEL,   // 0 auto, 1 registers (thread per walker), 2 warp per walker, 3 thread per walker (shared memory)
     OPT_ADJOINT_CTA,         // CTA-synchronous adjoint sweep
     OPT_PGRAD_DIRECT,        // direct parameter-gradient kernel (every hidden unit) instead of binned Taylor moments
-    OPT_PGRAD_TILE,          // walker-stages per tile of the binned kernel (0 -> 32)
-    OPT_PGRAD_FIXED_RANGE,   // eta nodes over the fixed range instead of the sampled 99.9 % quantile
-    OPT_ADJOINT_NO_PREFETCH, // adjoint sweep without the bulk prefetch of the next stage's stash into L2
-    OPT_FINALE_CTA,          // CTA-synchronous finale of the register-resident E_loc sweeps instead of one warp per walker
-    OPT_METROPOLIS_NO_SPLIT, // register sampler: always one thread per walker (never one thread per spin block)
     OPT_COUNT
 };
 extern std::atomic<int> g_opt[OPT_COUNT];

@@ -7,33 +7,19 @@ using namespace ffc;
 
 namespace {
 
-// Geometry of the finale kernel's walker block: [state: y, L, gDelta, (Delta, lapDelta), J D8 x DP][Slater scratch,
-// g0, reduction buffer][M = J J^T][x0]
-int plan_finale(ff::FlowArgs& a, int W) {
-    const int n = a.n, D = 2 * n, D8 = (D + 7) & ~7, DP = D8 + 4, NP = n * (n - 1) / 2;
-    a.D = D; a.DP = DP; a.NP = NP; a.W = W;
-    a.NSV = even(3 * D + 2 + D8 * DP);
-    a.off_sl = a.NSV;
-    const int scratch = ff::slater_scratch_size(a.n_up, n - a.n_up) + D + n * n + NP + 8 + D;
-    a.off_AM = even(a.off_sl + scratch);
-    a.off_x0 = a.off_AM + D8 * DP;
-    a.wstride = even(a.off_x0 + D);
-    return 2 * ((NP + 7) / 8) + 2 + W * a.wstride;          // doubles of dynamic shared memory
-}
-
 // Finale from the final states in global memory (fin: `stride` doubles per walker): one warp per walker
-// (ff_finale.cuh); option "finale_cta" or an unusual particle number: the CTA-synchronous eloc_finale_kernel.
+// (ff_finale.cuh).  eloc5_kernel runs for N = 6 ... 20, i.e. NB8 = ceil(2 N / 8) = 2 ... 5.
 template <int NB8>
 int launch_finale_warp(const ff::FlowArgs& a, const double* fin, int stride, cudaStream_t st) {
     const DevInfo di = dev_info();
     const int warps = 4;
     const size_t smem = (size_t)warps * ff::finale_warp_slice(a.n, std::max(a.n_up, a.n - a.n_up)) * 8;
     auto kernel = ff::eloc_finale_warp_kernel<NB8>;
-    if ((long long)smem > di.smem_optin) return FF_FALLBACK;
+    if ((long long)smem > di.smem_optin) return fail(-2, "E_loc finale: n = %d needs %zu bytes of shared memory", a.n, smem);
     FF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
     FF_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, 32 * warps, smem));
-    if (occ < 1) return FF_FALLBACK;
+    if (occ < 1) return fail(-2, "E_loc finale kernel does not fit (n = %d)", a.n);
     const long long grid = std::min<long long>((a.B + warps - 1) / warps, (long long)di.sms * occ);
     kernel<<<(unsigned)grid, 32 * warps, smem, st>>>(a, fin, stride);
     FF_LAUNCHED();
@@ -41,32 +27,13 @@ int launch_finale_warp(const ff::FlowArgs& a, const double* fin, int stride, cud
 }
 
 int launch_finale(const ff::FlowArgs& a, const double* fin, int stride, cudaStream_t st) {
-    const DevInfo di = dev_info();
-    if (!opt(OPT_FINALE_CTA)) {
-        int r = FF_FALLBACK;
-        switch ((2 * a.n + 7) / 8) {
-            case 2: r = launch_finale_warp<2>(a, fin, stride, st); break;
-            case 3: r = launch_finale_warp<3>(a, fin, stride, st); break;
-            case 4: r = launch_finale_warp<4>(a, fin, stride, st); break;
-            case 5: r = launch_finale_warp<5>(a, fin, stride, st); break;
-            default: break;
-        }
-        if (r != FF_FALLBACK) return r;
+    switch ((2 * a.n + 7) / 8) {
+        case 2: return launch_finale_warp<2>(a, fin, stride, st);
+        case 3: return launch_finale_warp<3>(a, fin, stride, st);
+        case 4: return launch_finale_warp<4>(a, fin, stride, st);
+        case 5: return launch_finale_warp<5>(a, fin, stride, st);
+        default: return fail(-2, "E_loc finale: no kernel for n = %d", a.n);
     }
-    ff::FlowArgs f = a;
-    int W = 2;
-    size_t fsmem = (size_t)plan_finale(f, W) * 8;
-    if ((long long)fsmem > di.smem_optin) { W = 1; fsmem = (size_t)plan_finale(f, W) * 8; }
-    if ((long long)fsmem > di.smem_optin) return fail(-2, "E_loc finale: n = %d does not fit in shared memory", a.n);
-    FF_CUDA(cudaFuncSetAttribute(ff::eloc_finale_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem));
-    FF_CUDA(cudaFuncSetAttribute(ff::eloc_finale_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    int focc = 0;
-    FF_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&focc, ff::eloc_finale_kernel, 256, fsmem));
-    if (focc < 1) return fail(-2, "E_loc finale kernel does not fit");
-    const long long fgrid = std::min<long long>((a.B + W - 1) / W, (long long)di.sms * focc);
-    ff::eloc_finale_kernel<<<(unsigned)fgrid, 256, fsmem, st>>>(f, fin, stride);
-    FF_LAUNCHED();
-    return 0;
 }
 
 // Register-resident sweep (ff_eloc5.cuh eloc5_kernel) + finale kernel.
@@ -119,7 +86,7 @@ int launch_eloc5(ff::FlowArgs& a, cudaStream_t st) {
     const long long half = std::min<long long>(di.smem_sm / 2 - di.smem_reserved, di.smem_optin);
     const long long room = half - (long long)g.total * 8;
     // (at most 256 rows: small walker blocks leave the shared memory to more resident CTAs instead)
-    a.rt_cache_nodes = (a.rt_eta != nullptr && room > 0 && !opt(OPT_NO_RT_CACHE)) ? (int)std::min<long long>(room / (8 * ff::kRtPitch), 256) : 0;
+    a.rt_cache_nodes = (a.rt_eta != nullptr && room > 0) ? (int)std::min<long long>(room / (8 * ff::kRtPitch), 256) : 0;
     size_t smem = (size_t)(g.total + a.rt_cache_nodes * ff::kRtPitch) * 8;
 #ifdef FF_DEV_ONE_CTA
     smem = std::max<size_t>(smem, (size_t)di.smem_sm / 2 + 4096);          // (dev experiment: one resident CTA per SM)

@@ -87,7 +87,7 @@ int launch_flow_kernel(K kernel, ff::FlowArgs& a, int threads, size_t smem, cuda
     if (occ < 1) return fail(-2, "flow kernel does not fit on an SM (threads %d, smem %zu)", threads, smem);
     long long nb = (a.B + a.W - 1) / a.W;
     long long grid = (long long)di.sms * occ;
-    if (a.W > 1 && a.B > 0 && !opt(OPT_NO_W_BALANCE)) {
+    if (a.W > 1 && a.B > 0) {
         // several walkers per CTA (small n): spread them evenly over the rounds the resident CTAs need anyway --
         // 8000 walkers at W = 26 are 308 tasks for 296 CTAs (two rounds, the second almost empty); W = 14 gives 572
         // tasks, two full rounds of half the length.  threads / smem were sized for the larger W and stay valid.
@@ -114,8 +114,7 @@ int launch_flow_warp(ff::FlowArgs& a, cudaStream_t st) {
     if (smem > (size_t)di.smem_optin) return FF_FALLBACK;
     {   // spare shared memory at FF_WARP_MINB CTAs per SM mirrors the head of the eta Taylor table
         const long long room = (long long)di.smem_sm / FF_WARP_MINB - di.smem_reserved - (long long)smem - 64;
-        a.rt_cache_nodes = (a.rt_eta != nullptr && room > 0 && !opt(OPT_NO_RT_CACHE))
-                               ? (int)std::min<long long>(room / (8 * ff::kRtCoef), 2048) : 0;
+        a.rt_cache_nodes = (a.rt_eta != nullptr && room > 0) ? (int)std::min<long long>(room / (8 * ff::kRtCoef), 2048) : 0;
         smem += (size_t)a.rt_cache_nodes * 8 * ff::kRtCoef;
     }
     auto kernel = ff::flow_warp_kernel<MODE>;
@@ -138,15 +137,12 @@ int launch_flow(ff::FlowArgs& a, int threads, size_t smem, cudaStream_t st) {
         const int rounds = (a.NP + 31) / 32;
         // measured (scripts/dev_gen_time_n.py, 65536 walkers): N = 12 (66 pairs, 69 % of three rounds) 7.0 ms CTA-synchronous
         // against 5.7 ms warp-per-walker; N = 9 (36 pairs, 56 %) 4.3 against 4.9 ms; N = 6 (15 pairs, 47 %) 2.0 against 3.8 ms
-        const int min_fill = opt(OPT_FLOW_WARP_FILL) ? opt(OPT_FLOW_WARP_FILL) : 60;      // per cent of the lanes
+        constexpr int min_fill = 60;      // per cent of the lanes
         if (a.NP > 0 && a.n <= 255 && 100 * a.NP >= min_fill * 32 * rounds && !opt(OPT_FLOW_CTA)) {
             const int r = launch_flow_warp<MODE>(a, st);
             if (r != FF_FALLBACK) return r;
         }
-    }
-    if constexpr (MODE != ff::MODE_ELOC) {
-        if (threads <= 256 && !opt(OPT_FLOW_BIG))
-            return launch_flow_kernel(ff::flow_kernel_small<MODE>, a, threads, smem, st);
+        if (threads <= 256) return launch_flow_kernel(ff::flow_kernel_small<MODE>, a, threads, smem, st);
     }
     return launch_flow_kernel(ff::flow_kernel<MODE>, a, threads, smem, st);
 }

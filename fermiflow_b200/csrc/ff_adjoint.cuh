@@ -177,7 +177,7 @@ __global__ void __launch_bounds__(512) adjoint_kernel(const AdjArgs a) {
 // ---------------------------------------------------------------------------------------
 __host__ __device__ inline int adjoint_warp_slice(int D, int P) { return 6 * D + 2 * P; }
 
-template <bool RECOMPUTE, bool PREFETCH = true>
+template <bool RECOMPUTE>
 __global__ void __launch_bounds__(256, 4) adjoint_warp_kernel(const AdjArgs a) {
     extern __shared__ __align__(16) double smem[];
     const int tid = threadIdx.x, T = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarp = T >> 5;
@@ -211,7 +211,7 @@ __global__ void __launch_bounds__(256, 4) adjoint_warp_kernel(const AdjArgs a) {
             const int sub = stage & 3;
             // the stash of the stage after this one (5 KB, contiguous) is pulled into L2 by the bulk-copy engine while
             // this stage computes: no registers, no shared memory; the sweep is latency bound on exactly these loads
-            if (PREFETCH && lane == 0 && stage > 0) {
+            if (lane == 0 && stage > 0) {
                 // (16-byte granularity: the start is rounded down, the end too; both stay inside the stash)
                 auto bulk_prefetch = [](const double* p, int bytes) {
                     const unsigned long long a0 = reinterpret_cast<unsigned long long>(p), a1 = (a0 + bytes) & ~15ull, as = a0 & ~15ull;

@@ -63,33 +63,33 @@ struct FlowArgs {
 // State vector layout (MODE_ELOC): [y:D][L:D][gD:D][Delta, lapDelta][J: D x DP]
 // otherwise:                        [y:D][Delta]
 
-// Launch geometry shared by host planning (capi.cu) and the statically specialised kernels.
+// Walker-block geometry of the CTA-synchronous sweeps, planned on the host (capi_flow.h plan_flow) into FlowArgs.
 struct FlowGeom {
-    int n, D, D8, DP, NP, P, NV, NSV, NPAR, grec;
-    int off_G, off_AM, off_u, off_kLx, off_part, off_x0, off_sl, wstride, threads1;
+    int D, DP, NP, P, NV, NSV, NPAR, grec;
+    int off_G, off_AM, off_u, off_kLx, off_part, off_x0, off_sl, wstride;
 };
 __host__ __device__ constexpr int ff_even(int x) { return (x + 1) & ~1; }
-__host__ __device__ constexpr FlowGeom flow_geom(int mode, int n, bool has_mu, bool jglobal = false, int scratch_min = 0) {
+inline FlowGeom flow_geom(int mode, int n, bool has_mu, bool jglobal = false, int scratch_min = 0) {
     FlowGeom g{};
     const bool eloc = mode == MODE_ELOC;
-    g.n = n; g.D = 2 * n; g.D8 = (g.D + 7) & ~7;
+    g.D = 2 * n;
+    const int D8 = (g.D + 7) & ~7;
     g.NP = n * (n - 1) / 2; g.P = g.NP + (has_mu ? n : 0);
-    g.DP = eloc ? g.D8 + 4 : g.D;                 // DP mod 16 in {4, 12}: conflict-free DMMA fragments
+    g.DP = eloc ? D8 + 4 : g.D;                   // DP mod 16 in {4, 12}: conflict-free DMMA fragments
     g.NV = eloc ? 3 * g.D + 2 : g.D + (mode >= MODE_DIV ? 1 : 0);
-    g.NSV = eloc ? ff_even(g.NV + g.D8 * g.DP) : g.NV;
+    g.NSV = eloc ? ff_even(g.NV + D8 * g.DP) : g.NV;
     // (jglobal: the J parts of the RK partials are in FlowArgs::jpart; the area still holds the scratch of the finale)
     g.NPAR = eloc ? (jglobal ? ff_even(g.NV) : ff_even(g.NV + g.D * g.D)) : g.NV;
     g.grec = eloc ? kGRec : 3;
     int off = ff_even(g.NSV + (jglobal && 4 * g.NPAR < scratch_min ? scratch_min : 4 * g.NPAR));
     g.off_G = off; off = ff_even(off + g.P * g.grec);
-    g.off_AM = off; if (eloc) off = ff_even(off + g.D8 * g.DP);
+    g.off_AM = off; if (eloc) off = ff_even(off + D8 * g.DP);
     g.off_u = off; if (eloc) off += g.D;
     g.off_kLx = off; if (eloc) off += g.D;
     g.off_part = off; off = ff_even(off + 2 * n);
     g.off_x0 = off; if (eloc) off += g.D;
     g.off_sl = g.NSV;
     g.wstride = ff_even(off);
-    g.threads1 = ((g.P + 31) / 32) * 32 < 64 ? 64 : ((g.P + 31) / 32) * 32;
     return g;
 }
 
@@ -340,25 +340,18 @@ __device__ void eloc_finale(const FlowArgs& a, long long base, double* wbase,
     team.sync();
 }
 
-// SN > 0 fixes the particle number (and SMU the presence of the one-body MLP) at compile time:
-// every loop bound, offset and index division below then folds to a constant and the short
-// latency-bound phases unroll.  SN = 0 is the generic run-time version.
-template <int MODE, int SN, int SMU, int HELP = 1>
+// One sweep of W walkers per CTA with the run-time geometry of FlowArgs (plan_flow).
+template <int MODE>
 __device__ __forceinline__ void flow_body(const FlowArgs& a) {
     extern __shared__ __align__(16) double smem[];
-    constexpr bool kS = SN > 0;
-    constexpr FlowGeom GS = flow_geom(MODE, kS ? SN : 2, SMU != 0);
     // one extra "helper" warp (when the launch provides it) computes the Gram matrix while the
     // item warps are still in the MLP loop
-    const int tid = threadIdx.x, T = kS ? GS.threads1 + 32 * HELP : (int)blockDim.x;
-    const int n = kS ? GS.n : a.n, D = kS ? GS.D : a.D, DP = kS ? GS.DP : a.DP, P = kS ? GS.P : a.P;
-    const int NP = kS ? GS.NP : a.NP, W = kS ? 1 : a.W, NSV = kS ? GS.NSV : a.NSV;
-    const int off_G = kS ? GS.off_G : a.off_G, off_AM = kS ? GS.off_AM : a.off_AM, off_u = kS ? GS.off_u : a.off_u;
-    const int off_kLx = kS ? GS.off_kLx : a.off_kLx, off_part = kS ? GS.off_part : a.off_part;
-    const int off_x0 = kS ? GS.off_x0 : a.off_x0;
+    const int tid = threadIdx.x, T = blockDim.x;
+    const int n = a.n, D = a.D, DP = a.DP, P = a.P, NP = a.NP, W = a.W, NSV = a.NSV;
+    const int off_G = a.off_G, off_AM = a.off_AM, off_u = a.off_u, off_kLx = a.off_kLx, off_part = a.off_part, off_x0 = a.off_x0;
     const int D8 = (D + 7) & ~7;
     (void)DP; (void)D8; (void)off_AM; (void)off_u; (void)off_kLx; (void)off_x0;
-    const bool has_mu = kS ? (SMU != 0) : (a.H_mu > 0);
+    const bool has_mu = a.H_mu > 0;
     const int warp = tid >> 5, lane = tid & 31, nwarp = T >> 5;
 
     // ---- shared carve-up -------------------------------------------------------------
@@ -370,7 +363,7 @@ __device__ __forceinline__ void flow_body(const FlowArgs& a) {
     unsigned char* pair_j = pair_i + ((NP + 7) & ~7);
     double* wbase = smem + cbase + 2 * ((NP + 7) / 8);
     if ((wbase - smem) & 1) wbase += 1;
-    const int wstride = kS ? GS.wstride : a.wstride;
+    const int wstride = a.wstride;
 
     fill_exp_table(tab);
     const double* tabl = tab + (tid & 15);
@@ -388,10 +381,10 @@ __device__ __forceinline__ void flow_body(const FlowArgs& a) {
     constexpr int oY = 0;
     const int oL = D, oG = 2 * D, oS = 3 * D, oJ = 3 * D + 2;       // ELOC offsets
     const int oDelta = (MODE == MODE_ELOC) ? oS : D;
-    const int NV = kS ? GS.NV : a.NV, NPAR = kS ? GS.NPAR : a.NPAR;
+    const int NV = a.NV, NPAR = a.NPAR;
     const int oP3 = NSV, oP4 = NSV + NPAR, oPO = NSV + 2 * NPAR, oK = NSV + 3 * NPAR;
     // J part (D x D, unpadded) of RK block `which` (0: P3, 1: P4, 2: PO, 3: stage derivative) of walker w of this CTA
-    double* const jglob = (MODE == MODE_ELOC && !kS) ? a.jpart : nullptr;
+    double* const jglob = (MODE == MODE_ELOC) ? a.jpart : nullptr;
     auto jblock = [&](double* Sw, int w, int which) -> double* {
         return jglob ? jglob + (((size_t)blockIdx.x * W + w) * 4 + which) * (size_t)(D * D) : Sw + NSV + which * NPAR + NV;
     };
@@ -491,7 +484,7 @@ __device__ __forceinline__ void flow_body(const FlowArgs& a) {
             }
             if (MODE >= MODE_STASH && a.stash_y != nullptr) {
                 for (int q = tid; q < W * D; q += T) {              // flat over (walker, element): small n keeps every lane busy
-                    const int w = kS ? 0 : q / D, e = q - w * D;
+                    const int w = q / D, e = q - w * D;
                     const long long b = base + w;
                     if (b < a.B) a.stash_y[(b * NS + stage) * D + e] = (wbase + (size_t)w * wstride)[e];
                 }
@@ -530,7 +523,7 @@ __device__ __forceinline__ void flow_body(const FlowArgs& a) {
                 constexpr int GRg = (MODE == MODE_ELOC) ? kGRec : 3;      // record stride
                 constexpr int NC = (MODE == MODE_ELOC) ? kGRec : (MODE >= MODE_DIV ? 3 : 2);
                 for (int gg = tid; gg < W * n * NC; gg += T) {           // flat over (walker, particle, quantity)
-                    const int w = kS ? 0 : gg / (n * NC);
+                    const int w = gg / (n * NC);
                     const int g = gg - w * (n * NC);
                     double* Sw = wbase + (size_t)w * wstride;
                     const double* G = Sw + off_G;
@@ -539,39 +532,26 @@ __device__ __forceinline__ void flow_body(const FlowArgs& a) {
                         const int c = (MODE == MODE_ELOC) ? cc : (cc == 2 ? 6 : cc);   // logical quantity
                         const int gc = cc;                                             // column in the record
                         double accm = 0.0, accp = 0.0, accm2 = 0.0, accp2 = 0.0;
-                        if (kS) {
-                            // fixed trip count: every load of the particle's n-1 pair records is
-                            // independent of the others and issues back to back
-#pragma unroll
-                            for (int j = 0; j < (kS ? GS.n : 1); ++j) {
-                                const bool lower = j < i;
-                                const int idx = lower ? pair_index(j, i, n) : pair_index(i, j, n);
-                                const double v = (j == i) ? 0.0 : G[idx * GRg + gc];
-                                if (lower) { if (j & 1) accm2 += v; else accm += v; }
-                                else { if (j & 1) accp2 += v; else accp += v; }
+                        {   // pairs (j, i), j < i : stored with r = y_j - y_i
+                            int idx = i - 1;                       // pair_index(0, i)
+                            int j = 0;
+                            for (; j + 2 <= i; j += 2) {
+                                const int idx2 = idx + n - j - 2;
+                                const double v0 = G[idx * GRg + gc], v1 = G[idx2 * GRg + gc];
+                                accm += v0; accm2 += v1;
+                                idx = idx2 + n - j - 3;
                             }
-                        } else {
-                            {   // pairs (j, i), j < i : stored with r = y_j - y_i
-                                int idx = i - 1;                       // pair_index(0, i)
-                                int j = 0;
-                                for (; j + 2 <= i; j += 2) {
-                                    const int idx2 = idx + n - j - 2;
-                                    const double v0 = G[idx * GRg + gc], v1 = G[idx2 * GRg + gc];
-                                    accm += v0; accm2 += v1;
-                                    idx = idx2 + n - j - 3;
-                                }
-                                if (j < i) accm += G[idx * GRg + gc];
+                            if (j < i) accm += G[idx * GRg + gc];
+                        }
+                        {   // pairs (i, j), j > i : consecutive
+                            const double* Gi = G + pair_index(i, i + 1, n) * GRg + gc;
+                            int j = i + 1;
+                            for (; j + 4 <= n; j += 4) {
+                                const double v0 = Gi[0], v1 = Gi[GRg], v2 = Gi[2 * GRg], v3 = Gi[3 * GRg];
+                                accp += v0; accp2 += v1; accp += v2; accp2 += v3;
+                                Gi += 4 * GRg;
                             }
-                            {   // pairs (i, j), j > i : consecutive
-                                const double* Gi = G + pair_index(i, i + 1, n) * GRg + gc;
-                                int j = i + 1;
-                                for (; j + 4 <= n; j += 4) {
-                                    const double v0 = Gi[0], v1 = Gi[GRg], v2 = Gi[2 * GRg], v3 = Gi[3 * GRg];
-                                    accp += v0; accp2 += v1; accp += v2; accp2 += v3;
-                                    Gi += 4 * GRg;
-                                }
-                                for (; j < n; ++j) { accp += *Gi; Gi += GRg; }
-                            }
+                            for (; j < n; ++j) { accp += *Gi; Gi += GRg; }
                         }
                         accm += accm2; accp += accp2;
                         double acc = (c < 6) ? accp - accm : accp + accm;
@@ -706,7 +686,7 @@ __device__ __forceinline__ void flow_body(const FlowArgs& a) {
                 };
                 // flat over (walker, element): with many small walkers per CTA every lane stays busy
                 for (int q = tid; q < W * NV; q += T) {
-                    const int w = kS ? 0 : q / NV, e = q - w * NV;
+                    const int w = q / NV, e = q - w * NV;
                     double* Sw = wbase + (size_t)w * wstride;
                     upd(Sw + e, Sw + oP3 + e, Sw + oP4 + e, Sw + oPO + e, Sw + oK + e);
                 }
@@ -741,10 +721,10 @@ __device__ __forceinline__ void flow_body(const FlowArgs& a) {
                             *s2 = make_double2(fma(k.x, 0.125, ao.x), fma(k.y, 0.125, ao.y));
                         }
                     };
-                    if (kS || hD >= 16) {
+                    if (hD >= 16) {
                         // one (walker, row) per warp trip, two columns per lane (no integer division in the inner loop)
                         for (int wr = warp; wr < W * D; wr += nwarp) {
-                            const int w = kS ? 0 : wr / D, r = wr - w * D;
+                            const int w = wr / D, r = wr - w * D;
                             double* Sw = wbase + (size_t)w * wstride;
                             for (int c2 = lane; c2 < hD; c2 += 32) updJ(Sw, w, r, 2 * c2);
                         }
@@ -781,12 +761,12 @@ __device__ __forceinline__ void flow_body(const FlowArgs& a) {
 }
 
 template <int MODE>
-__global__ void __launch_bounds__(512, 1) flow_kernel(const FlowArgs a) { flow_body<MODE, 0, 0>(a); }
+__global__ void __launch_bounds__(512, 1) flow_kernel(const FlowArgs a) { flow_body<MODE>(a); }
 
 // Same body for CTAs of at most 256 threads, capped at 64 registers: four CTAs (32 warps) per SM
 // keep the FP64 pipe fed across the per-stage barriers of the value / divergence sweeps.
 template <int MODE>
-__global__ void __launch_bounds__(256, 4) flow_kernel_small(const FlowArgs a) { flow_body<MODE, 0, 0>(a); }
+__global__ void __launch_bounds__(256, 4) flow_kernel_small(const FlowArgs a) { flow_body<MODE>(a); }
 
 
 }  // namespace ff

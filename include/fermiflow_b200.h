@@ -33,11 +33,11 @@ typedef struct ff_model {
 int ff_version(void);
 const char* ff_last_error(void);
 
-/* Kernel-variant switches for tests and A/B timing (no reference counterpart; the library never reads the
- * environment).  Process-wide, thread-safe; 0 restores the default.  Names: no_table, no_w_balance, no_rt_cache,
- * flow_warp_fill, flow_cta, flow_big, eloc_generic, slater_cta, metropolis_kernel (0 auto, 1 registers, 2 warp per
- * walker, 3 thread per walker), adjoint_cta, pgrad_direct, pgrad_tile, pgrad_fixed_range, adjoint_no_prefetch,
- * finale_cta, metropolis_no_split (INTEGRATION.md has the table).  Unknown name: -1. */
+/* Kernel-path switches: each forces a path the library also picks by itself for some inputs, so that tests can
+ * compare it with the default one (no reference counterpart; the library never reads the environment).  Process-wide,
+ * thread-safe; 0 restores the default.  Names: no_table, flow_cta, eloc_generic, slater_cta, metropolis_kernel (0 auto,
+ * 1 registers, 2 warp per walker, 3 thread per walker), adjoint_cta, pgrad_direct (INTEGRATION.md has the table).
+ * Unknown name: -1. */
 /* Number of CUDA kernels this library has launched in the process so far (bench.py reports the difference over its
  * timed region as "gpu_launches"). */
 long long ff_launch_count(void);

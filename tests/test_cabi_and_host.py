@@ -58,6 +58,38 @@ def test_argument_errors_reported():
     assert lib.ff_potential(None, 5, 3, 1.0, 1, None, None) != 0
 
 
+def _option_names():
+    """The switch names listed in the ff_set_option comment of the header."""
+    hdr = open(os.path.join(ROOT, "include", "fermiflow_b200.h")).read()
+    names = re.search(r"Names:(.*?)\(INTEGRATION\.md", hdr, re.S).group(1)
+    names = re.sub(r"\([^)]*\)", "", names.replace("\n *", " "))
+    return [t.strip() for t in names.split(",")]
+
+
+def test_option_names_round_trip():
+    """Every switch the header names is accepted by ff_set_option and read back by ff_get_option; the switches that
+    only selected a variant for timing experiments are unknown names (-1)."""
+    from fermiflow_b200 import _lib as L
+    lib = L.lib()
+    names = _option_names()
+    assert "no_table" in names and all(re.fullmatch(r"[a-z_]+", n) for n in names), names
+    v = ctypes.c_int(-1)
+    try:
+        for n in names:
+            assert lib.ff_set_option(n.encode(), 3) == 0, n
+            assert lib.ff_get_option(n.encode(), ctypes.byref(v)) == 0 and v.value == 3, n
+    finally:
+        for n in names:
+            assert lib.ff_set_option(n.encode(), 0) == 0, n
+    for n in names:
+        assert lib.ff_get_option(n.encode(), ctypes.byref(v)) == 0 and v.value == 0, n
+    for n in ("no_w_balance", "no_rt_cache", "flow_warp_fill", "flow_big", "pgrad_tile", "pgrad_fixed_range",
+              "adjoint_no_prefetch", "finale_cta", "metropolis_no_split"):
+        assert lib.ff_set_option(n.encode(), 1) == -1, n
+        assert b"unknown option" in lib.ff_last_error(), n
+        assert lib.ff_get_option(n.encode(), ctypes.byref(v)) == -1, n
+
+
 def test_fermion_states_match_reference(golden):
     from fermiflow_b200 import HO2D
     ho, g = HO2D(), golden("states")

@@ -215,17 +215,15 @@ def test_eloc5_matches_generic(dev, nup, ndn, mu, large):
 
 
 @pytest.mark.parametrize("n,mu", ELOC5, ids=[_nid(*p) for p in ELOC5])
-def test_eloc5_variants_agree(dev, n, mu):
+def test_eloc5_generic_and_direct_paths_agree(dev, n, mu):
     """The kernel variants at every instantiation (balanced split, the large batch with the far walker): eloc5_kernel
-    with the Taylor tables (default) against the generic kernel with and without tables, eloc5_kernel evaluating every
-    hidden unit (no_table), without the shared-memory mirror of the eta table (no_rt_cache) and with the
-    CTA-synchronous finale (finale_cta)."""
+    with the Taylor tables (default) against the generic kernel with and without tables and eloc5_kernel evaluating
+    every hidden unit (no_table)."""
     from fermiflow_b200 import _lib as L
     model = _variant_model(dev, (n + 1) // 2, n // 2, mu)
     x, groups = _walkers(model, True)
     r0 = model.local_energy(x, stash=True)
-    for env in (dict(eloc_generic=1), dict(eloc_generic=1, no_table=1), dict(no_table=1), dict(no_rt_cache=1),
-                dict(finale_cta=1)):
+    for env in (dict(eloc_generic=1), dict(eloc_generic=1, no_table=1), dict(no_table=1)):
         with L.options(**env):
             r = model.local_energy(x, stash=True)
         _agree(r, r0, groups, str(env))
@@ -233,12 +231,10 @@ def test_eloc5_variants_agree(dev, n, mu):
 
 # ---------------------------------------------------------------------------------------
 @pytest.mark.parametrize("nup,ndn", [(5, 3), (8, 0)])
-def test_eloc5_excited_high_shell_occupations(dev, O, nup, ndn):
+def test_eloc5_warp_finale_excited_high_shell_occupations(dev, O, nup, ndn):
     """eloc5_kernel<8, 1> with a hand-made int32 occupation table and one row per walker (walker_state), passed to the
     sweep helper GSVMC.local_energy calls: orbitals up to index 35, i.e. nx or ny = 7, the top of the 8-entry Hermite
-    recursion of the finale.  Both finales (one warp per walker, CTA-synchronous) against the oracle with the same
-    occupation rows."""
-    from fermiflow_b200 import _lib as L
+    recursion of the finale (eloc_finale_warp_kernel).  Against the oracle with the same occupation rows."""
     from fermiflow_b200.utils import eloc_sweep
     n, S, B = nup + ndn, 3, 12
     rows = {(5, 3): [(0, 1, 2, 3, 4, 0, 1, 2),
@@ -258,11 +254,9 @@ def test_eloc5_excited_high_shell_occupations(dev, O, nup, ndn):
     x = model.cnf.generate(1.3 * torch.randn(B, n, 2, generator=gen).to(dev))
     occ = table[ws.long()].cpu().long()                                  # (B, n) HO2D orbital ids per walker
     ref = O.local_energy(x.cpu(), occ[:, :nup], occ[:, nup:], cpu_params(eta), cpu_params(mu), (0.0, 1.0), S, 2.0)
-    for env in (dict(), dict(finale_cta=1)):
-        with L.options(**env):
-            r = eloc_sweep(model.cnf, x, table, ws, nup, model._Z, model._harmonic)
-        for k in ("logp", "grad", "lap", "kinetic", "potential", "eloc"):
-            try:
-                close(getattr(r, k), ref[k])
-            except AssertionError as e:
-                raise AssertionError("%s, %s: %s" % (env, k, e)) from None
+    r = eloc_sweep(model.cnf, x, table, ws, nup, model._Z, model._harmonic)
+    for k in ("logp", "grad", "lap", "kinetic", "potential", "eloc"):
+        try:
+            close(getattr(r, k), ref[k])
+        except AssertionError as e:
+            raise AssertionError("%s: %s" % (k, e)) from None

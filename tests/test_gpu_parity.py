@@ -538,35 +538,35 @@ def _dot_model(dev, nsteps=8, H=50, nup=10, ndn=10):
     return GSVMC(nup, ndn, HO2D(), FreeFermion(dev), cnf, CoulombPairPotential(2.0), sp_potential=HO()).to(dev)
 
 
-def test_flow_kernel_variants_agree_full_size(dev):
-    """N = 20: one-warp-per-walker sweeps against the CTA-synchronous flow_kernel (option flow_cta)
-    and its 128-register build (flow_big) on the same walkers."""
-    model = _dot_model(dev)
-    z, _ = model.sample((777,))
-    outs = []
-    for env in (dict(flow_cta=0, flow_big=0), dict(flow_cta=1, flow_big=0), dict(flow_cta=1, flow_big=1)):
-        with _opts(**env):
-            x = model.cnf.generate(z)
-            zz, dl = model.cnf.delta_logp(x)
-            outs.append((x, zz, dl))
-    for o in outs[1:]:
-        close(o[0], outs[0][0], 1e-13)
-        close(o[1], outs[0][1], 1e-13)
-        close(o[2], outs[0][2], 1e-12, 1e-14)
+def test_flow_cta_sweeps_agree_with_warp_sweeps(dev):
+    """One-warp-per-walker sweeps against the CTA-synchronous ones (option flow_cta) on the same walkers: at N = 20
+    (P = 210 items: flow_kernel_small, 224 threads) and at N = 24 with the one-body MLP (P = 300: flow_kernel, 320
+    threads)."""
+    for nup in (10, 12):
+        model = _dot_model(dev, nup=nup, ndn=nup)
+        z, _ = model.sample((777,))
+        outs = []
+        for env in (dict(flow_cta=0), dict(flow_cta=1)):
+            with _opts(**env):
+                x = model.cnf.generate(z)
+                zz, dl = model.cnf.delta_logp(x)
+                outs.append((x, zz, dl))
+        close(outs[1][0], outs[0][0], 1e-13)
+        close(outs[1][1], outs[0][1], 1e-13)
+        close(outs[1][2], outs[0][2], 1e-12, 1e-14)
 
 
 @pytest.mark.parametrize("nup,ndn,B", [(10, 10, 1), (10, 10, 2), (10, 10, 297), (10, 10, 1500)])
-def test_eloc_kernel_variants_agree_full_size(dev, nup, ndn, B):
+def test_eloc_generic_and_direct_paths_agree_full_size(dev, nup, ndn, B):
     """N = 20 at H = 50, the benchmark's particle number, at four batch sizes: the default sweep (eloc5_kernel:
     register-resident Jacobian, specialised warps) against the generic flow_kernel<MODE_ELOC> (option eloc_generic),
     each with the Taylor tables and with direct evaluation of every hidden unit (no_table: eloc5_kernel evaluates every
-    item directly), against eloc5_kernel without the table mirror (no_rt_cache) and with the CTA-synchronous finale
-    (finale_cta).  Every other instantiation: tests/test_gpu_eloc_specialisations.py."""
+    item directly).  Every other instantiation: tests/test_gpu_eloc_specialisations.py."""
     model = _dot_model(dev, nsteps=4, nup=nup, ndn=ndn)
     _, x = model.sample((B,))
     res = []
     for env in (dict(eloc_generic=0, no_table=0), dict(eloc_generic=1, no_table=0), dict(eloc_generic=0, no_table=1),
-                dict(eloc_generic=1, no_table=1), dict(no_rt_cache=1), dict(finale_cta=1)):
+                dict(eloc_generic=1, no_table=1)):
         with _opts(**env):
             res.append(model.local_energy(x, stash=True))
     for r in res[1:]:
@@ -597,22 +597,26 @@ def test_free_fermion_logp_grad_laplacian_vs_oracle(dev, O, nup, ndn):
 
 
 @pytest.mark.parametrize("nup,ndn", [(10, 10), (3, 0), (6, 5)])
-def test_metropolis_kernels_bit_identical(dev, nup, ndn):
+def test_metropolis_samplers_bit_identical(dev, nup, ndn):
     """The one-warp-per-walker sampler reproduces the one-thread-per-walker chain bit for bit
     (same Philox counters, same LU arithmetic), including the acceptance counts."""
     from fermiflow_b200 import HO2D, FreeFermion
     ho = HO2D()
-    outs = []
-    for env in (dict(metropolis_kernel=2), dict(metropolis_kernel=3), dict(metropolis_kernel=1),
-                dict(metropolis_kernel=1, metropolis_no_split=1)):
-        with _opts(**env):
+
+    def chain(B, kernel):
+        with _opts(metropolis_kernel=kernel):
             ff = FreeFermion(dev)
             ff.manual_seed(77)
-            outs.append(ff.sample(ho.orbitals[:nup], ho.orbitals[:ndn], (1000,), equilibrim_steps=40))
-    assert torch.equal(outs[0], outs[1])
-    assert torch.equal(outs[0], outs[2])      # register-resident sampler (ff_metro_reg.cuh), one thread per spin block
-    assert torch.equal(outs[0], outs[3])      # ... and one thread per walker
-    assert torch.isfinite(outs[0]).all()
+            return ff.sample(ho.orbitals[:nup], ho.orbitals[:ndn], (B,), equilibrim_steps=40)
+
+    ref = chain(1000, 2)
+    assert torch.equal(ref, chain(1000, 3))
+    assert torch.equal(ref, chain(1000, 1))   # register-resident sampler (ff_metro_reg.cuh), one thread per spin block
+    assert torch.isfinite(ref).all()
+    if nup and ndn:
+        # more than 128 walkers per SM: the register sampler runs one thread per walker
+        B = 128 * torch.cuda.get_device_properties(dev).multi_processor_count + 77
+        assert torch.equal(chain(B, 2), chain(B, 1))
 
 
 def test_metropolis_register_kernel_default_at_bench_size(dev):
